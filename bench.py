@@ -2,6 +2,7 @@
 """bench.py -- throughput of the sequence-generation engine (Task-array execution) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c4] [--samples S]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -34,7 +35,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 from bench_support import (ClockSampler, StreamChecker, alg_bytes, c3_measure, cpu_engine_rate, dropin_measure,  # noqa: E402
-                           gzip_measure, make_workload, pipeline_measure, reference_binary_rate)
+                           dump_outputs, gzip_measure, make_workload, pipeline_measure, reference_binary_rate)
 
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 
@@ -88,7 +89,15 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true", help="skip the whole-cohort oracle check of the timed output")
     ap.add_argument("--ref-binary-samples", type=int, default=0,
                     help="also time the reference's prebuilt whole-tool binary on this many samples (slow)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's result tape of the last step (a fixed, seeded sample of "
+                         "it beyond 8 MiB) as float32 DIR/result_tape.npy, its window starts beside it")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.only_c3):
+        ap.error("--dump-outputs dumps the timed result tape of --impl ours; --impl reference and --only-c3 have none")
+    return args
 
 
 def ncu_traffic(args, n_res):
@@ -210,6 +219,8 @@ def main():
     total_haps = shard.sum_over_ranks(n_hap, dev)
     total_alg = shard.sum_over_ranks(b_alg, dev)
     ms_per_step = max_ms / args.steps
+    if args.dump_outputs and rank == 0:  # now: the store-ceiling probe below overwrites d_out
+        dump_outputs(args.dump_outputs, d_out, n_out)
 
     # ---- load balance of the copy grid (SURVEY 8d C4): wall time of every warp of the persistent grid, one extra launch
     eng.profile_warps(True)

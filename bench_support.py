@@ -321,6 +321,33 @@ def pipeline_measure(args, prot, cat, batch, eng, local_rank, barrier, shard, de
     return out
 
 
+# ------------------------------------------------------------------------------------------------ output dump
+DUMP_BYTES = 8 << 20  # result-tape bytes written by dump_outputs: 32 MiB as float32
+DUMP_WINDOW = 4096
+DUMP_SEED = 0x5EED00D0
+
+
+def dump_outputs(out_dir: str, tape, n_out: int) -> None:
+    """Write the result tape the timed path handed its caller (torch uint8 tape[:n_out]) under out_dir, so that two builds
+    can be compared output for output: result_tape.npy (float32 residue bytes) and result_tape_window_starts.npy (float64
+    tape offsets).  A tape of more than DUMP_BYTES is sampled in non-overlapping DUMP_WINDOW-byte windows whose starts
+    come from a fixed seed, so the same bench arguments always dump the same positions."""
+    import torch
+
+    if n_out <= DUMP_BYTES:
+        starts = np.zeros(1, np.int64)
+        sample = tape[:n_out]
+    else:
+        n_win = DUMP_BYTES // DUMP_WINDOW
+        rng = np.random.default_rng(DUMP_SEED)
+        starts = np.sort(rng.choice(n_out // DUMP_WINDOW, n_win, replace=False)).astype(np.int64) * DUMP_WINDOW
+        idx = torch.from_numpy((starts[:, None] + np.arange(DUMP_WINDOW)).reshape(-1)).to(tape.device)
+        sample = tape[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "result_tape.npy"), sample.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "result_tape_window_starts.npy"), starts.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------ whole-cohort parity
 class _DevPtr:
     """A raw device pointer as a __cuda_array_interface__ object (so torch can view library-owned HBM)."""

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -31,11 +32,40 @@ def test_reference_arm_line():
     assert "workload" in d["config"]
 
 
+def test_dump_outputs_samples_fixed_windows_of_a_long_tape(tmp_path):
+    import torch
+
+    from bench_support import DUMP_BYTES, DUMP_WINDOW, dump_outputs
+
+    n_out = DUMP_BYTES + 3 * DUMP_WINDOW + 5
+    tape = torch.from_numpy(np.random.default_rng(1).integers(0, 256, n_out + 64, dtype=np.uint8))
+    for d in ("a", "b"):
+        dump_outputs(str(tmp_path / d), tape, n_out)
+    got = {d: (np.load(tmp_path / d / "result_tape.npy"), np.load(tmp_path / d / "result_tape_window_starts.npy")) for d in "ab"}
+    sample, starts = got["a"]
+    assert sample.dtype == np.float32 and starts.dtype == np.float64 and sample.nbytes + starts.nbytes <= 64 << 20
+    assert np.array_equal(sample, got["b"][0]) and np.array_equal(starts, got["b"][1])  # same positions every run
+    s = starts.astype(np.int64)
+    assert len(s) == DUMP_BYTES // DUMP_WINDOW and (np.diff(s) >= DUMP_WINDOW).all() and s[-1] + DUMP_WINDOW <= n_out
+    want = tape.numpy()[(s[:, None] + np.arange(DUMP_WINDOW)).reshape(-1)]
+    assert np.array_equal(sample, want.astype(np.float32))
+
+
+@pytest.mark.parametrize("args,flag", [(["--steps", "0"], "--steps"),
+                                       (["--impl", "reference", "--dump-outputs", "d"], "--dump-outputs"),
+                                       (["--only-c3", "--dump-outputs", "d"], "--dump-outputs")])
+def test_meaningless_arguments_are_refused(args, flag):
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], stdout=subprocess.PIPE,
+                       stderr=subprocess.PIPE, text=True, timeout=120)
+    assert p.returncode == 2 and flag in p.stderr
+
+
 @pytest.mark.gpu
-def test_our_arm_line_on_a_tiny_cohort():
+def test_our_arm_line_on_a_tiny_cohort(tmp_path):
     d = run_bench("--samples", "24", "--steps", "3", "--warmup", "3", "--e2e-steps", "1", "--e2e-chunk-haps", "16", "--cpu-sample-haps", "8",
                   "--cpu-seconds", "0.5", "--maskdecode-samples", "8", "--gzip-samples", "8", "--pipeline-chunk", "5",
-                  "--written-samples", "6", "--c3-samples", "40", "--c3-chunk-samples", "16", "--dropin-haps", "6")
+                  "--written-samples", "6", "--c3-samples", "40", "--c3-chunk-samples", "16", "--dropin-haps", "6",
+                  "--dump-outputs", str(tmp_path))
     assert BASE <= set(d) and d["n_gpus"] == 1 and d["scaling"] == "weak" and d["dtype"] == "u8" and d["vs_baseline"] is None
     assert d["gpu_launches"] == 7 * d["steps"] and d["warmup"] >= 3  # init, plan x4, copy, status hand-off
     assert {"sm_mhz", "sm_max_mhz", "reasons"} <= set(d["clocks"])
@@ -60,3 +90,14 @@ def test_our_arm_line_on_a_tiny_cohort():
     for k in ("fasta", "fasta_gz"):
         assert d["pipeline"][k]["first_and_last_file_equal_oracle_text"] is True
         assert d["pipeline"]["written"][k]["first_file_equals_oracle_text"] is True
+    # the dump is the timed step's result tape: the oracle's bytes at the dumped windows
+    from bench_support import DUMP_WINDOW, make_workload
+    from oracle import cengine
+
+    prot, _, b = make_workload("c2", 24, 0)
+    want = np.zeros(b.n_residues, np.uint8)
+    assert cengine.batch_execute(b.task_begin, b.tasks, prot.residues, b.alt, b.alt_base, want, b.out_base, threads=4)[0] == 0
+    starts = np.load(tmp_path / "result_tape_window_starts.npy").astype(np.int64)
+    assert b.n_residues == d["config"]["result_tape_bytes_per_gpu"] and len(starts) > 1
+    sample = np.load(tmp_path / "result_tape.npy")
+    assert np.array_equal(sample, want[(starts[:, None] + np.arange(DUMP_WINDOW)).reshape(-1)].astype(np.float32))
