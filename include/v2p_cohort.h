@@ -92,10 +92,15 @@ int v2p_cohort_enable_all_records(v2p_cohort* c, const v2p_cohort_inputs* in);
 int v2p_cohort_run_lists(v2p_cohort* c, uint64_t n_samples, const uint64_t* site_begin, const uint32_t* sites,
                          uint32_t chunk_samples, uint32_t flags, v2p_file_sink sink, void* user, v2p_cohort_result* res);
 
-/* Same from the FORMAT/BCSQ mask matrix (host memory; arguments as v2p_sites_from_masks, include/v2p_taskgen.h).
+#define V2P_COHORT_DEVICE_MASKS 0x200u /* v2p_cohort_run_masks: `masks` is device memory on the FIRST worker's device (e.g.
+                                        * v2p_vcf_parse_masks, include/v2p_vcf.h); it is decoded there without an upload */
+
+/* Same from the FORMAT/BCSQ mask matrix (host memory, or with V2P_COHORT_DEVICE_MASKS device memory on the first
+ * worker's device; arguments as v2p_sites_from_masks, include/v2p_taskgen.h).
  * The matrix is decoded ONCE, on the first worker's device (the decode reads every record of every sample exactly once
  * and is a fraction of a percent of the job); its CSR lists -- 4 bytes per carried site -- come back to the host, are
- * split by the rule above and each worker uploads its own range.  res->total.decode_ms / h2d_bytes include the decode. */
+ * split by the rule above and each worker uploads its own range.  res->total.decode_ms includes the decode, and
+ * h2d_bytes the matrix upload (none with V2P_COHORT_DEVICE_MASKS). */
 int v2p_cohort_run_masks(v2p_cohort* c, uint64_t n_records, uint64_t n_samples, uint32_t words_per_cell,
                          const uint32_t* masks, const uint64_t* csq_begin, const int32_t* csq_site, uint32_t chunk_samples,
                          uint32_t flags, v2p_file_sink sink, void* user, v2p_cohort_result* res);

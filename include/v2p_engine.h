@@ -41,8 +41,9 @@ enum {
     V2P_ERR_NOT_CONTIGUOUS = 7, /* V2P_FLAG_VALIDATE: gir.rs:208-225 (DEBUG_CPU_EXEC / DEBUG_GPU) check */
     /* 8 is reserved (UTF-32 tapes are executed natively as 4-byte units, any code point is fine)       */
     V2P_ERR_NOT_GPU_ENGINE = 9, /* v2p_gir_execute called with ST/MT: those stay in the caller          */
-    V2P_ERR_TASKGEN = 10        /* device task generation: the reference aborts on this transcript (usize
+    V2P_ERR_TASKGEN = 10,       /* device task generation: the reference aborts on this transcript (usize
                                    underflow in add_till_next_ins / add_last_instruction, negative result size) */
+    V2P_ERR_VCF_PARSE = 11      /* VCF text outside the dialect of include/v2p_vcf.h (message: line, sample)  */
 };
 
 /* ---- engine selection (engines.rs:15-30) ------------------------------------------------------- */

@@ -31,6 +31,7 @@
 #include "v2p_engine.h"
 #include "v2p_cohort.h"
 #include "v2p_pipeline.h"
+#include "v2p_vcf.h"
 
 namespace v2p {
 
@@ -433,6 +434,64 @@ public:
 
 private:
     v2p_cohort* c_ = nullptr;
+};
+
+// VCF sample columns on the device (include/v2p_vcf.h): the text is loaded and indexed once; the host reads columns 1-9
+// of the records it wants (text[line_begin, cells_begin)) and parses their sample cells into the FORMAT/BCSQ mask
+// matrix, which stays on the device for v2p_pipeline_run_masks / v2p_cohort_run_masks.  RAII over v2p_vcf_create.
+class VcfText {
+public:
+    explicit VcfText(int cuda_device = 0) {
+        if (v2p_vcf_create(cuda_device, &v_) != V2P_OK) throw EngineError(V2P_ERR_CUDA, "v2p_vcf_create failed (no such device?)");
+    }
+    ~VcfText() { v2p_vcf_destroy(v_); }
+    VcfText(const VcfText&) = delete;
+    VcfText& operator=(const VcfText&) = delete;
+
+    // Host text (pinned memory uploads at the full PCIe rate), or device text on this object's device (16-byte aligned,
+    // alive until the next load).  The tables in the result are owned by this object until the next load.
+    const v2p_vcf_lines& load(const uint8_t* text, uint64_t n_bytes, bool device_text = false) {
+        const int st = v2p_vcf_load(v_, text, n_bytes, device_text ? V2P_FLAG_DEVICE_PTRS : 0u, &lines_);
+        if (st != V2P_OK) throw EngineError(st, v2p_vcf_last_error(v_));
+        names_.clear();
+        if (!device_text && lines_.n_samples) {
+            const std::string hdr(reinterpret_cast<const char*>(text) + lines_.header_begin, lines_.header_end - lines_.header_begin);
+            size_t col = 0, at = 0;
+            for (size_t tab = hdr.find('\t'); ; tab = hdr.find('\t', at)) {
+                if (col++ >= 9) names_.push_back(hdr.substr(at, tab == std::string::npos ? std::string::npos : tab - at));
+                if (tab == std::string::npos) break;
+                at = tab + 1;
+            }
+        }
+        return lines_;
+    }
+    const v2p_vcf_lines& load(const std::string& text) { return load(reinterpret_cast<const uint8_t*>(text.data()), text.size()); }
+
+    // Sample names of the #CHROM line (host text only).
+    const std::vector<std::string>& sample_names() const { return names_; }
+
+    // Row r of the matrix = data line rec_line[r].  The matrix is device memory owned by this object until the next call.
+    v2p_vcf_masks parse_masks(const std::vector<uint64_t>& rec_line) {
+        v2p_vcf_masks m{};
+        const int st = v2p_vcf_parse_masks(v_, rec_line.size(), rec_line.data(), 0, &m);
+        if (st != V2P_OK) throw EngineError(st, v2p_vcf_last_error(v_));
+        return m;
+    }
+
+    // Device -> host copy of a matrix (tests, debugging).
+    static std::vector<uint32_t> read(const v2p_vcf_masks& m) {
+        std::vector<uint32_t> out(m.n_records * m.n_samples * m.words_per_cell);
+        if (!out.empty() && v2p_device_read(out.data(), m.masks, out.size() * sizeof(uint32_t)) != V2P_OK)
+            throw EngineError(V2P_ERR_CUDA, "v2p_device_read failed");
+        return out;
+    }
+
+    v2p_vcf* get() { return v_; }
+
+private:
+    v2p_vcf* v_ = nullptr;
+    v2p_vcf_lines lines_{};
+    std::vector<std::string> names_;
 };
 
 }  // namespace v2p

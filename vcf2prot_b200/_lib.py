@@ -10,14 +10,15 @@ LIB_PATH = os.environ.get("V2P_ENGINE_LIB") or os.path.join(HERE, "libv2p_engine
 
 V2P_OK = 0
 ERR_INVALID_ARG, ERR_CUDA, ERR_BAD_ENGINE, ERR_BAD_STREAM, ERR_RES_OOB, ERR_SRC_OOB = 1, 2, 3, 4, 5, 6
-ERR_NOT_CONTIGUOUS, ERR_NOT_GPU_ENGINE, ERR_TASKGEN = 7, 9, 10
+ERR_NOT_CONTIGUOUS, ERR_NOT_GPU_ENGINE, ERR_TASKGEN, ERR_VCF_PARSE = 7, 9, 10, 11
 ENGINE_ST, ENGINE_MT, ENGINE_GPU = 0, 1, 2
 FLAG_FILL_DOT, FLAG_VALIDATE, FLAG_DEVICE_PTRS, FLAG_ASYNC, FLAG_ALIGNED_LAYOUT = 1, 2, 4, 8, 16
 REF_NO_TMA = 0x200
 GEN_ALIGNED, GEN_FASTA, GEN_SKIP_ABORTS = 1, 2, 4
 
 STATUS_NAMES = {0: "OK", 1: "INVALID_ARG", 2: "CUDA", 3: "BAD_ENGINE", 4: "BAD_STREAM", 5: "RES_OOB", 6: "SRC_OOB",
-                7: "NOT_CONTIGUOUS", 9: "NOT_GPU_ENGINE", 10: "TASKGEN"}
+                7: "NOT_CONTIGUOUS", 9: "NOT_GPU_ENGINE", 10: "TASKGEN",
+                11: "VCF_PARSE"}
 
 
 class Task16(C.Structure):
@@ -63,6 +64,18 @@ class PipelineResult(C.Structure):
 
 COHORT_MAX_DEVICES = 16
 COHORT_CONCURRENT_SINK = 0x100
+COHORT_DEVICE_MASKS = 0x200
+
+
+class VcfLines(C.Structure):  # include/v2p_vcf.h: v2p_vcf_lines
+    _fields_ = [("n_samples", C.c_uint64), ("header_begin", C.c_uint64), ("header_end", C.c_uint64), ("n_lines", C.c_uint64),
+                ("line_begin", C.c_void_p), ("cells_begin", C.c_void_p), ("h2d_bytes", C.c_uint64), ("h2d_ms", C.c_float),
+                ("index_ms", C.c_float)]
+
+
+class VcfMasks(C.Structure):  # v2p_vcf_masks
+    _fields_ = [("masks", C.c_void_p), ("n_records", C.c_uint64), ("n_samples", C.c_uint64), ("words_per_cell", C.c_uint32),
+                ("parse_ms", C.c_float)]
 
 
 class CohortInputs(C.Structure):  # include/v2p_cohort.h: v2p_cohort_inputs
@@ -145,6 +158,12 @@ SYMBOLS = {
                                        C.POINTER(CohortResult)]),
     "v2p_pipeline_run_masks": (C.c_int, [_P, C.c_uint64, C.c_uint64, C.c_uint32, _P, _P, _P, C.c_uint32, C.c_uint32, C.c_uint32,
                                          _P, C.c_uint64, _P, FILE_SINK, _P, C.POINTER(PipelineResult)]),
+    # include/v2p_vcf.h
+    "v2p_vcf_create": (C.c_int, [C.c_int, C.POINTER(_P)]),
+    "v2p_vcf_destroy": (None, [_P]),
+    "v2p_vcf_last_error": (C.c_char_p, [_P]),
+    "v2p_vcf_load": (C.c_int, [_P, _P, C.c_uint64, C.c_uint32, C.POINTER(VcfLines)]),
+    "v2p_vcf_parse_masks": (C.c_int, [_P, C.c_uint64, _P, C.c_uint32, C.POINTER(VcfMasks)]),
 }
 
 _lib = None

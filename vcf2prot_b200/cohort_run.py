@@ -71,16 +71,22 @@ class CohortRunner:
             raise EngineError(st, (self._lib.v2p_cohort_last_error(self._h) or b"").decode())
         return res
 
-    def run_masks(self, masks: np.ndarray, csq_begin: np.ndarray, csq_site: np.ndarray, chunk_samples: int = 128, gzip: bool = False,
-                  sink: Optional[Callable] = None, concurrent_sink: bool = False, all_records: bool = False) -> L.CohortResult:
-        """masks[n_records, n_samples, W] (FORMAT/BCSQ integers): decoded once on the first device, then as run_lists."""
-        masks = np.ascontiguousarray(masks, np.uint32)
-        n_rec, n_samp, w = masks.shape
+    def run_masks(self, masks, csq_begin: np.ndarray, csq_site: np.ndarray, chunk_samples: int = 128, gzip: bool = False,
+                  sink: Optional[Callable] = None, concurrent_sink: bool = False, all_records: bool = False, shape=None) -> L.CohortResult:
+        """masks[n_records, n_samples, W] (FORMAT/BCSQ integers): decoded once on the first device, then as run_lists.
+        numpy array, or a device pointer (int) on the first worker's device with shape=(n_records, n_samples, W)."""
+        flags = (L.PIPE_GZIP if gzip else 0) | (L.COHORT_CONCURRENT_SINK if concurrent_sink else 0) | (L.PIPE_ALL_RECORDS if all_records else 0)
+        if isinstance(masks, np.ndarray):
+            masks = np.ascontiguousarray(masks, np.uint32)
+            n_rec, n_samp, w = masks.shape
+            mp = masks.ctypes.data_as(C.c_void_p)
+        else:
+            n_rec, n_samp, w = shape
+            mp, flags = C.c_void_p(int(masks)), flags | L.COHORT_DEVICE_MASKS
         cbeg, csite = np.ascontiguousarray(csq_begin, np.uint64), np.ascontiguousarray(csq_site, np.int32)
         cb, user, keep = DevicePipeline._sink(sink)
         res = L.CohortResult()
-        flags = (L.PIPE_GZIP if gzip else 0) | (L.COHORT_CONCURRENT_SINK if concurrent_sink else 0) | (L.PIPE_ALL_RECORDS if all_records else 0)
-        st = self._lib.v2p_cohort_run_masks(self._h, n_rec, n_samp, w, masks.ctypes.data_as(C.c_void_p), cbeg.ctypes.data_as(C.c_void_p),
+        st = self._lib.v2p_cohort_run_masks(self._h, n_rec, n_samp, w, mp, cbeg.ctypes.data_as(C.c_void_p),
                                             csite.ctypes.data_as(C.c_void_p), chunk_samples, flags, cb, user, C.byref(res))
         del keep
         if st:

@@ -255,7 +255,9 @@ int v2p_cohort_run_masks(v2p_cohort* c, uint64_t n_records, uint64_t n_samples, 
     if (cudaSetDevice(w0.device) != cudaSuccess) return cofail(c, V2P_ERR_CUDA, "cudaSetDevice(%d) failed", w0.device);
     v2p_site_lists lists;
     memset(&lists, 0, sizeof lists);
-    int rc = v2p_sites_from_masks(w0.lanes[0], n_records, n_samples, words_per_cell, masks, csq_begin, csq_site, 0, &lists);
+    const bool dev = flags & V2P_COHORT_DEVICE_MASKS;
+    int rc = v2p_sites_from_masks(w0.lanes[0], n_records, n_samples, words_per_cell, masks, csq_begin, csq_site,
+                                  dev ? V2P_FLAG_DEVICE_PTRS : 0u, &lists);
     if (rc != V2P_OK) return cofail(c, rc, "mask decode on device %d: %s", w0.device, v2p_catalogue_last_error(w0.lanes[0]));
     std::vector<uint64_t> sb(2 * n_samples + 1, 0);
     std::vector<uint32_t> sites(lists.n_sites);
@@ -264,9 +266,9 @@ int v2p_cohort_run_masks(v2p_cohort* c, uint64_t n_records, uint64_t n_samples, 
     if (rc != V2P_OK) return cofail(c, rc, "reading the decoded lists back from device %d failed", w0.device);
     v2p_cohort_result local;
     memset(&local, 0, sizeof local);
-    rc = v2p_cohort_run_lists(c, n_samples, sb.data(), sites.data(), chunk_samples, flags, sink, user, &local);
+    rc = v2p_cohort_run_lists(c, n_samples, sb.data(), sites.data(), chunk_samples, flags & ~V2P_COHORT_DEVICE_MASKS, sink, user, &local);
     local.total.decode_ms += lists.decode_ms, local.per_device[0].decode_ms += lists.decode_ms;
-    const uint64_t up = n_records * n_samples * (uint64_t)words_per_cell * sizeof(uint32_t);
+    const uint64_t up = dev ? 0 : n_records * n_samples * (uint64_t)words_per_cell * sizeof(uint32_t);
     local.total.h2d_bytes += up, local.per_device[0].h2d_bytes += up;
     if (res) *res = local;
     return rc;
