@@ -43,7 +43,8 @@ enum {
     V2P_ERR_NOT_GPU_ENGINE = 9, /* v2p_gir_execute called with ST/MT: those stay in the caller          */
     V2P_ERR_TASKGEN = 10,       /* device task generation: the reference aborts on this transcript (usize
                                    underflow in add_till_next_ins / add_last_instruction, negative result size) */
-    V2P_ERR_VCF_PARSE = 11      /* VCF text outside the dialect of include/v2p_vcf.h (message: line, sample)  */
+    V2P_ERR_VCF_PARSE = 11,     /* VCF text outside the dialect of include/v2p_vcf.h (message: line, sample)  */
+    V2P_ERR_BGZF = 12           /* input that is not valid BGZF (include/v2p_vcf.h; message: block, byte, class) */
 };
 
 /* ---- engine selection (engines.rs:15-30) ------------------------------------------------------- */

@@ -32,6 +32,7 @@
 #include "v2p_cohort.h"
 #include "v2p_pipeline.h"
 #include "v2p_vcf.h"
+#include "v2p_vcf_bgzf.h"
 
 namespace v2p {
 
@@ -453,21 +454,32 @@ public:
     const v2p_vcf_lines& load(const uint8_t* text, uint64_t n_bytes, bool device_text = false) {
         const int st = v2p_vcf_load(v_, text, n_bytes, device_text ? V2P_FLAG_DEVICE_PTRS : 0u, &lines_);
         if (st != V2P_OK) throw EngineError(st, v2p_vcf_last_error(v_));
-        names_.clear();
-        if (!device_text && lines_.n_samples) {
-            const std::string hdr(reinterpret_cast<const char*>(text) + lines_.header_begin, lines_.header_end - lines_.header_begin);
-            size_t col = 0, at = 0;
-            for (size_t tab = hdr.find('\t'); ; tab = hdr.find('\t', at)) {
-                if (col++ >= 9) names_.push_back(hdr.substr(at, tab == std::string::npos ? std::string::npos : tab - at));
-                if (tab == std::string::npos) break;
-                at = tab + 1;
-            }
-        }
+        bgzf_ = v2p_vcf_bgzf{};
+        set_names(device_text ? nullptr : text);
         return lines_;
     }
     const v2p_vcf_lines& load(const std::string& text) { return load(reinterpret_cast<const uint8_t*>(text.data()), text.size()); }
 
-    // Sample names of the #CHROM line (host text only).
+    // A bgzip'd file (host memory; pinned uploads at the full PCIe rate), inflated and indexed on the device.  Offsets
+    // in the result are into the inflated text; the host reads columns 1-9 from bgzf().fixed (sliced by fixed_begin)
+    // and the header lines from bgzf().head.  Both are owned by this object until the next load.
+    const v2p_vcf_lines& load_bgzf(const uint8_t* data, uint64_t n_bytes) {
+        const int st = v2p_vcf_load_bgzf(v_, data, n_bytes, 0, &lines_, &bgzf_);
+        if (st != V2P_OK) throw EngineError(st, v2p_vcf_last_error(v_));
+        set_names(bgzf_.head);
+        return lines_;
+    }
+    const v2p_vcf_lines& load_bgzf(const std::string& data) { return load_bgzf(reinterpret_cast<const uint8_t*>(data.data()), data.size()); }
+
+    // What the last load_bgzf found (zeroed after a plain load).
+    const v2p_vcf_bgzf& bgzf() const { return bgzf_; }
+
+    // Columns 1-9 of data line l after load_bgzf.
+    std::string fixed(uint64_t l) const {
+        return std::string(reinterpret_cast<const char*>(bgzf_.fixed) + bgzf_.fixed_begin[l], bgzf_.fixed_begin[l + 1] - bgzf_.fixed_begin[l]);
+    }
+
+    // Sample names of the #CHROM line (host text or BGZF input).
     const std::vector<std::string>& sample_names() const { return names_; }
 
     // Row r of the matrix = data line rec_line[r].  The matrix is device memory owned by this object until the next call.
@@ -489,8 +501,21 @@ public:
     v2p_vcf* get() { return v_; }
 
 private:
+    void set_names(const uint8_t* text) {  // text[header_begin, header_end) is the #CHROM line
+        names_.clear();
+        if (!text || !lines_.n_samples) return;
+        const std::string hdr(reinterpret_cast<const char*>(text) + lines_.header_begin, lines_.header_end - lines_.header_begin);
+        size_t col = 0, at = 0;
+        for (size_t tab = hdr.find('\t'); ; tab = hdr.find('\t', at)) {
+            if (col++ >= 9) names_.push_back(hdr.substr(at, tab == std::string::npos ? std::string::npos : tab - at));
+            if (tab == std::string::npos) break;
+            at = tab + 1;
+        }
+    }
+
     v2p_vcf* v_ = nullptr;
     v2p_vcf_lines lines_{};
+    v2p_vcf_bgzf bgzf_{};
     std::vector<std::string> names_;
 };
 

@@ -13,6 +13,8 @@
  *                        reads INFO/BCSQ there, keeps the records it supports and maps their consequences to catalogue
  *                        sites (per record, not per sample).
  *   v2p_vcf_parse_masks  parse the sample cells of the chosen data lines into the mask matrix.
+ * A bgzip'd file (.vcf.gz) goes in through v2p_vcf_load_bgzf (include/v2p_vcf_bgzf.h) instead of v2p_vcf_load: it is
+ * inflated on the device, and the host gets columns 1-9 of every data line back, since it has no text of its own.
  *
  * Dialect (the minimal VCF the reference reads, SURVEY.md section 8c):
  *   - Lines end at '\n'; a '\r' that ends a line is not part of it; a last line without '\n' counts.

@@ -10,7 +10,7 @@ LIB_PATH = os.environ.get("V2P_ENGINE_LIB") or os.path.join(HERE, "libv2p_engine
 
 V2P_OK = 0
 ERR_INVALID_ARG, ERR_CUDA, ERR_BAD_ENGINE, ERR_BAD_STREAM, ERR_RES_OOB, ERR_SRC_OOB = 1, 2, 3, 4, 5, 6
-ERR_NOT_CONTIGUOUS, ERR_NOT_GPU_ENGINE, ERR_TASKGEN, ERR_VCF_PARSE = 7, 9, 10, 11
+ERR_NOT_CONTIGUOUS, ERR_NOT_GPU_ENGINE, ERR_TASKGEN, ERR_VCF_PARSE, ERR_BGZF = 7, 9, 10, 11, 12
 ENGINE_ST, ENGINE_MT, ENGINE_GPU = 0, 1, 2
 FLAG_FILL_DOT, FLAG_VALIDATE, FLAG_DEVICE_PTRS, FLAG_ASYNC, FLAG_ALIGNED_LAYOUT = 1, 2, 4, 8, 16
 REF_NO_TMA = 0x200
@@ -18,7 +18,7 @@ GEN_ALIGNED, GEN_FASTA, GEN_SKIP_ABORTS = 1, 2, 4
 
 STATUS_NAMES = {0: "OK", 1: "INVALID_ARG", 2: "CUDA", 3: "BAD_ENGINE", 4: "BAD_STREAM", 5: "RES_OOB", 6: "SRC_OOB",
                 7: "NOT_CONTIGUOUS", 9: "NOT_GPU_ENGINE", 10: "TASKGEN",
-                11: "VCF_PARSE"}
+                11: "VCF_PARSE", 12: "BGZF"}
 
 
 class Task16(C.Structure):
@@ -71,6 +71,11 @@ class VcfLines(C.Structure):  # include/v2p_vcf.h: v2p_vcf_lines
     _fields_ = [("n_samples", C.c_uint64), ("header_begin", C.c_uint64), ("header_end", C.c_uint64), ("n_lines", C.c_uint64),
                 ("line_begin", C.c_void_p), ("cells_begin", C.c_void_p), ("h2d_bytes", C.c_uint64), ("h2d_ms", C.c_float),
                 ("index_ms", C.c_float)]
+
+
+class VcfBgzf(C.Structure):  # v2p_vcf_bgzf
+    _fields_ = [("n_blocks", C.c_uint64), ("text_bytes", C.c_uint64), ("text", C.c_void_p), ("head", C.c_void_p),
+                ("fixed", C.c_void_p), ("fixed_begin", C.c_void_p), ("inflate_ms", C.c_float), ("fixed_ms", C.c_float)]
 
 
 class VcfMasks(C.Structure):  # v2p_vcf_masks
@@ -163,6 +168,7 @@ SYMBOLS = {
     "v2p_vcf_destroy": (None, [_P]),
     "v2p_vcf_last_error": (C.c_char_p, [_P]),
     "v2p_vcf_load": (C.c_int, [_P, _P, C.c_uint64, C.c_uint32, C.POINTER(VcfLines)]),
+    "v2p_vcf_load_bgzf": (C.c_int, [_P, _P, C.c_uint64, C.c_uint32, C.POINTER(VcfLines), C.POINTER(VcfBgzf)]),
     "v2p_vcf_parse_masks": (C.c_int, [_P, C.c_uint64, _P, C.c_uint32, C.POINTER(VcfMasks)]),
 }
 

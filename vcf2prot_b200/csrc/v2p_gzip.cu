@@ -19,6 +19,7 @@
 #include <string>
 #include <vector>
 
+#include "v2p_crc32.cuh"
 #include "v2p_gzip.h"
 #include "v2p_mapped.cuh"
 
@@ -28,63 +29,12 @@ constexpr int CH = V2P_GZIP_CHUNK;
 constexpr int NT = 256;
 constexpr int PIECE = CH / NT;  // bytes of a chunk one thread owns
 constexpr int LENS_STRIDE = 272;  // 257 code lengths, [260] = 1 when the chunk is a stored block
-constexpr uint32_t POLY = 0xEDB88320u;
 static_assert(PIECE == 64, "piece = 16 words");
 
 // code-length alphabet: fixed complete code, thirteen 4-bit + six 5-bit symbols; codes are canonical, bit-reversed
 __constant__ uint8_t c_cl_len[19] = {4, 5, 5, 5, 4, 4, 4, 4, 4, 4, 4, 4, 4, 5, 5, 5, 4, 4, 4};
 __constant__ uint8_t c_cl_code[19] = {0, 11, 27, 7, 8, 4, 12, 2, 10, 6, 14, 1, 9, 23, 15, 31, 5, 13, 3};
 __constant__ uint8_t c_cl_order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-
-__device__ uint32_t g_crc_tab[4][256];  // slicing-by-4: [k][b] = CRC of byte b followed by k zero bytes
-__device__ uint32_t g_xp8[40];   // x^(8 * 2^j) mod P, reflected
-__device__ uint32_t g_x64[256];  // x^(8 * 64 * k): a CRC moved past k whole pieces
-__device__ uint32_t g_xb[65];    // x^(8 * m),  m = 0..64
-
-// a*b mod P, reflected representation (bit 31 is x^0)
-__device__ __forceinline__ uint32_t gf_mul(uint32_t a, uint32_t b) {
-    uint32_t p = 0;
-#pragma unroll
-    for (int i = 0; i < 32; ++i) {
-        p ^= (a & (0x80000000u >> i)) ? b : 0u;
-        b = (b >> 1) ^ ((b & 1u) ? POLY : 0u);
-    }
-    return p;
-}
-
-__device__ __forceinline__ uint32_t x_pow_8n(uint64_t n) {  // x^(8n) mod P
-    uint32_t r = 0x80000000u;
-    for (int j = 0; n; ++j, n >>= 1)
-        if (n & 1) r = gf_mul(r, g_xp8[j]);
-    return r;
-}
-
-__global__ void k_gz_init() {
-    const int t = threadIdx.x;
-    uint32_t c = (uint32_t)t;
-    for (int k = 0; k < 8; ++k) c = (c >> 1) ^ ((c & 1u) ? POLY : 0u);
-    g_crc_tab[0][t] = c;
-    __syncthreads();
-    for (int k = 1; k < 4; ++k) {
-        c = (c >> 8) ^ g_crc_tab[0][c & 255u];
-        g_crc_tab[k][t] = c;
-    }
-    uint32_t x8 = 0x80000000u >> 8, xb = 0x80000000u, x64;  // x^8, then x^(8t) by t multiplications
-    for (int k = 0; k < t && k < 65; ++k) xb = gf_mul(xb, x8);
-    if (t < 65) g_xb[t] = xb;
-    x64 = x8;
-    for (int k = 0; k < 6; ++k) x64 = gf_mul(x64, x64);  // x^(8*64)
-    uint32_t v = 0x80000000u;
-    for (int k = 0; k < t; ++k) v = gf_mul(v, x64);
-    g_x64[t] = v;
-    if (t == 0) {
-        uint32_t sq = x8;
-        for (int j = 0; j < 40; ++j) {
-            g_xp8[j] = sq;
-            sq = gf_mul(sq, sq);
-        }
-    }
-}
 
 struct GzArgs {
     const uint8_t* in;        // base such that file bytes are in[file_begin[f] ..)
@@ -743,7 +693,7 @@ int v2p_gzip_create(int cuda_device, v2p_gzip** out) {
         return V2P_ERR_CUDA;
     }
     cudaDeviceGetAttribute(&z->sms, cudaDevAttrMultiProcessorCount, cuda_device);
-    k_gz_init<<<1, 256, 0, z->stream>>>();
+    k_crc32_init<<<1, 256, 0, z->stream>>>();
     if (cudaStreamSynchronize(z->stream) != cudaSuccess) {
         v2p_gzip_destroy(z);
         return V2P_ERR_CUDA;

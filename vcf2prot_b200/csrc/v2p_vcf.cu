@@ -16,6 +16,10 @@
 //   check       cell counts per line and the first error in file order (lowest line, then sample column)
 //   pass 2      every cell is parsed by the lane holding the tab in front of it (cell 0: the line's first lane),
 //               reading past the segment as far as the cell goes, and writes its zero-padded words
+// BGZF input (v2p_vcf_load_bgzf): the host walks the block headers while the compressed bytes upload, k_inflate
+// (v2p_inflate.cuh) writes the text, then the same index runs on it, and
+//   fixed_len   one thread per data line: bytes of columns 1-9; (scan) -> fixed_begin
+//   fixed       one warp per data line, 16-byte loads: columns 1-9 of every data line, concatenated, for the host
 // Small results come back through mapped memory (v2p_mapped.cuh), not the copy engine: load waits for the line count
 // (to size the line arrays) and for the header counters before it copies the line tables back; parse waits once, for the
 // matrix width and the first error.
@@ -31,8 +35,10 @@
 #include <string>
 #include <vector>
 
+#include "v2p_inflate.cuh"
 #include "v2p_mapped.cuh"
 #include "v2p_vcf.h"
+#include "v2p_vcf_bgzf.h"
 
 namespace {
 
@@ -218,6 +224,30 @@ __global__ void k_find_cells(const uint8_t* __restrict__ text, const uint64_t* _
     }
 }
 
+// columns 1-9 of every data line, concatenated in file order (BGZF input: the host has no text of its own)
+__global__ void k_fixed_len(const uint64_t* __restrict__ line_begin, const uint64_t* __restrict__ cells_begin, uint64_t n,
+                            uint64_t* __restrict__ len) {
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i == n) len[n] = 0;
+    if (i < n) len[i] = cells_begin[i] - line_begin[i];
+}
+
+__global__ void k_fixed(const uint8_t* __restrict__ text, const uint64_t* __restrict__ line_begin, const uint64_t* __restrict__ cells_begin,
+                        const uint64_t* __restrict__ fixed_x, uint64_t n_lines, uint8_t* __restrict__ fixed) {
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t warp = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * (uint64_t)blockDim.x) >> 5;
+    for (uint64_t l = warp; l < n_lines; l += n_warps) {
+        const uint64_t b = line_begin[l], e = cells_begin[l], x = fixed_x[l];
+        for (uint64_t o = (b & ~15ull) + 16 * lane; o < e; o += kSeg) {
+            const uint4 v = load16(text, o);
+            for (uint32_t m = range_bits(o, b, e); m; m &= m - 1) {
+                const uint32_t k = __ffs(m) - 1;
+                fixed[x + (o + k - b)] = (uint8_t)byte_of(v, k);
+            }
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------- parse
 struct ParseArgs {
     const uint8_t* text;
@@ -385,11 +415,16 @@ __global__ void k_check(ParseArgs a) {
 
 }  // namespace
 
+struct HostBuf {  // pinned host memory
+    void* p = nullptr;
+    size_t cap = 0;
+};
+
 struct v2p_vcf {
     int device = 0;
     int sms = 148;
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    cudaEvent_t ev[7] = {};
     std::string err;
     v2p::MappedBuf pub;
     // the loaded text and its index
@@ -398,6 +433,10 @@ struct v2p_vcf {
     uint64_t n_bytes = 0, n_lines = 0, n_samples = 0;
     Buf buf_text, tile_cnt, tile_x, starts, ends, is_data, data_x, line_begin, line_end, line_no, cells_begin, has_cells, ctr, cub_tmp;
     std::vector<uint64_t> h_line_begin, h_cells_begin;
+    // BGZF input: compressed bytes, block table; columns 1-9 for the host
+    Buf comp, blocks, fixed_len, fixed_x, fixed;
+    std::vector<BgzfBlock> h_blocks;
+    HostBuf h_head, h_fixed, h_fixed_begin;
     // parse
     Buf rec_line, n_seg, seg_begin, seg_tabs, seg_tab_x, seg_err, seg_rec, masks;
 };
@@ -450,68 +489,23 @@ int fetch(v2p_vcf* v, const void* src, uint64_t n_words, void* dst) {
 
 inline unsigned blocks(uint64_t n) { return (unsigned)((n + 255) / 256); }
 
-}  // namespace
-
-extern "C" {
-
-int v2p_vcf_create(int cuda_device, v2p_vcf** out) {
-    if (!out) return V2P_ERR_INVALID_ARG;
-    *out = nullptr;
-    v2p_vcf* v = new (std::nothrow) v2p_vcf();
-    if (!v) return V2P_ERR_INVALID_ARG;
-    v->device = cuda_device;
-    bool ok = cudaSetDevice(cuda_device) == cudaSuccess && cudaStreamCreateWithFlags(&v->stream, cudaStreamNonBlocking) == cudaSuccess &&
-              cudaDeviceGetAttribute(&v->sms, cudaDevAttrMultiProcessorCount, cuda_device) == cudaSuccess;
-    for (int i = 0; ok && i < 4; ++i) ok = cudaEventCreate(&v->ev[i]) == cudaSuccess;
-    if (!ok) {
-        v2p_vcf_destroy(v);
-        return V2P_ERR_CUDA;
-    }
-    *out = v;
+int hneed(v2p_vcf* v, HostBuf& b, size_t bytes) {
+    bytes = bytes < 256 ? 256 : bytes;
+    if (b.cap >= bytes) return V2P_OK;
+    if (b.p) CU(v, cudaFreeHost(b.p));
+    b.p = nullptr, b.cap = 0;
+    CU(v, cudaHostAlloc(&b.p, bytes + bytes / 8, cudaHostAllocDefault));
+    b.cap = bytes + bytes / 8;
     return V2P_OK;
 }
 
-void v2p_vcf_destroy(v2p_vcf* v) {
-    if (!v) return;
-    cudaSetDevice(v->device);
-    if (v->stream) cudaStreamSynchronize(v->stream);
-    Buf* all[] = {&v->buf_text, &v->tile_cnt, &v->tile_x, &v->starts, &v->ends, &v->is_data, &v->data_x, &v->line_begin,
-                  &v->line_end, &v->line_no, &v->cells_begin, &v->has_cells, &v->ctr, &v->cub_tmp, &v->rec_line, &v->n_seg,
-                  &v->seg_begin, &v->seg_tabs, &v->seg_tab_x, &v->seg_err, &v->seg_rec, &v->masks};
-    for (Buf* b : all)
-        if (b->p) cudaFree(b->p);
-    v->pub.release();
-    for (cudaEvent_t e : v->ev)
-        if (e) cudaEventDestroy(e);
-    if (v->stream) cudaStreamDestroy(v->stream);
-    delete v;
-}
-
-const char* v2p_vcf_last_error(v2p_vcf* v) { return v ? v->err.c_str() : "vcf object is NULL"; }
-
-int v2p_vcf_load(v2p_vcf* v, const uint8_t* text, uint64_t n_bytes, uint32_t flags, v2p_vcf_lines* out) {
-    if (!v || !out) return V2P_ERR_INVALID_ARG;
-    memset(out, 0, sizeof *out);
-    v->err.clear();
-    v->loaded = false;
-    if (flags & ~V2P_FLAG_DEVICE_PTRS) return vfail(v, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
-    if (n_bytes && !text) return vfail(v, V2P_ERR_INVALID_ARG, "text is NULL");
-    const bool dev = flags & V2P_FLAG_DEVICE_PTRS;
-    if (dev && ((uintptr_t)text & 15)) return vfail(v, V2P_ERR_INVALID_ARG, "device text must be 16-byte aligned");
-    CU(v, cudaSetDevice(v->device));
+// Index of v->text[0, n): line tables on the device, their host copies, n_lines / n_samples; the index kernels end
+// with `done` recorded.  h = the counters of the #CHROM line.
+int index_text(v2p_vcf* v, uint64_t n, cudaEvent_t done, LoadCtr& h) {
     cudaStream_t st = v->stream;
     int rc;
-    CU(v, cudaEventRecord(v->ev[0], st));
-    if (dev) {
-        v->text = text;
-    } else {
-        if ((rc = need(v, v->buf_text, n_bytes + 16))) return rc;
-        if (n_bytes) CU(v, cudaMemcpyAsync(v->buf_text.p, text, n_bytes, cudaMemcpyHostToDevice, st));
-        v->text = (const uint8_t*)v->buf_text.p;
-    }
-    CU(v, cudaEventRecord(v->ev[1], st));
-    const uint64_t n = n_bytes, n_tiles = (n + kTile - 1) / kTile;
-    LoadCtr h{0, kNone, 0, 0, 0};
+    const uint64_t n_tiles = (n + kTile - 1) / kTile;
+    h = LoadCtr{0, kNone, 0, 0, 0};
     if ((rc = need(v, v->ctr, sizeof(LoadCtr))) || (rc = need(v, v->tile_cnt, (n_tiles + 1) * 8)) ||
         (rc = need(v, v->tile_x, (n_tiles + 1) * 8)))
         return rc;
@@ -546,7 +540,7 @@ int v2p_vcf_load(v2p_vcf* v, const uint8_t* text, uint64_t n_bytes, uint32_t fla
             (uint8_t*)v->has_cells.p);
         CU(v, cudaGetLastError());
     }
-    CU(v, cudaEventRecord(v->ev[2], st));
+    CU(v, cudaEventRecord(done, st));
     static_assert(sizeof(LoadCtr) == 40, "LoadCtr is published as five 8-byte words");
     if ((rc = fetch(v, ctr, 5, &h))) return rc;
     if (h.chrom == kNone) return vfail(v, V2P_ERR_VCF_PARSE, "no #CHROM line: the number of samples is unknown");
@@ -557,12 +551,220 @@ int v2p_vcf_load(v2p_vcf* v, const uint8_t* text, uint64_t n_bytes, uint32_t fla
         CU(v, cudaMemcpyAsync(v->h_cells_begin.data(), v->cells_begin.p, v->n_lines * 8, cudaMemcpyDeviceToHost, st));
     }
     CU(v, cudaStreamSynchronize(st));
+    return V2P_OK;
+}
+
+void fill_lines(const v2p_vcf* v, const LoadCtr& h, v2p_vcf_lines* out) {
+    out->n_samples = v->n_samples, out->header_begin = h.hb, out->header_end = h.he, out->n_lines = v->n_lines;
+    out->line_begin = v->h_line_begin.data(), out->cells_begin = v->h_cells_begin.data();
+}
+
+constexpr uint64_t kBgzfMaxIsize = 65536;
+const char* const kBgzfWhat[] = {"", "bad BGZF block header", "invalid DEFLATE data",
+                                 "inflated size differs from the trailer's ISIZE", "CRC-32 differs from the trailer's"};
+
+inline uint32_t le16(const uint8_t* p) { return p[0] | (uint32_t)p[1] << 8; }
+inline uint32_t le32(const uint8_t* p) { return le16(p) | le16(p + 2) << 16; }
+
+// SAM spec 4.1 block headers from `d`: the block table (out_off = exclusive sum of ISIZE) and each block's file offset.
+// Stops at the first bad header: returns false with `why` set and its offset last in `at`; the blocks before it are in
+// the table.
+bool walk_bgzf(const uint8_t* d, uint64_t n, std::vector<BgzfBlock>& tab, std::vector<uint64_t>& at, uint64_t& text_bytes,
+               char* why, size_t why_len) {
+    tab.clear(), at.clear();
+    text_bytes = 0;
+    for (uint64_t o = 0; o < n;) {
+        const uint64_t left = n - o;
+        const uint8_t* h = d + o;
+        at.push_back(o);
+        if (left < 18) return snprintf(why, why_len, "%llu bytes left, a header takes 18", (unsigned long long)left), false;
+        if (h[0] != 31 || h[1] != 139 || h[2] != 8 || h[3] != 4)
+            return snprintf(why, why_len, "no gzip header with FEXTRA alone (not BGZF: recompress with bgzip)"), false;
+        const uint32_t xlen = le16(h + 10);
+        if (xlen < 6 || 12 + (uint64_t)xlen > left) return snprintf(why, why_len, "XLEN %u", xlen), false;
+        int64_t bsize = -1;
+        for (uint32_t x = 0; x + 4 <= xlen;) {
+            const uint32_t slen = le16(h + 12 + x + 2);
+            if (x + 4 + slen > xlen) break;
+            if (h[12 + x] == 'B' && h[12 + x + 1] == 'C' && slen == 2) bsize = le16(h + 12 + x + 4);
+            x += 4 + slen;
+        }
+        if (bsize < 0) return snprintf(why, why_len, "no BC subfield (not BGZF: recompress with bgzip)"), false;
+        const uint64_t total = (uint64_t)bsize + 1;
+        if (total < 12 + (uint64_t)xlen + 8 || total > left)
+            return snprintf(why, why_len, "BSIZE %lld with %llu bytes left", (long long)bsize, (unsigned long long)left), false;
+        const uint32_t isize = le32(h + total - 4);
+        if (isize > kBgzfMaxIsize) return snprintf(why, why_len, "ISIZE %u > 65536", isize), false;
+        BgzfBlock b{};
+        b.c_off = o + 12 + xlen, b.c_len = (uint32_t)(total - 12 - xlen - 8), b.out_off = text_bytes, b.isize = isize;
+        b.crc = le32(h + total - 8);
+        tab.push_back(b);
+        text_bytes += isize, o += total;
+    }
+    return true;
+}
+
+}  // namespace
+
+extern "C" {
+
+int v2p_vcf_create(int cuda_device, v2p_vcf** out) {
+    if (!out) return V2P_ERR_INVALID_ARG;
+    *out = nullptr;
+    v2p_vcf* v = new (std::nothrow) v2p_vcf();
+    if (!v) return V2P_ERR_INVALID_ARG;
+    v->device = cuda_device;
+    bool ok = cudaSetDevice(cuda_device) == cudaSuccess && cudaStreamCreateWithFlags(&v->stream, cudaStreamNonBlocking) == cudaSuccess &&
+              cudaDeviceGetAttribute(&v->sms, cudaDevAttrMultiProcessorCount, cuda_device) == cudaSuccess;
+    for (cudaEvent_t& e : v->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
+    if (ok) {
+        k_crc32_init<<<1, 256, 0, v->stream>>>();
+        ok = cudaStreamSynchronize(v->stream) == cudaSuccess;
+    }
+    if (!ok) {
+        v2p_vcf_destroy(v);
+        return V2P_ERR_CUDA;
+    }
+    *out = v;
+    return V2P_OK;
+}
+
+void v2p_vcf_destroy(v2p_vcf* v) {
+    if (!v) return;
+    cudaSetDevice(v->device);
+    if (v->stream) cudaStreamSynchronize(v->stream);
+    Buf* all[] = {&v->buf_text, &v->tile_cnt, &v->tile_x, &v->starts, &v->ends, &v->is_data, &v->data_x, &v->line_begin,
+                  &v->line_end, &v->line_no, &v->cells_begin, &v->has_cells, &v->ctr, &v->cub_tmp, &v->rec_line, &v->n_seg,
+                  &v->seg_begin, &v->seg_tabs, &v->seg_tab_x, &v->seg_err, &v->seg_rec, &v->masks, &v->comp, &v->blocks,
+                  &v->fixed_len, &v->fixed_x, &v->fixed};
+    for (Buf* b : all)
+        if (b->p) cudaFree(b->p);
+    for (HostBuf* b : {&v->h_head, &v->h_fixed, &v->h_fixed_begin})
+        if (b->p) cudaFreeHost(b->p);
+    v->pub.release();
+    for (cudaEvent_t e : v->ev)
+        if (e) cudaEventDestroy(e);
+    if (v->stream) cudaStreamDestroy(v->stream);
+    delete v;
+}
+
+const char* v2p_vcf_last_error(v2p_vcf* v) { return v ? v->err.c_str() : "vcf object is NULL"; }
+
+int v2p_vcf_load(v2p_vcf* v, const uint8_t* text, uint64_t n_bytes, uint32_t flags, v2p_vcf_lines* out) {
+    if (!v || !out) return V2P_ERR_INVALID_ARG;
+    memset(out, 0, sizeof *out);
+    v->err.clear();
+    v->loaded = false;
+    if (flags & ~V2P_FLAG_DEVICE_PTRS) return vfail(v, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
+    if (n_bytes && !text) return vfail(v, V2P_ERR_INVALID_ARG, "text is NULL");
+    const bool dev = flags & V2P_FLAG_DEVICE_PTRS;
+    if (dev && ((uintptr_t)text & 15)) return vfail(v, V2P_ERR_INVALID_ARG, "device text must be 16-byte aligned");
+    CU(v, cudaSetDevice(v->device));
+    cudaStream_t st = v->stream;
+    int rc;
+    CU(v, cudaEventRecord(v->ev[0], st));
+    if (dev) {
+        v->text = text;
+    } else {
+        if ((rc = need(v, v->buf_text, n_bytes + 16))) return rc;
+        if (n_bytes) CU(v, cudaMemcpyAsync(v->buf_text.p, text, n_bytes, cudaMemcpyHostToDevice, st));
+        v->text = (const uint8_t*)v->buf_text.p;
+    }
+    CU(v, cudaEventRecord(v->ev[1], st));
+    LoadCtr h;
+    if ((rc = index_text(v, n_bytes, v->ev[2], h))) return rc;
     float h2d = 0, idx = 0;
     CU(v, cudaEventElapsedTime(&h2d, v->ev[0], v->ev[1]));
     CU(v, cudaEventElapsedTime(&idx, v->ev[1], v->ev[2]));
-    out->n_samples = v->n_samples, out->header_begin = h.hb, out->header_end = h.he, out->n_lines = v->n_lines;
-    out->line_begin = v->h_line_begin.data(), out->cells_begin = v->h_cells_begin.data();
-    out->h2d_bytes = dev ? 0 : n, out->h2d_ms = h2d, out->index_ms = idx;
+    fill_lines(v, h, out);
+    out->h2d_bytes = dev ? 0 : n_bytes, out->h2d_ms = h2d, out->index_ms = idx;
+    v->loaded = true;
+    return V2P_OK;
+}
+
+int v2p_vcf_load_bgzf(v2p_vcf* v, const uint8_t* data, uint64_t n_bytes, uint32_t flags, v2p_vcf_lines* out, v2p_vcf_bgzf* bz) {
+    if (!v || !out || !bz) return V2P_ERR_INVALID_ARG;
+    memset(out, 0, sizeof *out);
+    memset(bz, 0, sizeof *bz);
+    v->err.clear();
+    v->loaded = false;
+    if (flags & V2P_FLAG_DEVICE_PTRS) return vfail(v, V2P_ERR_INVALID_ARG, "BGZF input must be host memory (V2P_FLAG_DEVICE_PTRS)");
+    if (flags) return vfail(v, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
+    if (n_bytes && !data) return vfail(v, V2P_ERR_INVALID_ARG, "data is NULL");
+    CU(v, cudaSetDevice(v->device));
+    cudaStream_t st = v->stream;
+    int rc;
+    // the upload runs while the host walks the block headers
+    CU(v, cudaEventRecord(v->ev[0], st));
+    if ((rc = need(v, v->comp, n_bytes + 16))) return rc;
+    if (n_bytes) CU(v, cudaMemcpyAsync(v->comp.p, data, n_bytes, cudaMemcpyHostToDevice, st));
+    CU(v, cudaEventRecord(v->ev[1], st));
+    std::vector<uint64_t> at;
+    uint64_t text_bytes = 0;
+    char why[160] = "";
+    const bool walked = walk_bgzf(data, n_bytes, v->h_blocks, at, text_bytes, why, sizeof why);
+    const uint64_t n_blk = v->h_blocks.size();
+    if ((rc = need(v, v->blocks, n_blk * sizeof(BgzfBlock))) || (rc = need(v, v->buf_text, text_bytes + 16)) ||
+        (rc = need(v, v->ctr, sizeof(LoadCtr))))
+        return rc;
+    if (n_blk) CU(v, cudaMemcpyAsync(v->blocks.p, v->h_blocks.data(), n_blk * sizeof(BgzfBlock), cudaMemcpyHostToDevice, st));
+    unsigned long long* ekey = (unsigned long long*)v->ctr.p;
+    CU(v, cudaMemsetAsync(ekey, 0xff, 8, st));
+    v->text = (const uint8_t*)v->buf_text.p;
+    CU(v, cudaEventRecord(v->ev[2], st));
+    if (n_blk) {
+        int per_sm = 1;
+        CU(v, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_inflate, kInfWarps * 32, 0));
+        const uint64_t grid = std::min<uint64_t>((uint64_t)v->sms * std::max(per_sm, 1), (n_blk + kInfWarps - 1) / kInfWarps);
+        k_inflate<<<(unsigned)grid, kInfWarps * 32, 0, st>>>((const uint8_t*)v->comp.p, (const BgzfBlock*)v->blocks.p, n_blk,
+                                                             (uint8_t*)v->buf_text.p, ekey);
+        CU(v, cudaGetLastError());
+    }
+    CU(v, cudaEventRecord(v->ev[3], st));
+    unsigned long long key = kNone;
+    if ((rc = fetch(v, ekey, 1, &key))) return rc;
+    // blocks before a bad header were inflated: a bad one among them comes first in file order
+    if (key != kNone || !walked) {
+        const uint64_t b = key != kNone ? key >> 3 : n_blk;
+        const unsigned cls = key != kNone ? (unsigned)(key & 7) : (unsigned)BGZF_HEADER;
+        const unsigned long long off = at[b];
+        if (cls == BGZF_HEADER)
+            return vfail(v, V2P_ERR_BGZF, "BGZF block %llu at byte %llu: %s (%s)", (unsigned long long)b, off, kBgzfWhat[cls], why);
+        return vfail(v, V2P_ERR_BGZF, "BGZF block %llu at byte %llu: %s", (unsigned long long)b, off, kBgzfWhat[cls]);
+    }
+    CU(v, cudaEventRecord(v->ev[4], st));
+    LoadCtr h;
+    if ((rc = index_text(v, text_bytes, v->ev[5], h))) return rc;
+    // columns 1-9 of every data line and the header lines back to the host
+    const uint64_t nl = v->n_lines;
+    uint64_t n_fixed = 0;
+    for (uint64_t l = 0; l < nl; ++l) n_fixed += v->h_cells_begin[l] - v->h_line_begin[l];
+    if ((rc = need(v, v->fixed_len, (nl + 1) * 8)) || (rc = need(v, v->fixed_x, (nl + 1) * 8)) || (rc = need(v, v->fixed, n_fixed)) ||
+        (rc = hneed(v, v->h_fixed_begin, (nl + 1) * 8)) || (rc = hneed(v, v->h_fixed, n_fixed)) || (rc = hneed(v, v->h_head, h.he)))
+        return rc;
+    const uint64_t* lb = (const uint64_t*)v->line_begin.p;
+    const uint64_t* cb = (const uint64_t*)v->cells_begin.p;
+    k_fixed_len<<<blocks(nl + 1), 256, 0, st>>>(lb, cb, nl, (uint64_t*)v->fixed_len.p);
+    if ((rc = xsum(v, (const uint64_t*)v->fixed_len.p, (uint64_t*)v->fixed_x.p, nl + 1))) return rc;
+    if (nl)
+        k_fixed<<<(unsigned)std::min<uint64_t>((nl + 7) / 8, (uint64_t)v->sms * 32), 256, 0, st>>>(v->text, lb, cb, (const uint64_t*)v->fixed_x.p,
+                                                                                                   nl, (uint8_t*)v->fixed.p);
+    CU(v, cudaGetLastError());
+    CU(v, cudaMemcpyAsync(v->h_fixed_begin.p, v->fixed_x.p, (nl + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (n_fixed) CU(v, cudaMemcpyAsync(v->h_fixed.p, v->fixed.p, n_fixed, cudaMemcpyDeviceToHost, st));
+    if (h.he) CU(v, cudaMemcpyAsync(v->h_head.p, v->text, h.he, cudaMemcpyDeviceToHost, st));
+    CU(v, cudaEventRecord(v->ev[6], st));
+    CU(v, cudaStreamSynchronize(st));
+    float h2d = 0, inf = 0, idx = 0, fix = 0;
+    CU(v, cudaEventElapsedTime(&h2d, v->ev[0], v->ev[1]));
+    CU(v, cudaEventElapsedTime(&inf, v->ev[2], v->ev[3]));
+    CU(v, cudaEventElapsedTime(&idx, v->ev[4], v->ev[5]));
+    CU(v, cudaEventElapsedTime(&fix, v->ev[5], v->ev[6]));
+    fill_lines(v, h, out);
+    out->h2d_bytes = n_bytes, out->h2d_ms = h2d, out->index_ms = idx;
+    bz->n_blocks = n_blk, bz->text_bytes = text_bytes, bz->text = v->text;
+    bz->head = (const uint8_t*)v->h_head.p, bz->fixed = (const uint8_t*)v->h_fixed.p, bz->fixed_begin = (const uint64_t*)v->h_fixed_begin.p;
+    bz->inflate_ms = inf, bz->fixed_ms = fix;
     v->loaded = true;
     return V2P_OK;
 }

@@ -30,6 +30,34 @@ class VcfIndex:
         return [c.decode() for c in self._header.split(b"\t")[9:]] if self.n_samples else []
 
 
+class BgzfVcfIndex(VcfIndex):
+    """What v2p_vcf_load_bgzf found: the VcfIndex of the inflated text (offsets are into that text), plus what the host
+    needs without a text of its own: `head` (every line up to and including #CHROM) and columns 1-9 of every data line
+    (`fixed_text`, sliced by `fixed_begin`).  The text itself stays on the device at `text_ptr` until the next load."""
+
+    def __init__(self, res: L.VcfLines, bz: L.VcfBgzf, owner: "DeviceVcf"):
+        self.head = C.string_at(bz.head, int(res.header_end)) if res.header_end else b""
+        super().__init__(res, self.head[int(res.header_begin):])
+        n = int(res.n_lines)
+        self.fixed_begin = np.ctypeslib.as_array(C.cast(bz.fixed_begin, C.POINTER(C.c_uint64)), shape=(n + 1,)).copy()
+        n_fixed = int(self.fixed_begin[-1])
+        self.fixed_text = np.frombuffer(C.string_at(bz.fixed, n_fixed), np.uint8).copy() if n_fixed else np.zeros(0, np.uint8)
+        self.text_ptr, self.text_bytes, self.n_blocks = int(bz.text or 0), int(bz.text_bytes), int(bz.n_blocks)
+        self.inflate_ms, self.fixed_ms = float(bz.inflate_ms), float(bz.fixed_ms)
+        self._owner = owner
+
+    def fixed(self, l: int) -> bytes:
+        """Columns 1-9 of data line l, with the tab after FORMAT when the line has sample cells."""
+        return self.fixed_text[int(self.fixed_begin[l]):int(self.fixed_begin[l + 1])].tobytes()
+
+    def read_text(self) -> bytes:
+        """Device -> host copy of the inflated text (tests, debugging); valid until the owner's next load."""
+        out = np.zeros(self.text_bytes, np.uint8)
+        if out.size and self._owner._lib.v2p_device_read(out.ctypes.data_as(C.c_void_p), C.c_void_p(self.text_ptr), out.nbytes):
+            raise EngineError(L.ERR_CUDA, "v2p_device_read failed")
+        return out.tobytes()
+
+
 class DeviceMasks:
     """masks[n_records][n_samples][words_per_cell] (uint32) on the device, owned by the DeviceVcf until its next call.
     `ptr` / `shape` go straight to DevicePipeline.run_masks(ptr, ..., shape=shape) and CohortRunner.run_masks."""
@@ -103,6 +131,17 @@ class DeviceVcf:
                 raise EngineError(L.ERR_CUDA, "reading the #CHROM line back failed")
             header = hdr.tobytes()
         return VcfIndex(res, header)
+
+    def load_bgzf(self, data: Union[bytes, np.ndarray]) -> BgzfVcfIndex:
+        """A bgzip'd VCF (bytes or a uint8 array in host memory; pinned memory uploads at the full PCIe rate), inflated
+        and indexed on the device.  parse_masks then works as after load()."""
+        buf = np.frombuffer(data, np.uint8) if isinstance(data, (bytes, bytearray, memoryview)) else np.ascontiguousarray(data, np.uint8)
+        res, bz = L.VcfLines(), L.VcfBgzf()
+        st = self._lib.v2p_vcf_load_bgzf(self._h, buf.ctypes.data_as(C.c_void_p), buf.nbytes, 0, C.byref(res), C.byref(bz))
+        self._text = None
+        if st:
+            raise EngineError(st, self._err())
+        return BgzfVcfIndex(res, bz, self)
 
     def parse_masks(self, rec_line: Sequence[int]) -> DeviceMasks:
         """Row r of the matrix = data line rec_line[r] of the last load (any order)."""
