@@ -95,6 +95,39 @@ def test_product_never_imports_oracle():
                 assert not pat.search(txt), "%s reaches into the oracle" % fn
 
 
+def _without_bodies(src, names):
+    """src with the definitions of the named functions cut out (from the name to the brace that closes the body)."""
+    for name in names:
+        m = re.search(r"\b%s\([^)]*\)\s*\{" % name, src)
+        assert m, "no definition of %s" % name
+        depth, i = 1, m.end()
+        while depth:
+            depth += {"{": 1, "}": -1}.get(src[i], 0)
+            i += 1
+        src = src[:m.start()] + src[i:]
+    return src
+
+
+def test_host_objects_share_one_buffer_and_error_implementation():
+    """Device and pinned memory is allocated and freed only by the owning buffer types of csrc/v2p_hostres.cuh and
+    csrc/v2p_mapped.cuh (whose destructors free it, so no destroy function keeps a list of buffers to forget one from)
+    and by the public v2p_host_alloc / v2p_host_free.  Error messages are formatted only in csrc/v2p_hostres.cuh."""
+    csrc = os.path.join(ROOT, "vcf2prot_b200", "csrc")
+    alloc = re.compile(r"\b(cudaMalloc\w*|cudaHostAlloc|cudaFree\w*)\s*\(")
+    fmt = re.compile(r"\bvsnprintf\s*\(")
+    names = sorted(fn for fn in os.listdir(csrc) if fn.endswith((".cu", ".cuh")))
+    assert "v2p_hostres.cuh" in names and "v2p_engine.cu" in names
+    for fn in names:
+        src = open(os.path.join(csrc, fn)).read()
+        if fn == "v2p_engine.cu":
+            src = _without_bodies(src, ("v2p_host_alloc", "v2p_host_free"))
+        if fn not in ("v2p_hostres.cuh", "v2p_mapped.cuh"):
+            m = alloc.search(src)
+            assert not m, "%s calls %s: use DevBuf / PinnedBuf (v2p_hostres.cuh) or MappedBuf" % (fn, m.group(1))
+        if fn != "v2p_hostres.cuh":
+            assert not fmt.search(src), "%s formats its own messages: use v2p::fail / v2p::vformat" % fn
+
+
 def test_dir_writer_sink_writes_one_file_per_proband(lib, tmp_path):
     """The ready-made sink of include/v2p_pipeline.h is host code (parts/io.rs:35-57 naming): no GPU needed."""
     import numpy as np

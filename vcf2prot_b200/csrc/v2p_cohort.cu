@@ -7,7 +7,6 @@
 #include <atomic>
 #include <chrono>
 #include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <mutex>
 #include <new>
@@ -16,6 +15,7 @@
 #include <vector>
 
 #include "v2p_cohort.h"
+#include "v2p_hostres.cuh"
 #include "v2p_taskgen.h"
 
 namespace {
@@ -39,15 +39,12 @@ struct v2p_cohort {
 namespace {
 
 int cofail(v2p_cohort* c, int code, const char* fmt, ...) {
-    char buf[768];
     va_list ap;
     va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
+    std::string msg = v2p::vformat(fmt, ap);
     va_end(ap);
-    if (c) {
-        std::lock_guard<std::mutex> g(c->err_mu);
-        if (c->err.empty()) c->err = buf;  // the first failure is the one reported
-    }
+    std::lock_guard<std::mutex> g(c->err_mu);
+    if (c->err.empty()) c->err = std::move(msg);  // the first failure is the one reported
     return code;
 }
 

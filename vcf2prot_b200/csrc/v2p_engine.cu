@@ -13,8 +13,6 @@
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
-#include <cstdarg>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -23,17 +21,13 @@
 #include <vector>
 
 #include "v2p_engine.h"
+#include "v2p_hostres.cuh"
 #include "v2p_kernels.cuh"
 #include "v2p_mapped.cuh"
 
 using namespace v2p;
 
 namespace {
-
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-};
 
 struct Scratch {  // per-stream planning scratch
     DevBuf lb, tile_hap, chunk_hap, order, status, hap_flags, ser_list;
@@ -54,9 +48,8 @@ struct SoaSlot {  // everything one in-flight single-haplotype call needs: nobod
     cudaStream_t stream = nullptr;
     Scratch sc;
     DevBuf d_soa[4], tasks, ref, alt, out, bases;
-    DevStatus* h_status = nullptr;  // pinned + mapped
-    uint8_t* h_stage = nullptr;     // pinned staging of the 1-byte tapes (ref | alt | res), grown on demand
-    size_t stage_cap = 0;
+    MappedBuf h_status;  // one DevStatus
+    PinnedBuf h_stage;   // staging of the 1-byte tapes (ref | alt | res), grown on demand
     bool busy = false;
 };
 
@@ -64,7 +57,7 @@ struct SoaSlot {  // everything one in-flight single-haplotype call needs: nobod
 
 struct v2p_event {
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_done = nullptr, ev_copy = nullptr;
-    DevStatus* h_status = nullptr;  // pinned; filled by a stream-ordered D2H right behind the launch group
+    MappedBuf h_status;             // one DevStatus, published right behind the launch group
     KParams kp;                     // for the deferred serial fallback
     cudaStream_t stream = nullptr;
     Slot* slot = nullptr;  // host-pointer mode
@@ -110,43 +103,6 @@ namespace {
 // worker in the reference, parts/exec.rs:36-39), and a shared string could be overwritten under the reader's eyes.
 thread_local std::string t_err;
 
-int fail(v2p_engine* e, int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    (void)e;
-    t_err = buf;
-    return code;
-}
-
-#define CUDA_TRY(e, call)                                                                                   \
-    do {                                                                                                    \
-        cudaError_t _st = (call);                                                                           \
-        if (_st != cudaSuccess)                                                                             \
-            return fail((e), V2P_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_st), __FILE__, \
-                        __LINE__);                                                                          \
-    } while (0)
-
-int reserve(v2p_engine* e, DevBuf& b, size_t bytes) {
-    bytes = std::max<size_t>(bytes, 256);
-    if (b.cap >= bytes) return V2P_OK;
-    if (b.p) CUDA_TRY(e, cudaFree(b.p));
-    b.p = nullptr;
-    b.cap = 0;
-    size_t want = bytes + bytes / 8 + 256;
-    CUDA_TRY(e, cudaMalloc(&b.p, want));
-    b.cap = want;
-    return V2P_OK;
-}
-
-void release(DevBuf& b) {
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr;
-    b.cap = 0;
-}
-
 // Copy-kernel variants selectable through v2p_engine_set_tuning (profiling sweeps); 0 is the shipped default.
 struct CopyVariant {
     int tile;
@@ -178,22 +134,21 @@ int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, KParams& kp, cudaEv
     kp.tile_bytes = (uint32_t)T;
     kp.tile_shift = T == 8192 ? 13u : T == 4096 ? 12u : 11u;
     kp.n_tiles = (kp.n_out + T - 1) / T;
-    if (kp.n_tasks >= 0xFFFFFFFEull) return fail(e, V2P_ERR_INVALID_ARG, "more than 2^32-2 tasks in one launch");
-    if (kp.n_hap >= 0x80000000ull) return fail(e, V2P_ERR_INVALID_ARG, "more than 2^31 haplotypes in one launch");  // bit 31 of tile_hap[] is a flag
-    int rc;
-    if ((rc = reserve(e, sc.lb, (kp.n_tiles + 1) * sizeof(uint32_t)))) return rc;
-    if ((rc = reserve(e, sc.tile_hap, std::max<uint64_t>(kp.n_tiles, 1) * sizeof(uint32_t)))) return rc;
-    if ((rc = reserve(e, sc.status, sizeof(DevStatus)))) return rc;
+    if (kp.n_tasks >= 0xFFFFFFFEull) return fail(t_err, V2P_ERR_INVALID_ARG, "more than 2^32-2 tasks in one launch");
+    if (kp.n_hap >= 0x80000000ull) return fail(t_err, V2P_ERR_INVALID_ARG, "more than 2^31 haplotypes in one launch");  // bit 31 of tile_hap[] is a flag
+    CU(t_err, sc.lb.need((kp.n_tiles + 1) * sizeof(uint32_t)));
+    CU(t_err, sc.tile_hap.need(std::max<uint64_t>(kp.n_tiles, 1) * sizeof(uint32_t)));
+    CU(t_err, sc.status.need(sizeof(DevStatus)));
     const uint64_t n_chunks = (kp.n_tasks + kPlanWarpTasks - 1) / kPlanWarpTasks;
-    if ((rc = reserve(e, sc.chunk_hap, std::max<uint64_t>(n_chunks, 1) * sizeof(uint32_t)))) return rc;
+    CU(t_err, sc.chunk_hap.need(std::max<uint64_t>(n_chunks, 1) * sizeof(uint32_t)));
     kp.chunk_hap = (uint32_t*)sc.chunk_hap.p;
     // per-haplotype "needs serial order" flags (+ one counter word behind them) and the compacted list of those
-    if ((rc = reserve(e, sc.hap_flags, (kp.n_hap + 1) * sizeof(uint32_t)))) return rc;
-    if ((rc = reserve(e, sc.ser_list, std::max<uint64_t>(kp.n_hap, 1) * sizeof(uint32_t)))) return rc;
+    CU(t_err, sc.hap_flags.need((kp.n_hap + 1) * sizeof(uint32_t)));
+    CU(t_err, sc.ser_list.need(std::max<uint64_t>(kp.n_hap, 1) * sizeof(uint32_t)));
     kp.hap_flags = (uint32_t*)sc.hap_flags.p;
     kp.ser_list = (uint32_t*)sc.ser_list.p;
     // tile order: 16-byte header (s_max) + one slot per (tile rank within its haplotype, haplotype)
-    if (kp.n_tiles >= 0xFFF00000ull) return fail(e, V2P_ERR_INVALID_ARG, "more than 2^32 tiles in one launch");
+    if (kp.n_tiles >= 0xFFF00000ull) return fail(t_err, V2P_ERR_INVALID_ARG, "more than 2^32 tiles in one launch");
     // tape order = identity over n_tiles (n_hap "1"): the cap then only has to hold the identity
     // Tile order: haplotype-interleaved (DESIGN.md section 4) unless the caller says the layout is phase-aligned
     // (V2P_FLAG_ALIGNED_LAYOUT: every run then comes from the one plain tape and tape order is ~3 % faster).
@@ -201,18 +156,18 @@ int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, KParams& kp, cudaEv
     kp.order_gshift = (uint32_t)e->order_gshift;
     const uint64_t order_cap =
         interleave ? std::min<uint64_t>(2 * kp.n_tiles + ((kp.n_hap + 64) << kp.order_gshift), 0xFFF00000ull) : 0;
-    if ((rc = reserve(e, sc.order, 16 + order_cap * sizeof(uint32_t)))) return rc;
+    CU(t_err, sc.order.need(16 + order_cap * sizeof(uint32_t)));
     kp.order_hdr = (uint32_t*)sc.order.p;
     kp.order = kp.order_hdr + 4;
     kp.order_cap = order_cap;
     kp.lb = (uint32_t*)sc.lb.p;
     kp.tile_hap = (uint32_t*)sc.tile_hap.p;
     kp.status = (DevStatus*)sc.status.p;
-    if (ev_start) CUDA_TRY(e, cudaEventRecord(ev_start, s));
-    CUDA_TRY(e, cudaMemsetAsync(kp.lb, 0xFF, (kp.n_tiles + 1) * sizeof(uint32_t), s));
-    CUDA_TRY(e, cudaMemsetAsync(kp.order_hdr, 0, 16, s));
-    CUDA_TRY(e, cudaMemsetAsync(kp.hap_flags, 0, (kp.n_hap + 1) * sizeof(uint32_t), s));
-    if (order_cap) CUDA_TRY(e, cudaMemsetAsync(kp.order, 0xFF, order_cap * sizeof(uint32_t), s));
+    if (ev_start) CU(t_err, cudaEventRecord(ev_start, s));
+    CU(t_err, cudaMemsetAsync(kp.lb, 0xFF, (kp.n_tiles + 1) * sizeof(uint32_t), s));
+    CU(t_err, cudaMemsetAsync(kp.order_hdr, 0, 16, s));
+    CU(t_err, cudaMemsetAsync(kp.hap_flags, 0, (kp.n_hap + 1) * sizeof(uint32_t), s));
+    if (order_cap) CU(t_err, cudaMemsetAsync(kp.order, 0xFF, order_cap * sizeof(uint32_t), s));
     if (init_status) {
         k_init_status<<<1, 1, 0, s>>>(kp.status);
         e->launches++;
@@ -233,7 +188,7 @@ int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, KParams& kp, cudaEv
         k_plan_fix<<<(unsigned)((kp.n_hap + 255) / 256), 256, 0, s>>>(kp, kp.hap_flags + kp.n_hap);
         e->launches++;
     }
-    if (ev_copy) CUDA_TRY(e, cudaEventRecord(ev_copy, s));
+    if (ev_copy) CU(t_err, cudaEventRecord(ev_copy, s));
     if (kp.n_tiles) {
         const int per_sm = e->ctas_per_sm > 0 ? e->ctas_per_sm : cv.ctas_per_sm;
         uint64_t want = (kp.n_tiles + kWarpsPerCta - 1) / kWarpsPerCta;
@@ -241,21 +196,21 @@ int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, KParams& kp, cudaEv
         size_t smem = (size_t)kWarpsPerCta * (cv.tile + cv.tile / 16 + kTileScratch) + 17 * 16;
         kp.warp_ns = nullptr;
         if (e->profile_warps && s == e->stream) {
-            if ((rc = reserve(e, e->warp_ns, (size_t)grid * kWarpsPerCta * sizeof(unsigned long long)))) return rc;
+            CU(t_err, e->warp_ns.need((size_t)grid * kWarpsPerCta * sizeof(unsigned long long)));
             kp.warp_ns = (unsigned long long*)e->warp_ns.p;
             e->warp_ns_n = grid * kWarpsPerCta;
         }
         void (*fn)(const KParams) = interleave ? cv.fn_il : cv.fn;
-        if (smem > 48 * 1024) CUDA_TRY(e, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 48 * 1024) CU(t_err, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         fn<<<grid, kThreads, smem, s>>>(kp);
         e->launches++;
     }
-    if (ev_stop) CUDA_TRY(e, cudaEventRecord(ev_stop, s));
-    CUDA_TRY(e, cudaGetLastError());
+    if (ev_stop) CU(t_err, cudaEventRecord(ev_stop, s));
+    CU(t_err, cudaGetLastError());
     // status rides the stream right behind the kernels, so a later launch cannot overwrite it first; it is stored
     // into mapped pinned memory by a kernel (v2p_mapped.cuh) so it never queues behind a result tape on the copy engine
     static_assert(sizeof(DevStatus) == 32, "DevStatus is published as four 8-byte words");
-    CUDA_TRY(e, publish_words(reinterpret_cast<unsigned long long*>(h_status), kp.status, 4, s));
+    CU(t_err, publish_words(reinterpret_cast<unsigned long long*>(h_status), kp.status, 4, s));
     e->launches++;
     return V2P_OK;
 }
@@ -310,7 +265,7 @@ int launch_serial(v2p_engine* e, cudaStream_t s, const KParams& kp, uint32_t n_s
     unsigned grid = (unsigned)e->sm_count * 4;
     k_serial<<<grid, kSerialThreads, 0, s>>>(kp, n_ser);
     e->launches++;
-    CUDA_TRY(e, cudaGetLastError());
+    CU(t_err, cudaGetLastError());
     return V2P_OK;
 }
 
@@ -319,7 +274,6 @@ void free_event(v2p_event* ev) {
     if (ev->ev_stop) cudaEventDestroy(ev->ev_stop);
     if (ev->ev_done) cudaEventDestroy(ev->ev_done);
     if (ev->ev_copy) cudaEventDestroy(ev->ev_copy);
-    if (ev->h_status) cudaFreeHost(ev->h_status);
     delete ev;
 }
 
@@ -344,7 +298,7 @@ v2p_event* acquire_event(v2p_engine* e) {
     if (cudaEventCreate(&ev->ev_start) != cudaSuccess || cudaEventCreate(&ev->ev_stop) != cudaSuccess ||
         cudaEventCreate(&ev->ev_copy) != cudaSuccess ||
         cudaEventCreateWithFlags(&ev->ev_done, cudaEventDisableTiming) != cudaSuccess ||
-        cudaHostAlloc((void**)&ev->h_status, sizeof(DevStatus), cudaHostAllocMapped | cudaHostAllocPortable) != cudaSuccess) {
+        ev->h_status.reserve(4) != cudaSuccess) {
         free_event(ev);
         return nullptr;
     }
@@ -362,16 +316,16 @@ int wait_locked(v2p_engine* e, v2p_event* ev, v2p_result* res) {
     };
     cudaSetDevice(e->device);
     if (cudaEventSynchronize(ev->ev_done) != cudaSuccess)
-        return finish(fail(e, V2P_ERR_CUDA, "launch group failed: %s", cudaGetErrorString(cudaGetLastError())));
-    const DevStatus& st = *ev->h_status;
+        return finish(fail(t_err, V2P_ERR_CUDA, "launch group failed: %s", cudaGetErrorString(cudaGetLastError())));
+    const DevStatus& st = *reinterpret_cast<const DevStatus*>(ev->h_status.p);
     if (needs_serial(st)) {
         int rc = launch_serial(e, ev->stream, ev->kp, st.unsorted);
         if (rc) return finish(rc);
         if (ev->slot && ev->out_bytes &&
             cudaMemcpyAsync(ev->h_out, ev->kp.out, ev->out_bytes, cudaMemcpyDeviceToHost, ev->stream) != cudaSuccess)
-            return finish(fail(e, V2P_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(cudaGetLastError())));
+            return finish(fail(t_err, V2P_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(cudaGetLastError())));
         if (cudaStreamSynchronize(ev->stream) != cudaSuccess)
-            return finish(fail(e, V2P_ERR_CUDA, "serial-order kernel failed: %s", cudaGetErrorString(cudaGetLastError())));
+            return finish(fail(t_err, V2P_ERR_CUDA, "serial-order kernel failed: %s", cudaGetErrorString(cudaGetLastError())));
     }
     std::vector<uint64_t> tb_copy;
     const uint64_t* tb = ev->h_task_begin;
@@ -386,7 +340,7 @@ int wait_locked(v2p_engine* e, v2p_event* ev, v2p_result* res) {
     if (cudaEventElapsedTime(&ms, ev->ev_start, ev->ev_stop) == cudaSuccess) local.kernel_ms = ms;
     if (cudaEventElapsedTime(&ms, ev->ev_copy, ev->ev_stop) == cudaSuccess) local.copy_ms = ms;
     if (local.status != V2P_OK)
-        fail(e, local.status, "haplotype %llu task %llu rejected with status %d", (unsigned long long)local.bad_hap,
+        fail(t_err, local.status, "haplotype %llu task %llu rejected with status %d", (unsigned long long)local.bad_hap,
              (unsigned long long)local.bad_task, local.status);
     return finish(local.status);
 }
@@ -437,25 +391,13 @@ void v2p_engine_destroy(v2p_engine* e) {
     if (!e) return;
     cudaSetDevice(e->device);
     cudaDeviceSynchronize();
-    DevBuf* bufs[] = {&e->warp_ns, &e->sc.hap_flags, &e->sc.ser_list, &e->sc.order, &e->sc.chunk_hap, &e->sc.lb, &e->sc.tile_hap, &e->sc.status, &e->ref_rep};
-    for (DevBuf* b : bufs) release(*b);
-    for (SoaSlot& sl : e->soa) {
-        DevBuf* sb[] = {&sl.sc.hap_flags, &sl.sc.ser_list, &sl.sc.order, &sl.sc.chunk_hap, &sl.sc.lb, &sl.sc.tile_hap, &sl.sc.status,
-                        &sl.d_soa[0], &sl.d_soa[1], &sl.d_soa[2], &sl.d_soa[3], &sl.tasks, &sl.ref, &sl.alt, &sl.out, &sl.bases};
-        for (DevBuf* b : sb) release(*b);
-        if (sl.h_status) cudaFreeHost(sl.h_status);
-        if (sl.h_stage) cudaFreeHost(sl.h_stage);
+    for (SoaSlot& sl : e->soa)
         if (sl.stream) cudaStreamDestroy(sl.stream);
-    }
-    for (Slot& sl : e->slots) {
-        DevBuf* sb[] = {&sl.sc.hap_flags, &sl.sc.ser_list, &sl.sc.order, &sl.sc.chunk_hap, &sl.sc.lb,      &sl.sc.tile_hap, &sl.sc.status,  &sl.d_tasks, &sl.d_task_begin, &sl.d_ref,
-                        &sl.d_ref_base, &sl.d_alt,       &sl.d_alt_base, &sl.d_out,   &sl.d_out_base};
-        for (DevBuf* b : sb) release(*b);
+    for (Slot& sl : e->slots)
         if (sl.stream) cudaStreamDestroy(sl.stream);
-    }
     for (v2p_event* ev : e->event_pool) free_event(ev);
     if (e->own_stream && e->stream) cudaStreamDestroy(e->stream);
-    delete e;
+    delete e;  // frees every buffer
 }
 
 const char* v2p_last_error(v2p_engine* e) { return e ? t_err.c_str() : "engine is NULL"; }
@@ -488,9 +430,9 @@ int v2p_engine_read_warp_ns(v2p_engine* e, uint64_t* ns_out, uint64_t cap, uint6
     std::lock_guard<std::mutex> g(e->mu);
     *n_warps = e->warp_ns_n;
     if (!ns_out || cap < e->warp_ns_n || !e->warp_ns_n) return e->warp_ns_n && ns_out ? V2P_ERR_INVALID_ARG : V2P_OK;
-    CUDA_TRY(e, cudaSetDevice(e->device));
-    CUDA_TRY(e, cudaStreamSynchronize(e->stream));
-    CUDA_TRY(e, cudaMemcpy(ns_out, e->warp_ns.p, (size_t)e->warp_ns_n * 8, cudaMemcpyDeviceToHost));
+    CU(t_err, cudaSetDevice(e->device));
+    CU(t_err, cudaStreamSynchronize(e->stream));
+    CU(t_err, cudaMemcpy(ns_out, e->warp_ns.p, (size_t)e->warp_ns_n * 8, cudaMemcpyDeviceToHost));
     return V2P_OK;
 }
 
@@ -514,27 +456,26 @@ int v2p_engine_set_reference(v2p_engine* e, const uint8_t* ref, uint64_t n_ref, 
     if (!e || (n_ref && !ref)) return V2P_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> g(e->mu);
     t_err.clear();
-    CUDA_TRY(e, cudaSetDevice(e->device));
-    CUDA_TRY(e, cudaDeviceSynchronize());  // nothing in flight may still read the previous tape
+    CU(t_err, cudaSetDevice(e->device));
+    CU(t_err, cudaDeviceSynchronize());  // nothing in flight may still read the previous tape
     e->has_ref = false;
     const bool replicas = (flags & V2P_REF_NO_TMA) == 0;
     const uint64_t stride = (n_ref + 64 + 255) & ~255ull;
     const uint64_t bytes = (replicas ? 16 : 1) * stride + 256;
-    int rc = reserve(e, e->ref_rep, bytes);
-    if (rc) return rc;
+    CU(t_err, e->ref_rep.need(bytes));
     uint8_t* rep = (uint8_t*)e->ref_rep.p;
-    CUDA_TRY(e, cudaMemsetAsync(rep, 0, bytes, e->stream));
+    CU(t_err, cudaMemsetAsync(rep, 0, bytes, e->stream));
     if (n_ref) {
-        CUDA_TRY(e, cudaMemcpyAsync(rep, ref, n_ref,
+        CU(t_err, cudaMemcpyAsync(rep, ref, n_ref,
                                     (flags & V2P_FLAG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
                                     e->stream));
         if (replicas) {
             k_build_replicas<<<(unsigned)((n_ref + 255) / 256), 256, 0, e->stream>>>(rep, n_ref, rep, stride);
             e->launches++;
-            CUDA_TRY(e, cudaGetLastError());
+            CU(t_err, cudaGetLastError());
         }
     }
-    CUDA_TRY(e, cudaStreamSynchronize(e->stream));
+    CU(t_err, cudaStreamSynchronize(e->stream));
     e->ref_tma_mode = replicas ? 1 : 0;
     e->rep_stride = stride;
     e->reg_n_ref = n_ref;
@@ -547,20 +488,20 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
     if (!e) return V2P_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> g(e->mu);
     t_err.clear();
-    if (!b) return fail(e, V2P_ERR_INVALID_ARG, "batch is NULL");
+    if (!b) return fail(t_err, V2P_ERR_INVALID_ARG, "batch is NULL");
     if (b->n_hap && (!b->task_begin || !b->alt_base || !b->out_base))
-        return fail(e, V2P_ERR_INVALID_ARG, "task_begin/alt_base/out_base must not be NULL");
+        return fail(t_err, V2P_ERR_INVALID_ARG, "task_begin/alt_base/out_base must not be NULL");
     const bool async = (flags & V2P_FLAG_ASYNC) != 0;
-    if (async && !done) return fail(e, V2P_ERR_INVALID_ARG, "ASYNC needs an event out-pointer");
-    if (!async && !res) return fail(e, V2P_ERR_INVALID_ARG, "synchronous call needs a result out-pointer");
-    CUDA_TRY(e, cudaSetDevice(e->device));
+    if (async && !done) return fail(t_err, V2P_ERR_INVALID_ARG, "ASYNC needs an event out-pointer");
+    if (!async && !res) return fail(t_err, V2P_ERR_INVALID_ARG, "synchronous call needs a result out-pointer");
+    CU(t_err, cudaSetDevice(e->device));
     if (res) memset(res, 0, sizeof *res);
     const bool use_reg_ref = b->ref == nullptr && b->ref_base == nullptr;
     if (use_reg_ref && !e->has_ref)
-        return fail(e, V2P_ERR_INVALID_ARG, "ref == NULL but no reference was registered (v2p_engine_set_reference)");
+        return fail(t_err, V2P_ERR_INVALID_ARG, "ref == NULL but no reference was registered (v2p_engine_set_reference)");
 
     v2p_event* ev = acquire_event(e);
-    if (!ev) return fail(e, V2P_ERR_CUDA, "event/pinned allocation failed");
+    if (!ev) return fail(t_err, V2P_ERR_CUDA, "event/pinned allocation failed");
     auto bail = [&](int code) {
         destroy_event(e, ev);
         return code;
@@ -576,7 +517,7 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
     int rc;
 
     if (flags & V2P_FLAG_DEVICE_PTRS) {
-        if (((uintptr_t)b->out & 15u) != 0) return bail(fail(e, V2P_ERR_INVALID_ARG, "out must be 16-byte aligned"));
+        if (((uintptr_t)b->out & 15u) != 0) return bail(fail(t_err, V2P_ERR_INVALID_ARG, "out must be 16-byte aligned"));
         kp.tasks = b->tasks;
         kp.task_begin = b->task_begin;
         kp.ref = b->ref;
@@ -593,7 +534,7 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
         // host pointers: stage through the next slot's device buffers on that slot's stream
         Slot* sl = &e->slots[e->next_slot];
         if (sl->busy)
-            return bail(fail(e, V2P_ERR_INVALID_ARG,
+            return bail(fail(t_err, V2P_ERR_INVALID_ARG,
                              "%d host-pointer batches already in flight: wait for the oldest event first", kSlots));
         const uint64_t H = b->n_hap;
         const uint64_t t0 = H ? b->task_begin[0] : 0, t1 = H ? b->task_begin[H] : 0;
@@ -601,7 +542,7 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
         const uint64_t o0 = H ? b->out_base[0] : 0, o1 = H ? b->out_base[H] : 0;
         uint64_t r0 = 0, r1 = use_reg_ref ? 0 : b->n_ref;
         if (b->ref_base && H) r0 = b->ref_base[0], r1 = b->ref_base[H];
-        if (t1 < t0 || a1 < a0 || o1 < o0 || r1 < r0) return bail(fail(e, V2P_ERR_INVALID_ARG, "base arrays not monotone"));
+        if (t1 < t0 || a1 < a0 || o1 < o0 || r1 < r0) return bail(fail(t_err, V2P_ERR_INVALID_ARG, "base arrays not monotone"));
         kp.n_tasks = t1 - t0;
         kp.n_alt = a1 - a0;
         kp.n_out = o1 - o0;
@@ -611,13 +552,20 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
         kp.out_origin = o0;
         kp.ref_origin = r0;
         if ((kp.n_tasks && !b->tasks) || (kp.n_out && !b->out) || (kp.n_ref && !b->ref) || (kp.n_alt && !b->alt))
-            return bail(fail(e, V2P_ERR_INVALID_ARG, "NULL data pointer"));
+            return bail(fail(t_err, V2P_ERR_INVALID_ARG, "NULL data pointer"));
         const size_t nb = (H + 1) * sizeof(uint64_t);
-        if ((rc = reserve(e, sl->d_tasks, kp.n_tasks * sizeof(v2p_task16))) || (rc = reserve(e, sl->d_task_begin, nb)) ||
-            (rc = reserve(e, sl->d_ref, kp.n_ref + 32)) || (rc = reserve(e, sl->d_ref_base, nb)) ||
-            (rc = reserve(e, sl->d_alt, kp.n_alt + 32)) || (rc = reserve(e, sl->d_alt_base, nb)) ||
-            (rc = reserve(e, sl->d_out, kp.n_out + 32)) || (rc = reserve(e, sl->d_out_base, nb)))
-            return bail(rc);
+        auto stage = [&]() -> int {
+            CU(t_err, sl->d_tasks.need(kp.n_tasks * sizeof(v2p_task16)));
+            CU(t_err, sl->d_task_begin.need(nb));
+            CU(t_err, sl->d_ref.need(kp.n_ref + 32));
+            CU(t_err, sl->d_ref_base.need(nb));
+            CU(t_err, sl->d_alt.need(kp.n_alt + 32));
+            CU(t_err, sl->d_alt_base.need(nb));
+            CU(t_err, sl->d_out.need(kp.n_out + 32));
+            CU(t_err, sl->d_out_base.need(nb));
+            return V2P_OK;
+        };
+        if ((rc = stage())) return bail(rc);
         s = sl->stream;
         sc = &sl->sc;
         auto h2d = [&](void* d, const void* h, size_t n) {
@@ -629,7 +577,7 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
             (b->ref_base && h2d(sl->d_ref_base.p, b->ref_base, nb) != cudaSuccess) ||
             h2d(sl->d_alt.p, b->alt + a0, kp.n_alt) != cudaSuccess || h2d(sl->d_alt_base.p, b->alt_base, nb) != cudaSuccess ||
             h2d(sl->d_out_base.p, b->out_base, nb) != cudaSuccess)
-            return bail(fail(e, V2P_ERR_CUDA, "H2D failed: %s", cudaGetErrorString(cudaGetLastError())));
+            return bail(fail(t_err, V2P_ERR_CUDA, "H2D failed: %s", cudaGetErrorString(cudaGetLastError())));
         kp.tasks = (const v2p_task16*)sl->d_tasks.p;
         kp.task_begin = (const uint64_t*)sl->d_task_begin.p;
         kp.ref = (const uint8_t*)sl->d_ref.p;
@@ -655,15 +603,15 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
         kp.tma_mode = e->ref_tma_mode;
     }
     ev->stream = s;
-    rc = launch_group(e, s, *sc, kp, ev->ev_start, ev->ev_stop, ev->h_status, true, ev->ev_copy,
+    rc = launch_group(e, s, *sc, kp, ev->ev_start, ev->ev_stop, reinterpret_cast<DevStatus*>(ev->h_status.p), true, ev->ev_copy,
                       (flags & V2P_FLAG_ALIGNED_LAYOUT) != 0);
     if (rc) return bail(rc);
     // host mode: the copy-back is enqueued right away (a batch that needs the serial-order kernel repeats it later)
     if (ev->slot && ev->out_bytes &&
         cudaMemcpyAsync(ev->h_out, kp.out, ev->out_bytes, cudaMemcpyDeviceToHost, s) != cudaSuccess)
-        return bail(fail(e, V2P_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(cudaGetLastError())));
+        return bail(fail(t_err, V2P_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(cudaGetLastError())));
     if (cudaEventRecord(ev->ev_done, s) != cudaSuccess)
-        return bail(fail(e, V2P_ERR_CUDA, "event record failed: %s", cudaGetErrorString(cudaGetLastError())));
+        return bail(fail(t_err, V2P_ERR_CUDA, "event record failed: %s", cudaGetErrorString(cudaGetLastError())));
     ev->kp = kp;
     if (async) {
         *done = ev;
@@ -725,50 +673,45 @@ void widen_u8(const uint8_t* __restrict__ src, uint32_t* __restrict__ dst, size_
 int soa_run(v2p_engine* e, SoaSlot* sl, size_t n_tasks, const uint64_t* exec_code, const uint64_t* start_pos,
             const uint64_t* length, const uint64_t* start_pos_res, const uint32_t* ref_utf32, size_t n_ref,
             const uint32_t* alt_utf32, size_t n_alt, uint32_t* res_utf32, size_t n_res, uint32_t flags, uint64_t* bad_index) {
-    CUDA_TRY(e, cudaSetDevice(e->device));
-    if (!sl->stream) CUDA_TRY(e, cudaStreamCreateWithFlags(&sl->stream, cudaStreamNonBlocking));
-    if (!sl->h_status)
-        CUDA_TRY(e, cudaHostAlloc((void**)&sl->h_status, sizeof(DevStatus), cudaHostAllocMapped | cudaHostAllocPortable));
+    CU(t_err, cudaSetDevice(e->device));
+    if (!sl->stream) CU(t_err, cudaStreamCreateWithFlags(&sl->stream, cudaStreamNonBlocking));
+    CU(t_err, sl->h_status.reserve(4));
+    DevStatus* const h_status = reinterpret_cast<DevStatus*>(sl->h_status.p);
     cudaStream_t s = sl->stream;
     const bool keep = !(flags & V2P_FLAG_FILL_DOT);
     int rc;
     // ---- narrow the tapes into pinned staging (ref | alt | res), unless a residue needs more than a byte
-    const size_t stage_need = n_ref + n_alt + n_res + 64;
-    if (sl->stage_cap < stage_need) {
-        if (sl->h_stage) CUDA_TRY(e, cudaFreeHost(sl->h_stage));
-        sl->h_stage = nullptr, sl->stage_cap = 0;
-        CUDA_TRY(e, cudaHostAlloc((void**)&sl->h_stage, stage_need + stage_need / 4, cudaHostAllocPortable));
-        sl->stage_cap = stage_need + stage_need / 4;
-    }
-    uint8_t* const h_ref = sl->h_stage;
+    CU(t_err, sl->h_stage.need(n_ref + n_alt + n_res + 64));
+    uint8_t* const h_ref = (uint8_t*)sl->h_stage.p;
     uint8_t* const h_alt = h_ref + n_ref;
     uint8_t* const h_res = h_alt + n_alt;
     uint32_t wide = narrow_u32(ref_utf32, h_ref, n_ref) | narrow_u32(alt_utf32, h_alt, n_alt);
     if (keep) wide |= narrow_u32(res_utf32, h_res, n_res);
     const uint32_t unit = wide > 0xFFu ? 4u : 1u;  // bytes per residue on the device
     const size_t tb = n_tasks * sizeof(uint64_t);
-    for (int i = 0; i < 4; ++i)
-        if ((rc = reserve(e, sl->d_soa[i], tb))) return rc;
-    if ((rc = reserve(e, sl->tasks, n_tasks * sizeof(v2p_task16))) || (rc = reserve(e, sl->ref, n_ref * unit + 32)) ||
-        (rc = reserve(e, sl->alt, n_alt * unit + 32)) || (rc = reserve(e, sl->out, n_res * unit + 32)) ||
-        (rc = reserve(e, sl->bases, 64)) || (rc = reserve(e, sl->sc.status, sizeof(DevStatus))))
-        return rc;
+    for (int i = 0; i < 4; ++i) CU(t_err, sl->d_soa[i].need(tb));
+    CU(t_err, sl->tasks.need(n_tasks * sizeof(v2p_task16)));
+    CU(t_err, sl->ref.need(n_ref * unit + 32));
+    CU(t_err, sl->alt.need(n_alt * unit + 32));
+    CU(t_err, sl->out.need(n_res * unit + 32));
+    CU(t_err, sl->bases.need(64));
+    CU(t_err, sl->sc.status.need(sizeof(DevStatus)));
     const uint64_t* soa[4] = {exec_code, start_pos, length, start_pos_res};
     for (int i = 0; i < 4; ++i)
-        if (tb) CUDA_TRY(e, cudaMemcpyAsync(sl->d_soa[i].p, soa[i], tb, cudaMemcpyHostToDevice, s));
+        if (tb) CU(t_err, cudaMemcpyAsync(sl->d_soa[i].p, soa[i], tb, cudaMemcpyHostToDevice, s));
     if (unit == 1) {
-        if (n_ref) CUDA_TRY(e, cudaMemcpyAsync(sl->ref.p, h_ref, n_ref, cudaMemcpyHostToDevice, s));
-        if (n_alt) CUDA_TRY(e, cudaMemcpyAsync(sl->alt.p, h_alt, n_alt, cudaMemcpyHostToDevice, s));
-        if (keep && n_res) CUDA_TRY(e, cudaMemcpyAsync(sl->out.p, h_res, n_res, cudaMemcpyHostToDevice, s));
+        if (n_ref) CU(t_err, cudaMemcpyAsync(sl->ref.p, h_ref, n_ref, cudaMemcpyHostToDevice, s));
+        if (n_alt) CU(t_err, cudaMemcpyAsync(sl->alt.p, h_alt, n_alt, cudaMemcpyHostToDevice, s));
+        if (keep && n_res) CU(t_err, cudaMemcpyAsync(sl->out.p, h_res, n_res, cudaMemcpyHostToDevice, s));
     } else {
-        if (n_ref) CUDA_TRY(e, cudaMemcpyAsync(sl->ref.p, ref_utf32, n_ref * 4, cudaMemcpyHostToDevice, s));
-        if (n_alt) CUDA_TRY(e, cudaMemcpyAsync(sl->alt.p, alt_utf32, n_alt * 4, cudaMemcpyHostToDevice, s));
-        if (keep && n_res) CUDA_TRY(e, cudaMemcpyAsync(sl->out.p, res_utf32, n_res * 4, cudaMemcpyHostToDevice, s));
+        if (n_ref) CU(t_err, cudaMemcpyAsync(sl->ref.p, ref_utf32, n_ref * 4, cudaMemcpyHostToDevice, s));
+        if (n_alt) CU(t_err, cudaMemcpyAsync(sl->alt.p, alt_utf32, n_alt * 4, cudaMemcpyHostToDevice, s));
+        if (keep && n_res) CU(t_err, cudaMemcpyAsync(sl->out.p, res_utf32, n_res * 4, cudaMemcpyHostToDevice, s));
     }
     // task_begin | alt_base | out_base, two entries each (staged in the pinned status block's neighbourhood is not
     // worth it: 48 bytes from the stack, consumed before this frame returns because the call is synchronous)
     const uint64_t bases[6] = {0, n_tasks, 0, n_alt * unit, 0, n_res * unit};
-    CUDA_TRY(e, cudaMemcpyAsync(sl->bases.p, bases, sizeof bases, cudaMemcpyHostToDevice, s));
+    CU(t_err, cudaMemcpyAsync(sl->bases.p, bases, sizeof bases, cudaMemcpyHostToDevice, s));
 
     KParams kp;
     memset(&kp, 0, sizeof kp);
@@ -799,28 +742,28 @@ int soa_run(v2p_engine* e, SoaSlot* sl, size_t n_tasks, const uint64_t* exec_cod
             (const uint64_t*)sl->d_soa[3].p, n_ref, n_alt, n_res, unit, kp.validate, (v2p_task16*)sl->tasks.p, kp.status);
         e->launches++;
     }
-    rc = launch_group(e, s, sl->sc, kp, nullptr, nullptr, sl->h_status, /*init_status=*/false, nullptr, false);
+    rc = launch_group(e, s, sl->sc, kp, nullptr, nullptr, h_status, /*init_status=*/false, nullptr, false);
     if (rc) return rc;
-    CUDA_TRY(e, cudaStreamSynchronize(s));
-    if (needs_serial(*sl->h_status)) {
-        if ((rc = launch_serial(e, s, kp, sl->h_status->unsorted))) return rc;
-        CUDA_TRY(e, cudaStreamSynchronize(s));
+    CU(t_err, cudaStreamSynchronize(s));
+    if (needs_serial(*h_status)) {
+        if ((rc = launch_serial(e, s, kp, h_status->unsorted))) return rc;
+        CU(t_err, cudaStreamSynchronize(s));
     }
     v2p_result r;
     memset(&r, 0, sizeof r);
-    decode_status(*sl->h_status, nullptr, 0, 0, &r);
+    decode_status(*h_status, nullptr, 0, 0, &r);
     if (r.status != V2P_OK) {
         if (bad_index) *bad_index = r.bad_task;
-        return fail(e, r.status, "task %llu rejected with status %d", (unsigned long long)r.bad_task, r.status);
+        return fail(t_err, r.status, "task %llu rejected with status %d", (unsigned long long)r.bad_task, r.status);
     }
     if (n_res) {
         if (unit == 1) {
-            CUDA_TRY(e, cudaMemcpyAsync(h_res, sl->out.p, n_res, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(e, cudaStreamSynchronize(s));
+            CU(t_err, cudaMemcpyAsync(h_res, sl->out.p, n_res, cudaMemcpyDeviceToHost, s));
+            CU(t_err, cudaStreamSynchronize(s));
             widen_u8(h_res, res_utf32, n_res);
         } else {
-            CUDA_TRY(e, cudaMemcpyAsync(res_utf32, sl->out.p, n_res * 4, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(e, cudaStreamSynchronize(s));
+            CU(t_err, cudaMemcpyAsync(res_utf32, sl->out.p, n_res * 4, cudaMemcpyDeviceToHost, s));
+            CU(t_err, cudaStreamSynchronize(s));
         }
     }
     return V2P_OK;
@@ -836,12 +779,12 @@ int v2p_execute_soa(v2p_engine* e, size_t n_tasks, const uint64_t* exec_code, co
     t_err.clear();
     if (bad_index) *bad_index = 0;
     if (n_tasks && (!exec_code || !start_pos || !length || !start_pos_res))
-        return fail(e, V2P_ERR_INVALID_ARG, "NULL task array");
+        return fail(t_err, V2P_ERR_INVALID_ARG, "NULL task array");
     if ((n_ref && !ref_utf32) || (n_alt && !alt_utf32) || (n_res && !res_utf32))
-        return fail(e, V2P_ERR_INVALID_ARG, "NULL tape");
+        return fail(t_err, V2P_ERR_INVALID_ARG, "NULL tape");
     const uint64_t lim = 0xFFFFFFFFull / 4;
     if (n_ref > lim || n_alt > lim || n_res > lim)
-        return fail(e, V2P_ERR_INVALID_ARG, "tape longer than 2^30 residues: use v2p_execute_batch");
+        return fail(t_err, V2P_ERR_INVALID_ARG, "tape longer than 2^30 residues: use v2p_execute_batch");
     SoaSlot* sl = soa_acquire(e);
     const int rc = soa_run(e, sl, n_tasks, exec_code, start_pos, length, start_pos_res, ref_utf32, n_ref, alt_utf32, n_alt,
                            res_utf32, n_res, flags, bad_index);
@@ -855,7 +798,7 @@ int v2p_gir_execute(v2p_engine* e, int engine_kind, size_t n_tasks, const uint64
                     const uint32_t* alt_utf32, size_t n_alt, uint32_t* res_utf32, size_t n_res, uint32_t flags,
                     uint64_t* bad_index) {
     if (engine_kind != V2P_ENGINE_GPU)
-        return fail(e, V2P_ERR_NOT_GPU_ENGINE, "engine kind %d is executed by the caller (gir.rs:201-235)", engine_kind);
+        return fail(t_err, V2P_ERR_NOT_GPU_ENGINE, "engine kind %d is executed by the caller (gir.rs:201-235)", engine_kind);
     return v2p_execute_soa(e, n_tasks, exec_code, start_pos, length, start_pos_res, ref_utf32, n_ref, alt_utf32, n_alt,
                            res_utf32, n_res, flags, bad_index);
 }

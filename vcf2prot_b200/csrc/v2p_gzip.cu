@@ -11,8 +11,6 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <cub/device/device_scan.cuh>
 #include <new>
@@ -21,6 +19,7 @@
 
 #include "v2p_crc32.cuh"
 #include "v2p_gzip.h"
+#include "v2p_hostres.cuh"
 #include "v2p_mapped.cuh"
 
 namespace {
@@ -631,11 +630,6 @@ __global__ void __launch_bounds__(NT, 5) k_gz_encode(GzArgs a) {
     }
 }
 
-struct Buf {
-    void* p = nullptr;
-    size_t cap = 0;
-};
-
 }  // namespace
 
 struct v2p_gzip {
@@ -643,39 +637,9 @@ struct v2p_gzip {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string err;
-    Buf file_begin, chunk_first, lens, csize, ccrc, coff, out_begin, ctr, cub_tmp, in_stage, out_stage;
+    v2p::DevBuf file_begin, chunk_first, lens, csize, ccrc, coff, out_begin, ctr, cub_tmp, in_stage, out_stage;
     v2p::MappedBuf pub;  // totals and per-file offsets come back through mapped pinned memory (v2p_mapped.cuh)
 };
-
-namespace {
-
-int zfail(v2p_gzip* z, int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (z) z->err = buf;
-    return code;
-}
-#define ZCU(z, call)                                                                                                  \
-    do {                                                                                                              \
-        cudaError_t _st = (call);                                                                                     \
-        if (_st != cudaSuccess) return zfail((z), V2P_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_st), \
-                                             __FILE__, __LINE__);                                                      \
-    } while (0)
-
-int zneed(v2p_gzip* z, Buf& b, size_t bytes) {
-    bytes = bytes < 256 ? 256 : bytes;
-    if (b.cap >= bytes) return V2P_OK;
-    if (b.p) ZCU(z, cudaFree(b.p));
-    b.p = nullptr, b.cap = 0;
-    ZCU(z, cudaMalloc(&b.p, bytes + bytes / 8));
-    b.cap = bytes + bytes / 8;
-    return V2P_OK;
-}
-
-}  // namespace
 
 extern "C" {
 
@@ -687,14 +651,14 @@ int v2p_gzip_create(int cuda_device, v2p_gzip** out) {
     v2p_gzip* z = new (std::nothrow) v2p_gzip;
     if (!z) return V2P_ERR_CUDA;
     z->device = cuda_device;
-    if (cudaSetDevice(cuda_device) != cudaSuccess || cudaStreamCreateWithFlags(&z->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreate(&z->ev0) != cudaSuccess || cudaEventCreate(&z->ev1) != cudaSuccess) {
-        delete z;
-        return V2P_ERR_CUDA;
+    bool ok = cudaSetDevice(cuda_device) == cudaSuccess && cudaStreamCreateWithFlags(&z->stream, cudaStreamNonBlocking) == cudaSuccess &&
+              cudaEventCreate(&z->ev0) == cudaSuccess && cudaEventCreate(&z->ev1) == cudaSuccess;
+    if (ok) {
+        cudaDeviceGetAttribute(&z->sms, cudaDevAttrMultiProcessorCount, cuda_device);
+        k_crc32_init<<<1, 256, 0, z->stream>>>();
+        ok = cudaStreamSynchronize(z->stream) == cudaSuccess;
     }
-    cudaDeviceGetAttribute(&z->sms, cudaDevAttrMultiProcessorCount, cuda_device);
-    k_crc32_init<<<1, 256, 0, z->stream>>>();
-    if (cudaStreamSynchronize(z->stream) != cudaSuccess) {
+    if (!ok) {
         v2p_gzip_destroy(z);
         return V2P_ERR_CUDA;
     }
@@ -705,16 +669,11 @@ int v2p_gzip_create(int cuda_device, v2p_gzip** out) {
 void v2p_gzip_destroy(v2p_gzip* z) {
     if (!z) return;
     cudaSetDevice(z->device);
-    cudaStreamSynchronize(z->stream);
-    Buf* all[] = {&z->file_begin, &z->chunk_first, &z->lens, &z->csize, &z->ccrc, &z->coff, &z->out_begin, &z->ctr, &z->cub_tmp,
-                  &z->in_stage, &z->out_stage};
-    for (Buf* b : all)
-        if (b->p) cudaFree(b->p);
-    z->pub.release();
+    if (z->stream) cudaStreamSynchronize(z->stream);
     if (z->ev0) cudaEventDestroy(z->ev0);
     if (z->ev1) cudaEventDestroy(z->ev1);
     if (z->stream) cudaStreamDestroy(z->stream);
-    delete z;
+    delete z;  // frees every buffer
 }
 
 const char* v2p_gzip_last_error(v2p_gzip* z) { return z ? z->err.c_str() : "gzip context is NULL"; }
@@ -729,12 +688,12 @@ int v2p_gzip_files(v2p_gzip* z, const uint8_t* in, const uint64_t* file_begin, u
     z->err.clear();
     if (res) memset(res, 0, sizeof *res);
     for (uint64_t f = 0; f < n_files; ++f)
-        if (file_begin[f + 1] < file_begin[f]) return zfail(z, V2P_ERR_INVALID_ARG, "file_begin not ascending at file %llu", (unsigned long long)f);
+        if (file_begin[f + 1] < file_begin[f]) return v2p::fail(z->err, V2P_ERR_INVALID_ARG, "file_begin not ascending at file %llu", (unsigned long long)f);
     const uint64_t lo = file_begin[0], hi = file_begin[n_files], in_bytes = hi - lo;
-    if ((in_bytes && !in) || (n_files && !out)) return zfail(z, V2P_ERR_INVALID_ARG, "in / out is NULL");
+    if ((in_bytes && !in) || (n_files && !out)) return v2p::fail(z->err, V2P_ERR_INVALID_ARG, "in / out is NULL");
     out_begin[0] = 0;
     if (!n_files) return V2P_OK;
-    ZCU(z, cudaSetDevice(z->device));
+    CU(z->err, cudaSetDevice(z->device));
     cudaStream_t st = z->stream;
     std::vector<uint64_t> chunk_first(n_files + 1);
     chunk_first[0] = 0;
@@ -743,65 +702,64 @@ int v2p_gzip_files(v2p_gzip* z, const uint8_t* in, const uint64_t* file_begin, u
         chunk_first[f + 1] = chunk_first[f] + std::max<uint64_t>(1, (len + CH - 1) / CH);
     }
     const uint64_t n_chunks = chunk_first[n_files];
-    int rc;
-    if ((rc = zneed(z, z->file_begin, (n_files + 1) * 8)) || (rc = zneed(z, z->chunk_first, (n_files + 1) * 8)) ||
-        (rc = zneed(z, z->out_begin, (n_files + 1) * 8)) || (rc = zneed(z, z->lens, n_chunks * LENS_STRIDE)) ||
-        (rc = zneed(z, z->csize, (n_chunks + 1) * 8)) || (rc = zneed(z, z->coff, (n_chunks + 1) * 8)) ||
-        (rc = zneed(z, z->ccrc, n_chunks * 4)) || (rc = zneed(z, z->ctr, 64)))
-        return rc;
+    CU(z->err, z->file_begin.need((n_files + 1) * 8));
+    CU(z->err, z->chunk_first.need((n_files + 1) * 8));
+    CU(z->err, z->out_begin.need((n_files + 1) * 8));
+    CU(z->err, z->lens.need(n_chunks * LENS_STRIDE));
+    CU(z->err, z->csize.need((n_chunks + 1) * 8));
+    CU(z->err, z->coff.need((n_chunks + 1) * 8));
+    CU(z->err, z->ccrc.need(n_chunks * 4));
+    CU(z->err, z->ctr.need(64));
     const bool dev = flags & V2P_FLAG_DEVICE_PTRS;
-    ZCU(z, cudaEventRecord(z->ev0, st));
+    CU(z->err, cudaEventRecord(z->ev0, st));
     GzArgs a{};
     if (dev) {
         a.in = in, a.in_lo = lo, a.in_hi = hi;
     } else {
-        if ((rc = zneed(z, z->in_stage, in_bytes + 16))) return rc;
-        if (in_bytes) ZCU(z, cudaMemcpyAsync(z->in_stage.p, in + lo, in_bytes, cudaMemcpyHostToDevice, st));
+        CU(z->err, v2p::upload(z->in_stage, in + lo, in_bytes, st));
         a.in = (const uint8_t*)z->in_stage.p - lo, a.in_lo = lo, a.in_hi = hi;  // only in[lo..hi) is ever dereferenced
     }
-    ZCU(z, cudaMemcpyAsync(z->file_begin.p, file_begin, (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
-    ZCU(z, cudaMemcpyAsync(z->chunk_first.p, chunk_first.data(), (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
-    ZCU(z, cudaMemsetAsync(z->ctr.p, 0, 64, st));
-    ZCU(z, cudaMemsetAsync((char*)z->csize.p + n_chunks * 8, 0, 8, st));
+    CU(z->err, cudaMemcpyAsync(z->file_begin.p, file_begin, (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
+    CU(z->err, cudaMemcpyAsync(z->chunk_first.p, chunk_first.data(), (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
+    CU(z->err, cudaMemsetAsync(z->ctr.p, 0, 64, st));
+    CU(z->err, cudaMemsetAsync((char*)z->csize.p + n_chunks * 8, 0, 8, st));
     a.file_begin = (const uint64_t*)z->file_begin.p, a.chunk_first = (const uint64_t*)z->chunk_first.p;
     a.n_files = n_files, a.n_chunks = n_chunks;
     a.lens = (uint8_t*)z->lens.p, a.csize = (uint64_t*)z->csize.p, a.ccrc = (uint32_t*)z->ccrc.p;
     a.coff = (const uint64_t*)z->coff.p, a.out_begin = (uint64_t*)z->out_begin.p, a.n_stored = (unsigned long long*)z->ctr.p;
     const unsigned grid = (unsigned)std::min<uint64_t>(n_chunks, (uint64_t)z->sms * 16);
     k_gz_plan<<<grid, NT, 0, st>>>(a);
-    ZCU(z, cudaGetLastError());
-    size_t tmp = 0;
-    ZCU(z, cub::DeviceScan::ExclusiveSum(nullptr, tmp, a.csize, (uint64_t*)z->coff.p, (int64_t)(n_chunks + 1), st));
-    if ((rc = zneed(z, z->cub_tmp, tmp))) return rc;
-    ZCU(z, cub::DeviceScan::ExclusiveSum(z->cub_tmp.p, tmp, a.csize, (uint64_t*)z->coff.p, (int64_t)(n_chunks + 1), st));
-    ZCU(z, z->pub.reserve(n_files + 1 + 8));
+    CU(z->err, cudaGetLastError());
+    const int rc = v2p::exclusive_sum(z->err, z->cub_tmp, a.csize, (uint64_t*)z->coff.p, n_chunks + 1, st);
+    if (rc) return rc;
+    CU(z->err, z->pub.reserve(n_files + 1 + 8));
     {
         v2p::PubList pl{};
         pl.src[0] = (const unsigned long long*)z->coff.p + n_chunks, pl.src[1] = (const unsigned long long*)z->ctr.p, pl.n = 2;
         v2p::k_publish_list<<<1, 32, 0, st>>>(z->pub.p, pl);
     }
-    ZCU(z, cudaStreamSynchronize(st));
+    CU(z->err, cudaStreamSynchronize(st));
     const uint64_t total = z->pub.p[0];
     const unsigned long long n_stored = z->pub.p[1];
     if (total > out_capacity)
-        return zfail(z, V2P_ERR_RES_OOB, "output needs %llu bytes, capacity is %llu (v2p_gzip_bound gives a safe size)",
-                     (unsigned long long)total, (unsigned long long)out_capacity);
+        return v2p::fail(z->err, V2P_ERR_RES_OOB, "output needs %llu bytes, capacity is %llu (v2p_gzip_bound gives a safe size)",
+                         (unsigned long long)total, (unsigned long long)out_capacity);
     if (dev) {
         a.out = out;
     } else {
-        if ((rc = zneed(z, z->out_stage, total + 16))) return rc;
+        CU(z->err, z->out_stage.need(total + 16));
         a.out = (uint8_t*)z->out_stage.p;
     }
     k_gz_files<<<(unsigned)((n_files + 1 + 127) / 128), 128, 0, st>>>(a);
     k_gz_encode<<<grid, NT, 0, st>>>(a);
-    ZCU(z, cudaGetLastError());
-    ZCU(z, v2p::publish_words(z->pub.p + 8, z->out_begin.p, n_files + 1, st));
-    if (!dev && total) ZCU(z, cudaMemcpyAsync(out, a.out, total, cudaMemcpyDeviceToHost, st));
-    ZCU(z, cudaEventRecord(z->ev1, st));
-    ZCU(z, cudaStreamSynchronize(st));
+    CU(z->err, cudaGetLastError());
+    CU(z->err, v2p::publish_words(z->pub.p + 8, z->out_begin.p, n_files + 1, st));
+    if (!dev && total) CU(z->err, cudaMemcpyAsync(out, a.out, total, cudaMemcpyDeviceToHost, st));
+    CU(z->err, cudaEventRecord(z->ev1, st));
+    CU(z->err, cudaStreamSynchronize(st));
     memcpy(out_begin, z->pub.p + 8, (n_files + 1) * 8);
     float ms = 0;
-    ZCU(z, cudaEventElapsedTime(&ms, z->ev0, z->ev1));
+    CU(z->err, cudaEventElapsedTime(&ms, z->ev0, z->ev1));
     if (res) res->in_bytes = in_bytes, res->out_bytes = total, res->n_chunks = n_chunks, res->n_stored_chunks = n_stored, res->ms = ms;
     return V2P_OK;
 }

@@ -9,6 +9,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <utility>
+
 namespace v2p {
 
 struct PubList {
@@ -28,10 +30,23 @@ static __global__ void k_publish_words(unsigned long long* __restrict__ dst, con
     __threadfence_system();
 }
 
-// pinned + mapped host scratch; under unified addressing the device uses the same pointer
+// pinned + mapped host scratch, freed by the destructor; under unified addressing the device uses the same pointer
 struct MappedBuf {
     unsigned long long* p = nullptr;
     size_t words = 0;
+
+    MappedBuf() = default;
+    MappedBuf(const MappedBuf&) = delete;
+    MappedBuf& operator=(const MappedBuf&) = delete;
+    MappedBuf(MappedBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), words(std::exchange(o.words, 0)) {}
+    MappedBuf& operator=(MappedBuf&& o) noexcept {
+        std::swap(p, o.p), std::swap(words, o.words);
+        return *this;
+    }
+    ~MappedBuf() {
+        if (p) cudaFreeHost(p);
+    }
+
     cudaError_t reserve(size_t n) {
         n = n < 64 ? 64 : n;
         if (words >= n) return cudaSuccess;
@@ -40,10 +55,6 @@ struct MappedBuf {
         cudaError_t st = cudaHostAlloc((void**)&p, (n + n / 4) * 8, cudaHostAllocMapped | cudaHostAllocPortable);
         if (st == cudaSuccess) words = n + n / 4;
         return st;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr, words = 0;
     }
 };
 

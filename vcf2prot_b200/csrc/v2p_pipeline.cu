@@ -15,16 +15,17 @@
 #include <mutex>
 #include <thread>
 #include <chrono>
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <new>
 #include <string>
 #include <vector>
 
 #include "v2p_allrecords.cuh"
+#include "v2p_hostres.cuh"
 #include "v2p_mapped.cuh"
 #include "v2p_pipeline.h"
+
+using namespace v2p;
 
 namespace {
 
@@ -33,16 +34,12 @@ struct Lane {
     v2p_gzip* gz = nullptr;        // owned
     cudaStream_t copy = nullptr;
     cudaEvent_t landed = nullptr;
-    void* d_gz = nullptr;  // compressed chunk (device)
-    size_t d_gz_cap = 0;
-    void* d_begin = nullptr;  // rebased site_begin of the chunk (mask entry point)
-    size_t d_begin_cap = 0;
-    v2p::MappedBuf pub;        // out_base of the chunk, published by a kernel (v2p_mapped.cuh)
-    uint8_t* h_buf = nullptr;  // pinned staging (sink mode)
-    size_t h_cap = 0;
+    DevBuf d_gz;      // compressed chunk
+    DevBuf d_begin;   // rebased site_begin of the chunk (mask entry point)
+    MappedBuf pub;    // out_base of the chunk, published by a kernel (v2p_mapped.cuh)
+    PinnedBuf h_buf;  // staging (sink mode)
     // `-a` expansion of the chunk (V2P_PIPE_ALL_RECORDS, v2p_allrecords.cuh): scratch, the merged Task array, its tape
-    void* ar[12] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    size_t ar_cap[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    DevBuf ar[12];
     // the chunk in flight
     bool pending = false;
     uint64_t first_sample = 0, n = 0;
@@ -62,57 +59,11 @@ struct v2p_pipeline {
     // `-a`: tables of the extended reference tape (v2p_pipeline_enable_all_records)
     bool all_on = false;
     v2p_ar::Tables tab{};
-    void* d_tab[4] = {nullptr, nullptr, nullptr, nullptr};
+    DevBuf d_tab[4];
     uint64_t n_proteome = 0;
 };
 
 namespace {
-
-int pfail(v2p_pipeline* p, int code, const char* fmt, ...) {
-    char buf[640];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (p) p->err = buf;
-    return code;
-}
-#define PCU(p, call)                                                                                                   \
-    do {                                                                                                               \
-        cudaError_t _st = (call);                                                                                      \
-        if (_st != cudaSuccess)                                                                                        \
-            return pfail((p), V2P_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_st), __FILE__, __LINE__); \
-    } while (0)
-
-// inside the chunk loop: record the failure and leave the loop, so that the drain loop still waits for every copy in flight
-#define PCU_BREAK(p, rc, call)                                                                                        \
-    {                                                                                                                 \
-        cudaError_t _st = (call);                                                                                     \
-        if (_st != cudaSuccess) {                                                                                     \
-            (rc) = pfail((p), V2P_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_st), __FILE__, __LINE__); \
-            break;                                                                                                    \
-        }                                                                                                             \
-    }
-
-int grow_dev(v2p_pipeline* p, void*& ptr, size_t& cap, size_t bytes) {
-    bytes = std::max<size_t>(bytes, 256);
-    if (cap >= bytes) return V2P_OK;
-    if (ptr) PCU(p, cudaFree(ptr));
-    ptr = nullptr, cap = 0;
-    PCU(p, cudaMalloc(&ptr, bytes + bytes / 8));
-    cap = bytes + bytes / 8;
-    return V2P_OK;
-}
-
-int grow_host(v2p_pipeline* p, Lane& l, size_t bytes) {
-    bytes = std::max<size_t>(bytes, 4096);
-    if (l.h_cap >= bytes) return V2P_OK;
-    if (l.h_buf) PCU(p, cudaFreeHost(l.h_buf));
-    l.h_buf = nullptr, l.h_cap = 0;
-    PCU(p, cudaMallocHost((void**)&l.h_buf, bytes + bytes / 8));
-    l.h_cap = bytes + bytes / 8;
-    return V2P_OK;
-}
 
 double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
@@ -121,13 +72,13 @@ int retire(v2p_pipeline* p, Lane& l, v2p_file_sink sink, void* user, v2p_pipelin
     if (!l.pending) return V2P_OK;
     l.pending = false;
     const double t0 = now_s();
-    PCU(p, cudaEventSynchronize(l.landed));
+    CU(p->err, cudaEventSynchronize(l.landed));
     const double t1 = now_s();
     res->wait_wall_s += t1 - t0;
     const int stop = sink ? sink(user, l.first_sample, l.n, l.h_data, l.fb_rel.data()) : 0;
     res->sink_wall_s += now_s() - t1;
     if (stop != 0)
-        return pfail(p, V2P_ERR_INVALID_ARG, "the file sink stopped the run at sample %llu", (unsigned long long)l.first_sample);
+        return fail(p->err, V2P_ERR_INVALID_ARG, "the file sink stopped the run at sample %llu", (unsigned long long)l.first_sample);
     return V2P_OK;
 }
 
@@ -138,46 +89,37 @@ int expand_all_records(v2p_pipeline* p, Lane& l, const v2p_generated& g, v2p_bat
     const uint64_t nh = g.batch.n_hap, nr = g.n_rows, nt = g.batch.n_tasks;
     cudaStream_t st = p->aux;
     int rc;
-    auto buf = [&](int i, size_t bytes) -> int { return grow_dev(p, l.ar[i], l.ar_cap[i], bytes); };
-    if ((rc = buf(0, (nh + 1) * 8)) || (rc = buf(1, (nr + 1) * 8)) || (rc = buf(2, (nr + 1) * 8)) || (rc = buf(3, (nh + 1) * 8)) ||
-        (rc = buf(4, (nh + 1) * 8)) || (rc = buf(5, (nh + 1) * 8)) || (rc = buf(6, (nh + 1) * 8)) || (rc = buf(7, (nh + 1) * 8)) ||
-        (rc = buf(8, (nh + 1) * 8)))
-        return rc;
+    for (int i : {0, 3, 4, 5, 6, 7, 8}) CU(p->err, l.ar[i].need((nh + 1) * 8));  // per haplotype
+    for (int i : {1, 2}) CU(p->err, l.ar[i].need((nr + 1) * 8));                 // per annotation row
     Chunk c{};
     c.n_hap = nh, c.n_rows = nr, c.n_tasks = nt;
     c.ann_hap = g.ann_hap, c.ann_tx = g.ann_tx, c.task_begin = g.batch.task_begin, c.out_base = g.batch.out_base, c.tasks = g.batch.tasks;
-    c.row_begin = (uint64_t*)l.ar[0], c.row_bytes = (uint64_t*)l.ar[1], c.row_x = (uint64_t*)l.ar[2];
-    c.ut = (uint64_t*)l.ar[3], c.ut_x = (uint64_t*)l.ar[4], c.ub = (uint64_t*)l.ar[5], c.ub_x = (uint64_t*)l.ar[6];
-    c.new_tb = (uint64_t*)l.ar[7], c.new_ob = (uint64_t*)l.ar[8];
-    auto blocks = [](uint64_t n) { return (unsigned)((n + 255) / 256); };
-    auto xsum = [&](const uint64_t* in, uint64_t* out, uint64_t n) -> int {
-        size_t tmp = 0;
-        PCU(p, cub::DeviceScan::ExclusiveSum(nullptr, tmp, in, out, (int64_t)n, st));
-        int r = buf(9, tmp);
-        if (r) return r;
-        PCU(p, cub::DeviceScan::ExclusiveSum(l.ar[9], tmp, in, out, (int64_t)n, st));
-        return V2P_OK;
-    };
+    c.row_begin = (uint64_t*)l.ar[0].p, c.row_bytes = (uint64_t*)l.ar[1].p, c.row_x = (uint64_t*)l.ar[2].p;
+    c.ut = (uint64_t*)l.ar[3].p, c.ut_x = (uint64_t*)l.ar[4].p, c.ub = (uint64_t*)l.ar[5].p, c.ub_x = (uint64_t*)l.ar[6].p;
+    c.new_tb = (uint64_t*)l.ar[7].p, c.new_ob = (uint64_t*)l.ar[8].p;
     k_ar_rows<<<blocks(std::max(nh, nr) + 1), 256, 0, st>>>(c, p->tab);
-    if ((rc = xsum(c.row_bytes, c.row_x, nr + 1))) return rc;
+    if ((rc = exclusive_sum(p->err, l.ar[9], (const uint64_t*)c.row_bytes, c.row_x, nr + 1, st))) return rc;
     k_ar_hap<<<blocks(nh + 1), 256, 0, st>>>(c, p->tab);
-    if ((rc = xsum(c.ut, c.ut_x, nh + 1)) || (rc = xsum(c.ub, c.ub_x, nh + 1))) return rc;
+    if ((rc = exclusive_sum(p->err, l.ar[9], (const uint64_t*)c.ut, c.ut_x, nh + 1, st)) ||
+        (rc = exclusive_sum(p->err, l.ar[9], (const uint64_t*)c.ub, c.ub_x, nh + 1, st)))
+        return rc;
     k_ar_bases<<<blocks(nh + 1), 256, 0, st>>>(c);
-    PCU(p, l.pub.reserve(64));
+    CU(p->err, l.pub.reserve(64));
     v2p::PubList pl{};
     pl.src[0] = (const unsigned long long*)(c.ut_x + nh), pl.src[1] = (const unsigned long long*)(c.ub_x + nh), pl.n = 2;
     v2p::k_publish_list<<<1, 32, 0, st>>>(l.pub.p, pl);
-    PCU(p, cudaStreamSynchronize(st));
+    CU(p->err, cudaStreamSynchronize(st));
     const uint64_t extra_tasks = l.pub.p[0], extra_bytes = l.pub.p[1];
     const uint64_t n_tasks = nt + extra_tasks, n_out = g.batch.n_out + extra_bytes;
-    if ((rc = buf(10, (n_tasks + 1) * sizeof(v2p_task16))) || (rc = buf(11, n_out + 64))) return rc;
-    c.new_tasks = (v2p_task16*)l.ar[10];
+    CU(p->err, l.ar[10].need((n_tasks + 1) * sizeof(v2p_task16)));
+    CU(p->err, l.ar[11].need(n_out + 64));
+    c.new_tasks = (v2p_task16*)l.ar[10].p;
     if (nt) k_ar_move<<<blocks(nt), 256, 0, st>>>(c);
     if (nh && p->tab.n_tx) k_ar_emit<<<blocks(nh * p->tab.n_tx), 256, 0, st>>>(c, p->tab, p->n_proteome);
-    PCU(p, cudaGetLastError());
-    PCU(p, cudaStreamSynchronize(st));
+    CU(p->err, cudaGetLastError());
+    CU(p->err, cudaStreamSynchronize(st));
     *xb = g.batch;
-    xb->task_begin = c.new_tb, xb->tasks = c.new_tasks, xb->out = (uint8_t*)l.ar[11], xb->out_base = c.new_ob;
+    xb->task_begin = c.new_tb, xb->tasks = c.new_tasks, xb->out = (uint8_t*)l.ar[11].p, xb->out_base = c.new_ob;
     xb->n_tasks = n_tasks, xb->n_out = n_out;
     *n_extra_records = extra_tasks / 3;
     return V2P_OK;
@@ -192,14 +134,14 @@ struct ListSource {
 
 int run(v2p_pipeline* p, uint64_t n_samples, const ListSource& src, uint32_t chunk_samples, uint32_t flags, uint8_t* out,
         uint64_t out_capacity, uint64_t* file_begin, v2p_file_sink sink, void* user, v2p_pipeline_result* res) {
-    if (!out && !sink) return pfail(p, V2P_ERR_INVALID_ARG, "neither an output buffer nor a sink was given");
-    if (out && !file_begin) return pfail(p, V2P_ERR_INVALID_ARG, "file_begin is NULL");
+    if (!out && !sink) return fail(p->err, V2P_ERR_INVALID_ARG, "neither an output buffer nor a sink was given");
+    if (out && !file_begin) return fail(p->err, V2P_ERR_INVALID_ARG, "file_begin is NULL");
     if (!chunk_samples) chunk_samples = 128;
     const bool gzip = (flags & V2P_PIPE_GZIP) != 0, all_records = (flags & V2P_PIPE_ALL_RECORDS) != 0;
     if (all_records && !p->all_on)
-        return pfail(p, V2P_ERR_INVALID_ARG, "V2P_PIPE_ALL_RECORDS needs v2p_pipeline_enable_all_records first");
+        return fail(p->err, V2P_ERR_INVALID_ARG, "V2P_PIPE_ALL_RECORDS needs v2p_pipeline_enable_all_records first");
     const uint32_t gen_flags = V2P_GEN_FASTA | ((flags & V2P_PIPE_SKIP_ABORTS) ? V2P_GEN_SKIP_ABORTS : 0u);
-    PCU(p, cudaSetDevice(p->device));
+    CU(p->err, cudaSetDevice(p->device));
     for (uint32_t i = 0; i < p->n_lanes; ++i) p->lanes[i].pending = false;
     uint64_t total = 0;
     if (file_begin) file_begin[0] = 0;
@@ -219,17 +161,17 @@ int run(v2p_pipeline* p, uint64_t n_samples, const ListSource& src, uint32_t chu
             rc = v2p_generate_tasks(l.cat, nh, sb.data(), src.h_sites + src.site_begin[h0], gen_flags, &g);
             res->h2d_bytes += sb[nh] * 4 + (nh + 1) * 8;
         } else {
-            if ((rc = grow_dev(p, l.d_begin, l.d_begin_cap, (nh + 1) * 8))) break;
-            PCU_BREAK(p, rc, cudaMemcpy(l.d_begin, sb.data(), (nh + 1) * 8, cudaMemcpyHostToDevice));
+            CU_BREAK(p->err, rc, l.d_begin.need((nh + 1) * 8));
+            CU_BREAK(p->err, rc, cudaMemcpy(l.d_begin.p, sb.data(), (nh + 1) * 8, cudaMemcpyHostToDevice));
             v2p_site_lists lists;
             memset(&lists, 0, sizeof lists);
             lists.n_hap = nh, lists.n_sites = sb[nh];
-            lists.site_begin = (const uint64_t*)l.d_begin, lists.sites = src.d_sites + src.site_begin[h0];
+            lists.site_begin = (const uint64_t*)l.d_begin.p, lists.sites = src.d_sites + src.site_begin[h0];
             rc = v2p_generate_tasks_from_lists(l.cat, &lists, gen_flags, &g);
             res->h2d_bytes += (nh + 1) * 8;
         }
         if (rc) {
-            pfail(p, rc, "task generation failed at sample %llu: %s", (unsigned long long)s0, v2p_catalogue_last_error(l.cat));
+            fail(p->err, rc, "task generation failed at sample %llu: %s", (unsigned long long)s0, v2p_catalogue_last_error(l.cat));
             break;
         }
         // ---- `-a`: the unaltered transcripts' records behind every haplotype's altered ones (write_all)
@@ -241,49 +183,49 @@ int run(v2p_pipeline* p, uint64_t n_samples, const ListSource& src, uint32_t chu
         // ---- the hot path: every haplotype's result tape == its FASTA text
         v2p_result er;
         if ((rc = v2p_execute_batch(p->eng, &xb, V2P_FLAG_DEVICE_PTRS, &er, nullptr))) {
-            pfail(p, rc, "execution failed at sample %llu (haplotype %llu task %llu): %s", (unsigned long long)s0,
-                  (unsigned long long)er.bad_hap, (unsigned long long)er.bad_task, v2p_last_error(p->eng));
+            fail(p->err, rc, "execution failed at sample %llu (haplotype %llu task %llu): %s", (unsigned long long)s0,
+                 (unsigned long long)er.bad_hap, (unsigned long long)er.bad_task, v2p_last_error(p->eng));
             break;
         }
         res->exec_wall_s += now_s() - t_exec0;
         // ---- file bounds: sample s owns haplotypes 2s, 2s+1
-        PCU_BREAK(p, rc, l.pub.reserve(nh + 1));
-        PCU_BREAK(p, rc, v2p::publish_words(l.pub.p, xb.out_base, nh + 1, p->aux));
-        PCU_BREAK(p, rc, cudaStreamSynchronize(p->aux));
+        CU_BREAK(p->err, rc, l.pub.reserve(nh + 1));
+        CU_BREAK(p->err, rc, v2p::publish_words(l.pub.p, xb.out_base, nh + 1, p->aux));
+        CU_BREAK(p->err, rc, cudaStreamSynchronize(p->aux));
         l.fb_rel.resize(ns + 1);
         for (uint64_t s = 0; s <= ns; ++s) l.fb_rel[s] = l.pub.p[2 * s];
         const uint8_t* d_src = xb.out;
         uint64_t bytes = xb.n_out;
         if (gzip) {
             const uint64_t cap = v2p_gzip_bound(xb.n_out, ns);
-            if ((rc = grow_dev(p, l.d_gz, l.d_gz_cap, cap))) break;
+            CU_BREAK(p->err, rc, l.d_gz.need(cap));
             std::vector<uint64_t> fb_abs(l.fb_rel);
             v2p_gzip_result zr;
-            if ((rc = v2p_gzip_files(l.gz, xb.out, fb_abs.data(), ns, (uint8_t*)l.d_gz, cap, l.fb_rel.data(),
+            if ((rc = v2p_gzip_files(l.gz, xb.out, fb_abs.data(), ns, (uint8_t*)l.d_gz.p, cap, l.fb_rel.data(),
                                      V2P_FLAG_DEVICE_PTRS, &zr))) {
-                pfail(p, rc, "gzip failed at sample %llu: %s", (unsigned long long)s0, v2p_gzip_last_error(l.gz));
+                fail(p->err, rc, "gzip failed at sample %llu: %s", (unsigned long long)s0, v2p_gzip_last_error(l.gz));
                 break;
             }
             res->gzip_ms += zr.ms;
             res->gzip_wall_s += zr.ms * 1e-3;
-            d_src = (const uint8_t*)l.d_gz;
+            d_src = (const uint8_t*)l.d_gz.p;
             bytes = l.fb_rel[ns];
         }
         // ---- copy-back on the lane's own stream: overlaps the next chunk's kernels
         uint8_t* h_dst;
         if (out) {
             if (total + bytes > out_capacity) {
-                rc = pfail(p, V2P_ERR_RES_OOB, "output needs more than %llu bytes (at sample %llu)", (unsigned long long)out_capacity,
-                           (unsigned long long)s0);
+                rc = fail(p->err, V2P_ERR_RES_OOB, "output needs more than %llu bytes (at sample %llu)", (unsigned long long)out_capacity,
+                          (unsigned long long)s0);
                 break;
             }
             h_dst = out + total;
         } else {
-            if ((rc = grow_host(p, l, bytes))) break;
-            h_dst = l.h_buf;
+            CU_BREAK(p->err, rc, l.h_buf.need(bytes));
+            h_dst = (uint8_t*)l.h_buf.p;
         }
-        if (bytes) PCU_BREAK(p, rc, cudaMemcpyAsync(h_dst, d_src, bytes, cudaMemcpyDeviceToHost, l.copy));
-        PCU_BREAK(p, rc, cudaEventRecord(l.landed, l.copy));
+        if (bytes) CU_BREAK(p->err, rc, cudaMemcpyAsync(h_dst, d_src, bytes, cudaMemcpyDeviceToHost, l.copy));
+        CU_BREAK(p->err, rc, cudaEventRecord(l.landed, l.copy));
         l.pending = true, l.first_sample = s0, l.n = ns, l.h_data = h_dst;
         if (file_begin)
             for (uint64_t s = 1; s <= ns; ++s) file_begin[s0 + s] = total + l.fb_rel[s];
@@ -345,17 +287,9 @@ void v2p_pipeline_destroy(v2p_pipeline* p) {
         if (l.copy) cudaStreamSynchronize(l.copy), cudaStreamDestroy(l.copy);
         if (l.landed) cudaEventDestroy(l.landed);
         if (l.gz) v2p_gzip_destroy(l.gz);
-        if (l.d_gz) cudaFree(l.d_gz);
-        if (l.d_begin) cudaFree(l.d_begin);
-        for (void* a : l.ar)
-            if (a) cudaFree(a);
-        if (l.h_buf) cudaFreeHost(l.h_buf);
-        l.pub.release();
     }
-    for (void* t : p->d_tab)
-        if (t) cudaFree(t);
     if (p->aux) cudaStreamDestroy(p->aux);
-    delete p;
+    delete p;  // frees every buffer
 }
 
 int v2p_pipeline_enable_all_records(v2p_pipeline* p, const uint8_t* proteome, uint64_t n_proteome, uint64_t n_tx,
@@ -363,14 +297,14 @@ int v2p_pipeline_enable_all_records(v2p_pipeline* p, const uint8_t* proteome, ui
     if (!p) return V2P_ERR_INVALID_ARG;
     p->err.clear();
     if (!tx_offsets || !name_off || (n_proteome && !proteome) || (n_tx && name_off[n_tx] && !names))
-        return pfail(p, V2P_ERR_INVALID_ARG, "NULL argument");
-    if (tx_offsets[n_tx] > n_proteome) return pfail(p, V2P_ERR_INVALID_ARG, "tx_offsets run past the proteome tape");
+        return fail(p->err, V2P_ERR_INVALID_ARG, "NULL argument");
+    if (tx_offsets[n_tx] > n_proteome) return fail(p->err, V2P_ERR_INVALID_ARG, "tx_offsets run past the proteome tape");
     // extended tape: proteome | for every transcript ">{name}_1\n" ">{name}_2\n"
     std::vector<uint8_t> ext(proteome, proteome + n_proteome);
     std::vector<uint64_t> hdr(n_tx), rec_x(n_tx + 1, 0);
     std::vector<uint32_t> nlen(n_tx);
     for (uint64_t t = 0; t < n_tx; ++t) {
-        if (name_off[t + 1] < name_off[t] || tx_offsets[t + 1] < tx_offsets[t]) return pfail(p, V2P_ERR_INVALID_ARG, "offsets not monotone");
+        if (name_off[t + 1] < name_off[t] || tx_offsets[t + 1] < tx_offsets[t]) return fail(p->err, V2P_ERR_INVALID_ARG, "offsets not monotone");
         const uint64_t nl = name_off[t + 1] - name_off[t];
         nlen[t] = (uint32_t)nl;
         hdr[t] = ext.size();
@@ -383,20 +317,18 @@ int v2p_pipeline_enable_all_records(v2p_pipeline* p, const uint8_t* proteome, ui
         }
         rec_x[t + 1] = rec_x[t] + nl + 5 + (tx_offsets[t + 1] - tx_offsets[t]);
     }
-    if (ext.size() >> 32) return pfail(p, V2P_ERR_INVALID_ARG, "extended reference tape exceeds 4 GiB");
+    if (ext.size() >> 32) return fail(p->err, V2P_ERR_INVALID_ARG, "extended reference tape exceeds 4 GiB");
     int rc = v2p_engine_set_reference(p->eng, ext.data(), ext.size(), 0);
-    if (rc) return pfail(p, rc, "registering the extended reference tape failed: %s", v2p_last_error(p->eng));
-    PCU(p, cudaSetDevice(p->device));
+    if (rc) return fail(p->err, rc, "registering the extended reference tape failed: %s", v2p_last_error(p->eng));
+    CU(p->err, cudaSetDevice(p->device));
     const void* src[4] = {tx_offsets, hdr.data(), nlen.data(), rec_x.data()};
     const size_t bytes[4] = {(n_tx + 1) * 8, n_tx * 8, n_tx * 4, (n_tx + 1) * 8};
     for (int i = 0; i < 4; ++i) {
-        if (p->d_tab[i]) PCU(p, cudaFree(p->d_tab[i]));
-        p->d_tab[i] = nullptr;
-        PCU(p, cudaMalloc(&p->d_tab[i], bytes[i] + 16));
-        PCU(p, cudaMemcpy(p->d_tab[i], src[i], bytes[i], cudaMemcpyHostToDevice));
+        CU(p->err, p->d_tab[i].need(bytes[i] + 16));
+        CU(p->err, cudaMemcpy(p->d_tab[i].p, src[i], bytes[i], cudaMemcpyHostToDevice));
     }
-    p->tab = v2p_ar::Tables{n_tx, (const uint64_t*)p->d_tab[0], (const uint64_t*)p->d_tab[1], (const uint32_t*)p->d_tab[2],
-                            (const uint64_t*)p->d_tab[3]};
+    p->tab = v2p_ar::Tables{n_tx, (const uint64_t*)p->d_tab[0].p, (const uint64_t*)p->d_tab[1].p, (const uint32_t*)p->d_tab[2].p,
+                            (const uint64_t*)p->d_tab[3].p};
     p->n_proteome = n_proteome;
     p->all_on = true;
     return V2P_OK;
@@ -412,10 +344,10 @@ int v2p_pipeline_run_lists(v2p_pipeline* p, uint64_t n_samples, const uint64_t* 
     v2p_pipeline_result local;
     memset(&local, 0, sizeof local);
     if (res) *res = local;  // (also on the argument errors below)
-    if (!site_begin || site_begin[0] != 0) return pfail(p, V2P_ERR_INVALID_ARG, "site_begin is NULL or does not start at 0");
+    if (!site_begin || site_begin[0] != 0) return fail(p->err, V2P_ERR_INVALID_ARG, "site_begin is NULL or does not start at 0");
     for (uint64_t h = 0; h < 2 * n_samples; ++h)
-        if (site_begin[h + 1] < site_begin[h]) return pfail(p, V2P_ERR_INVALID_ARG, "site_begin not monotone at haplotype %llu", (unsigned long long)h);
-    if (site_begin[2 * n_samples] && !sites) return pfail(p, V2P_ERR_INVALID_ARG, "sites is NULL");
+        if (site_begin[h + 1] < site_begin[h]) return fail(p->err, V2P_ERR_INVALID_ARG, "site_begin not monotone at haplotype %llu", (unsigned long long)h);
+    if (site_begin[2 * n_samples] && !sites) return fail(p->err, V2P_ERR_INVALID_ARG, "sites is NULL");
     const auto t0 = std::chrono::steady_clock::now();
     local.n_samples = n_samples;
     ListSource src{site_begin, sites ? sites : reinterpret_cast<const uint32_t*>(site_begin), nullptr};
@@ -441,7 +373,7 @@ int v2p_pipeline_run_masks(v2p_pipeline* p, uint64_t n_records, uint64_t n_sampl
     v2p_site_lists lists;
     int rc = v2p_sites_from_masks(dec, n_records, n_samples, words_per_cell, masks, csq_begin, csq_site, mask_flags, &lists);
     if (rc) {
-        pfail(p, rc, "mask decode failed: %s", v2p_catalogue_last_error(dec));
+        fail(p->err, rc, "mask decode failed: %s", v2p_catalogue_last_error(dec));
     } else {
         local.decode_ms = lists.decode_ms;
         if (!(mask_flags & V2P_FLAG_DEVICE_PTRS)) local.h2d_bytes += n_records * n_samples * words_per_cell * 4;
@@ -449,7 +381,7 @@ int v2p_pipeline_run_masks(v2p_pipeline* p, uint64_t n_records, uint64_t n_sampl
         cudaError_t st = cudaSetDevice(p->device);
         if (st == cudaSuccess) st = cudaMemcpy(sb.data(), lists.site_begin, sb.size() * 8, cudaMemcpyDeviceToHost);
         if (st != cudaSuccess) {
-            rc = pfail(p, V2P_ERR_CUDA, "reading the decoded list bounds failed: %s", cudaGetErrorString(st));
+            rc = fail(p->err, V2P_ERR_CUDA, "reading the decoded list bounds failed: %s", cudaGetErrorString(st));
         } else {
             ListSource src{sb.data(), nullptr, lists.sites};
             rc = run(p, n_samples, src, chunk_samples, flags, out, out_capacity, file_begin, sink, user, &local);

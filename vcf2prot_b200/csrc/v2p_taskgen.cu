@@ -13,8 +13,6 @@
 // Everything is integer work on HBM-resident arrays; no floating point, no host round trip except four 8-byte totals.
 #include <cuda_runtime.h>
 
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
@@ -22,16 +20,14 @@
 #include <new>
 #include <string>
 
+#include "v2p_hostres.cuh"
 #include "v2p_mapped.cuh"
 #include "v2p_taskgen.h"
 #include "v2p_taskgen_rules.cuh"
 
-namespace {
+using namespace v2p;
 
-struct Buf {
-    void* p = nullptr;
-    size_t cap = 0;
-};
+namespace {
 
 struct Cat {  // device views
     const uint64_t* tx_off;
@@ -575,66 +571,22 @@ struct v2p_catalogue {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string err;
     uint64_t n_tx = 0, n_sites = 0;
-    Buf tx_off, tx, pos, rlen, dlen, cls, doff, pool;
+    DevBuf tx_off, tx, pos, rlen, dlen, cls, doff, pool;
     bool is_ins = false;  // created by v2p_catalogue_create_ins (general rules) rather than the seven-class tables
-    Buf i_code, i_flags, i_pos_ref, i_pos_res, i_len;  // (+ tx, doff, dlen, pool shared with the class tables)
-    Buf gi_newg, gi_gx, gi_first, gi_size, gi_hap, gi_tx, gi_nsites, gi_status, gi_c[7], gi_x[7], gi_err;
+    DevBuf i_code, i_flags, i_pos_ref, i_pos_res, i_len;  // (+ tx, doff, dlen, pool shared with the class tables)
+    DevBuf gi_newg, gi_gx, gi_first, gi_size, gi_hap, gi_tx, gi_nsites, gi_status, gi_c[7], gi_x[7], gi_err;
     v2p::MappedBuf pub;   // totals come back through mapped pinned memory, not the copy engine (v2p_mapped.cuh)
-    Buf name_off, names;  // v2p_catalogue_set_names
+    DevBuf name_off, names;  // v2p_catalogue_set_names
     bool has_names = false;
     // per-generation buffers
-    Buf sites, site_begin, site_hap, flags, scan_in[6], scan_out[6], cub_tmp, totals, sel_err;
-    Buf g_first, g_len, g_slot, g_slot_x, g_hap, g_tx, ann_start, ann_end;
-    Buf tasks, task_begin, alt_base, out_base, alt_per_hap, short_tot, mut_dst, alt, out;
+    DevBuf sites, site_begin, site_hap, flags, scan_in[6], scan_out[6], cub_tmp, totals, sel_err;
+    DevBuf g_first, g_len, g_slot, g_slot_x, g_hap, g_tx, ann_start, ann_end;
+    DevBuf tasks, task_begin, alt_base, out_base, alt_per_hap, short_tot, mut_dst, alt, out;
     // mask decode (v2p_sites_from_masks)
-    Buf md_masks, md_csq_begin, md_csq_site, md_keys[2], md_uniq, md_begin, md_sites, md_ctr;
+    DevBuf md_masks, md_csq_begin, md_csq_site, md_keys[2], md_uniq, md_begin, md_sites, md_ctr;
 };
 
 namespace {
-
-int cfail(v2p_catalogue* c, int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (c) c->err = buf;
-    return code;
-}
-#define CU(c, call)                                                                                                  \
-    do {                                                                                                             \
-        cudaError_t _st = (call);                                                                                    \
-        if (_st != cudaSuccess) return cfail((c), V2P_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_st), \
-                                             __FILE__, __LINE__);                                                     \
-    } while (0)
-
-int need(v2p_catalogue* c, Buf& b, size_t bytes) {
-    bytes = bytes < 256 ? 256 : bytes;
-    if (b.cap >= bytes) return V2P_OK;
-    if (b.p) CU(c, cudaFree(b.p));
-    b.p = nullptr, b.cap = 0;
-    CU(c, cudaMalloc(&b.p, bytes + bytes / 8));
-    b.cap = bytes + bytes / 8;
-    return V2P_OK;
-}
-
-int upload(v2p_catalogue* c, Buf& b, const void* h, size_t bytes) {
-    int rc = need(c, b, bytes + 16);
-    if (rc) return rc;
-    if (bytes) CU(c, cudaMemcpyAsync(b.p, h, bytes, cudaMemcpyHostToDevice, c->stream));
-    return V2P_OK;
-}
-
-int xsum(v2p_catalogue* c, const uint64_t* in, uint64_t* out, uint64_t n) {
-    size_t tmp = 0;
-    CU(c, cub::DeviceScan::ExclusiveSum(nullptr, tmp, in, out, (int64_t)n, c->stream));
-    int rc = need(c, c->cub_tmp, tmp);
-    if (rc) return rc;
-    CU(c, cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tmp, in, out, (int64_t)n, c->stream));
-    return V2P_OK;
-}
-
-inline unsigned blocks(uint64_t n) { return (unsigned)((n + 255) / 256); }
 
 int generate_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, const uint64_t* d_site_begin, const uint32_t* d_sites,
                        uint32_t flags, v2p_generated* out);
@@ -659,20 +611,15 @@ int v2p_catalogue_create(int cuda_device, uint64_t n_tx, const uint64_t* tx_offs
     v2p_catalogue* c = new (std::nothrow) v2p_catalogue();
     if (!c) return V2P_ERR_INVALID_ARG;
     c->device = cuda_device;
-    if (cudaSetDevice(cuda_device) != cudaSuccess || cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreate(&c->ev0) != cudaSuccess || cudaEventCreate(&c->ev1) != cudaSuccess) {
-        delete c;
-        return V2P_ERR_CUDA;
-    }
     c->n_tx = n_tx, c->n_sites = n_sites;
-    int rc = 0;
-    if ((rc = upload(c, c->tx_off, tx_offsets, (n_tx + 1) * 8)) || (rc = upload(c, c->tx, site_tx, n_sites * 4)) ||
-        (rc = upload(c, c->pos, site_pos, n_sites * 4)) || (rc = upload(c, c->cls, site_cls, n_sites)) ||
-        (rc = upload(c, c->rlen, site_rlen, n_sites * 4)) || (rc = upload(c, c->doff, site_doff, n_sites * 8)) ||
-        (rc = upload(c, c->dlen, site_dlen, n_sites * 4)) || (rc = upload(c, c->pool, pool, n_pool)) ||
-        cudaStreamSynchronize(c->stream) != cudaSuccess) {
+    cudaStream_t& st = c->stream;
+    if (cudaSetDevice(cuda_device) || cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) || cudaEventCreate(&c->ev0) ||
+        cudaEventCreate(&c->ev1) || upload(c->tx_off, tx_offsets, (n_tx + 1) * 8, st) || upload(c->tx, site_tx, n_sites * 4, st) ||
+        upload(c->pos, site_pos, n_sites * 4, st) || upload(c->cls, site_cls, n_sites, st) ||
+        upload(c->rlen, site_rlen, n_sites * 4, st) || upload(c->doff, site_doff, n_sites * 8, st) ||
+        upload(c->dlen, site_dlen, n_sites * 4, st) || upload(c->pool, pool, n_pool, st) || cudaStreamSynchronize(st)) {
         v2p_catalogue_destroy(c);
-        return rc ? rc : V2P_ERR_CUDA;
+        return V2P_ERR_CUDA;
     }
     *out = c;
     return V2P_OK;
@@ -693,21 +640,16 @@ int v2p_catalogue_create_ins(int cuda_device, uint64_t n_tx, const uint64_t* tx_
     if (!c) return V2P_ERR_INVALID_ARG;
     c->device = cuda_device;
     c->is_ins = true;
-    if (cudaSetDevice(cuda_device) != cudaSuccess || cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreate(&c->ev0) != cudaSuccess || cudaEventCreate(&c->ev1) != cudaSuccess) {
-        delete c;
-        return V2P_ERR_CUDA;
-    }
     c->n_tx = n_tx, c->n_sites = n_sites;
-    int rc = 0;
-    if ((rc = upload(c, c->tx_off, tx_offsets, (n_tx + 1) * 8)) || (rc = upload(c, c->tx, site_tx, n_sites * 4)) ||
-        (rc = upload(c, c->i_code, ins_code, n_sites)) || (rc = upload(c, c->i_flags, ins_flags, n_sites)) ||
-        (rc = upload(c, c->i_pos_ref, ins_pos_ref, n_sites * 4)) || (rc = upload(c, c->i_pos_res, ins_pos_res, n_sites * 4)) ||
-        (rc = upload(c, c->i_len, ins_len, n_sites * 4)) || (rc = upload(c, c->doff, ins_doff, n_sites * 8)) ||
-        (rc = upload(c, c->dlen, ins_dlen, n_sites * 4)) || (rc = upload(c, c->pool, pool, n_pool)) ||
-        cudaStreamSynchronize(c->stream) != cudaSuccess) {
+    cudaStream_t& st = c->stream;
+    if (cudaSetDevice(cuda_device) || cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) || cudaEventCreate(&c->ev0) ||
+        cudaEventCreate(&c->ev1) || upload(c->tx_off, tx_offsets, (n_tx + 1) * 8, st) || upload(c->tx, site_tx, n_sites * 4, st) ||
+        upload(c->i_code, ins_code, n_sites, st) || upload(c->i_flags, ins_flags, n_sites, st) ||
+        upload(c->i_pos_ref, ins_pos_ref, n_sites * 4, st) || upload(c->i_pos_res, ins_pos_res, n_sites * 4, st) ||
+        upload(c->i_len, ins_len, n_sites * 4, st) || upload(c->doff, ins_doff, n_sites * 8, st) ||
+        upload(c->dlen, ins_dlen, n_sites * 4, st) || upload(c->pool, pool, n_pool, st) || cudaStreamSynchronize(st)) {
         v2p_catalogue_destroy(c);
-        return rc ? rc : V2P_ERR_CUDA;
+        return V2P_ERR_CUDA;
     }
     *out = c;
     return V2P_OK;
@@ -716,28 +658,11 @@ int v2p_catalogue_create_ins(int cuda_device, uint64_t n_tx, const uint64_t* tx_
 void v2p_catalogue_destroy(v2p_catalogue* c) {
     if (!c) return;
     cudaSetDevice(c->device);
-    cudaStreamSynchronize(c->stream);
-    Buf* all[] = {&c->i_code, &c->i_flags, &c->i_pos_ref, &c->i_pos_res, &c->i_len, &c->gi_newg, &c->gi_gx, &c->gi_first,
-                  &c->gi_size, &c->gi_hap, &c->gi_tx, &c->gi_nsites, &c->gi_status, &c->gi_err,
-                  &c->gi_c[0], &c->gi_c[1], &c->gi_c[2], &c->gi_c[3], &c->gi_c[4], &c->gi_c[5], &c->gi_c[6],
-                  &c->gi_x[0], &c->gi_x[1], &c->gi_x[2], &c->gi_x[3], &c->gi_x[4], &c->gi_x[5], &c->gi_x[6],
-                  &c->name_off, &c->names,
-                  &c->tx_off, &c->tx, &c->pos, &c->rlen, &c->dlen, &c->cls, &c->doff, &c->pool, &c->sites, &c->site_begin,
-                  &c->site_hap, &c->flags, &c->cub_tmp, &c->totals, &c->sel_err, &c->g_first, &c->g_len, &c->g_slot, &c->g_slot_x, &c->g_hap,
-                  &c->g_tx, &c->ann_start, &c->ann_end, &c->tasks, &c->task_begin, &c->alt_base, &c->out_base, &c->alt_per_hap,
-                  &c->short_tot, &c->mut_dst, &c->alt, &c->out, &c->md_masks, &c->md_csq_begin, &c->md_csq_site, &c->md_keys[0],
-                  &c->md_keys[1], &c->md_uniq, &c->md_begin, &c->md_sites, &c->md_ctr};
-    for (Buf* b : all)
-        if (b->p) cudaFree(b->p);
-    for (int i = 0; i < 6; ++i) {
-        if (c->scan_in[i].p) cudaFree(c->scan_in[i].p);
-        if (c->scan_out[i].p) cudaFree(c->scan_out[i].p);
-    }
-    c->pub.release();
+    if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;  // frees every buffer
 }
 
 const char* v2p_catalogue_last_error(v2p_catalogue* c) { return c ? c->err.c_str() : "catalogue is NULL"; }
@@ -746,14 +671,14 @@ int v2p_catalogue_set_names(v2p_catalogue* c, const uint64_t* name_off, const ui
     if (!c || !name_off) return V2P_ERR_INVALID_ARG;
     c->err.clear();
     c->has_names = false;
-    if (name_off[0] != 0) return cfail(c, V2P_ERR_INVALID_ARG, "name_off[0] must be 0");
+    if (name_off[0] != 0) return fail(c->err, V2P_ERR_INVALID_ARG, "name_off[0] must be 0");
     for (uint64_t t = 0; t < c->n_tx; ++t)
-        if (name_off[t + 1] < name_off[t]) return cfail(c, V2P_ERR_INVALID_ARG, "name_off not monotone");
-    if (name_off[c->n_tx] && !names) return cfail(c, V2P_ERR_INVALID_ARG, "names is NULL");
-    CU(c, cudaSetDevice(c->device));
-    int rc;
-    if ((rc = upload(c, c->name_off, name_off, (c->n_tx + 1) * 8)) || (rc = upload(c, c->names, names, name_off[c->n_tx]))) return rc;
-    CU(c, cudaStreamSynchronize(c->stream));
+        if (name_off[t + 1] < name_off[t]) return fail(c->err, V2P_ERR_INVALID_ARG, "name_off not monotone");
+    if (name_off[c->n_tx] && !names) return fail(c->err, V2P_ERR_INVALID_ARG, "names is NULL");
+    CU(c->err, cudaSetDevice(c->device));
+    CU(c->err, upload(c->name_off, name_off, (c->n_tx + 1) * 8, c->stream));
+    CU(c->err, upload(c->names, names, name_off[c->n_tx], c->stream));
+    CU(c->err, cudaStreamSynchronize(c->stream));
     c->has_names = true;
     return V2P_OK;
 }
@@ -768,14 +693,14 @@ int v2p_generate_tasks(v2p_catalogue* c, uint64_t n_hap, const uint64_t* site_be
     if (!c || !out || !site_begin || site_begin[0] != 0) return V2P_ERR_INVALID_ARG;
     memset(out, 0, sizeof *out);
     c->err.clear();
-    CU(c, cudaSetDevice(c->device));
+    CU(c->err, cudaSetDevice(c->device));
     const uint64_t n_sel = site_begin[n_hap];
-    if (n_sel && !sites) return cfail(c, V2P_ERR_INVALID_ARG, "sites is NULL");
+    if (n_sel && !sites) return fail(c->err, V2P_ERR_INVALID_ARG, "sites is NULL");
     for (uint64_t h = 0; h < n_hap; ++h)
-        if (site_begin[h + 1] < site_begin[h]) return cfail(c, V2P_ERR_INVALID_ARG, "site_begin not monotone");
-    int rc;
-    CU(c, cudaEventRecord(c->ev0, c->stream));
-    if ((rc = upload(c, c->sites, sites, n_sel * 4)) || (rc = upload(c, c->site_begin, site_begin, (n_hap + 1) * 8))) return rc;
+        if (site_begin[h + 1] < site_begin[h]) return fail(c->err, V2P_ERR_INVALID_ARG, "site_begin not monotone");
+    CU(c->err, cudaEventRecord(c->ev0, c->stream));
+    CU(c->err, upload(c->sites, sites, n_sel * 4, c->stream));
+    CU(c->err, upload(c->site_begin, site_begin, (n_hap + 1) * 8, c->stream));
     return generate_on_device(c, n_hap, n_sel, (const uint64_t*)c->site_begin.p, (const uint32_t*)c->sites.p, flags, out);
 }
 
@@ -786,36 +711,36 @@ int v2p_sites_from_masks(v2p_catalogue* c, uint64_t n_records, uint64_t n_sample
     memset(out, 0, sizeof *out);
     c->err.clear();
     const uint64_t n_words = n_records * n_samples * words_per_cell, n_hap = 2 * n_samples, n_csq = csq_begin[n_records];
-    if ((n_words && !masks) || (n_csq && !csq_site)) return cfail(c, V2P_ERR_INVALID_ARG, "masks / csq_site is NULL");
-    if (n_hap >> 31) return cfail(c, V2P_ERR_INVALID_ARG, "more than 2^30 samples");
+    if ((n_words && !masks) || (n_csq && !csq_site)) return fail(c->err, V2P_ERR_INVALID_ARG, "masks / csq_site is NULL");
+    if (n_hap >> 31) return fail(c->err, V2P_ERR_INVALID_ARG, "more than 2^30 samples");
     for (uint64_t r = 0; r < n_records; ++r)
-        if (csq_begin[r + 1] < csq_begin[r]) return cfail(c, V2P_ERR_INVALID_ARG, "csq_begin not monotone");
+        if (csq_begin[r + 1] < csq_begin[r]) return fail(c->err, V2P_ERR_INVALID_ARG, "csq_begin not monotone");
     for (uint64_t k = 0; k < n_csq; ++k)
         if (csq_site[k] >= 0 && (uint64_t)csq_site[k] >= c->n_sites)
-            return cfail(c, V2P_ERR_INVALID_ARG, "csq_site[%llu] = %d is not a catalogue site", (unsigned long long)k, csq_site[k]);
-    CU(c, cudaSetDevice(c->device));
+            return fail(c->err, V2P_ERR_INVALID_ARG, "csq_site[%llu] = %d is not a catalogue site", (unsigned long long)k, csq_site[k]);
+    CU(c->err, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
-    int rc;
-    CU(c, cudaEventRecord(c->ev0, st));
+    CU(c->err, cudaEventRecord(c->ev0, st));
     const uint32_t* d_masks = masks;
     if (!(flags & V2P_FLAG_DEVICE_PTRS)) {
-        if ((rc = upload(c, c->md_masks, masks, n_words * 4))) return rc;
+        CU(c->err, upload(c->md_masks, masks, n_words * 4, st));
         d_masks = (const uint32_t*)c->md_masks.p;
     } else if ((uintptr_t)masks & 15) {
-        return cfail(c, V2P_ERR_INVALID_ARG, "device mask matrix must be 16-byte aligned");
+        return fail(c->err, V2P_ERR_INVALID_ARG, "device mask matrix must be 16-byte aligned");
     }
-    if ((rc = upload(c, c->md_csq_begin, csq_begin, (n_records + 1) * 8)) || (rc = upload(c, c->md_csq_site, csq_site, n_csq * 4)) ||
-        (rc = need(c, c->md_ctr, sizeof(MdCtr))) || (rc = need(c, c->md_begin, (n_hap + 1) * 8)))
-        return rc;
+    CU(c->err, upload(c->md_csq_begin, csq_begin, (n_records + 1) * 8, st));
+    CU(c->err, upload(c->md_csq_site, csq_site, n_csq * 4, st));
+    CU(c->err, c->md_ctr.need(sizeof(MdCtr)));
+    CU(c->err, c->md_begin.need((n_hap + 1) * 8));
     MdCtr* ctr = (MdCtr*)c->md_ctr.p;
     MdCtr h{0, 0, ~0ull, 0};
-    CU(c, cudaMemcpyAsync(ctr, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    CU(c->err, cudaMemcpyAsync(ctr, &h, sizeof h, cudaMemcpyHostToDevice, st));
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device);
     const unsigned grid = (unsigned)std::min<uint64_t>((n_words + 1023) / 1024 + 1, (uint64_t)sms * 16);
     if (n_words) k_md_count<<<grid, 256, 0, st>>>(d_masks, n_words, ctr);
     static_assert(sizeof(MdCtr) == 32, "MdCtr is published as four 8-byte words");
-    CU(c, c->pub.reserve(64));
+    CU(c->err, c->pub.reserve(64));
     auto fetch_ctr = [&]() -> cudaError_t {  // counters -> mapped pinned memory -> h
         cudaError_t e1 = v2p::publish_words(c->pub.p, ctr, 4, st);
         if (e1 != cudaSuccess) return e1;
@@ -823,44 +748,45 @@ int v2p_sites_from_masks(v2p_catalogue* c, uint64_t n_records, uint64_t n_sample
         memcpy(&h, c->pub.p, sizeof h);
         return e1;
     };
-    CU(c, fetch_ctr());
+    CU(c->err, fetch_ctr());
     const uint64_t cap = h.n_bits;  // upper bound of the keys: every set bit
     uint32_t site_bits = 1, hap_bits = 1;
     while ((1ull << site_bits) < c->n_sites) ++site_bits;
     while ((1ull << hap_bits) < n_hap + 1) ++hap_bits;
-    if ((rc = need(c, c->md_keys[0], cap * 8 + 16)) || (rc = need(c, c->md_keys[1], cap * 8 + 16)) ||
-        (rc = need(c, c->md_uniq, cap * 8 + 16)) || (rc = need(c, c->md_sites, cap * 4 + 16)))
-        return rc;
+    CU(c->err, c->md_keys[0].need(cap * 8 + 16));
+    CU(c->err, c->md_keys[1].need(cap * 8 + 16));
+    CU(c->err, c->md_uniq.need(cap * 8 + 16));
+    CU(c->err, c->md_sites.need(cap * 4 + 16));
     uint64_t n_unique = 0;
     if (cap) {
         MdArgs a{d_masks, n_words, n_samples, words_per_cell, site_bits, (const uint64_t*)c->md_csq_begin.p,
                  (const int32_t*)c->md_csq_site.p, (uint64_t*)c->md_keys[0].p, ctr};
         k_md_emit<<<grid, 256, 0, st>>>(a);
-        CU(c, fetch_ctr());
+        CU(c->err, fetch_ctr());
         if (h.bad_record != ~0ull)
-            return cfail(c, V2P_ERR_SRC_OOB, "record %llu: a mask bit selects a consequence beyond the record's %llu (vcf_ds.rs:287)",
-                         h.bad_record, (unsigned long long)(csq_begin[h.bad_record + 1] - csq_begin[h.bad_record]));
+            return fail(c->err, V2P_ERR_SRC_OOB, "record %llu: a mask bit selects a consequence beyond the record's %llu (vcf_ds.rs:287)",
+                        h.bad_record, (unsigned long long)(csq_begin[h.bad_record + 1] - csq_begin[h.bad_record]));
         const uint64_t n_keys = h.cursor;
         if (n_keys) {
             cub::DoubleBuffer<uint64_t> db((uint64_t*)c->md_keys[0].p, (uint64_t*)c->md_keys[1].p);
             size_t tmp = 0;
-            CU(c, cub::DeviceRadixSort::SortKeys(nullptr, tmp, db, (int64_t)n_keys, 0, (int)(site_bits + hap_bits), st));
-            if ((rc = need(c, c->cub_tmp, tmp))) return rc;
-            CU(c, cub::DeviceRadixSort::SortKeys(c->cub_tmp.p, tmp, db, (int64_t)n_keys, 0, (int)(site_bits + hap_bits), st));
-            CU(c, cub::DeviceSelect::Unique(nullptr, tmp, db.Current(), (uint64_t*)c->md_uniq.p, &ctr->n_unique, (int64_t)n_keys, st));
-            if ((rc = need(c, c->cub_tmp, tmp))) return rc;
-            CU(c, cub::DeviceSelect::Unique(c->cub_tmp.p, tmp, db.Current(), (uint64_t*)c->md_uniq.p, &ctr->n_unique, (int64_t)n_keys, st));
-            CU(c, fetch_ctr());
+            CU(c->err, cub::DeviceRadixSort::SortKeys(nullptr, tmp, db, (int64_t)n_keys, 0, (int)(site_bits + hap_bits), st));
+            CU(c->err, c->cub_tmp.need(tmp));
+            CU(c->err, cub::DeviceRadixSort::SortKeys(c->cub_tmp.p, tmp, db, (int64_t)n_keys, 0, (int)(site_bits + hap_bits), st));
+            CU(c->err, cub::DeviceSelect::Unique(nullptr, tmp, db.Current(), (uint64_t*)c->md_uniq.p, &ctr->n_unique, (int64_t)n_keys, st));
+            CU(c->err, c->cub_tmp.need(tmp));
+            CU(c->err, cub::DeviceSelect::Unique(c->cub_tmp.p, tmp, db.Current(), (uint64_t*)c->md_uniq.p, &ctr->n_unique, (int64_t)n_keys, st));
+            CU(c->err, fetch_ctr());
             n_unique = h.n_unique;
         }
     }
     k_md_csr<<<blocks(std::max<uint64_t>(n_unique, n_hap + 1)), 256, 0, st>>>((const uint64_t*)c->md_uniq.p, ctr, n_hap, site_bits,
                                                                              (uint64_t*)c->md_begin.p, (uint32_t*)c->md_sites.p);
-    CU(c, cudaGetLastError());
-    CU(c, cudaEventRecord(c->ev1, st));
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaGetLastError());
+    CU(c->err, cudaEventRecord(c->ev1, st));
+    CU(c->err, cudaStreamSynchronize(st));
     float ms = 0;
-    CU(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+    CU(c->err, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
     out->n_hap = n_hap, out->n_sites = n_unique;
     out->site_begin = (const uint64_t*)c->md_begin.p, out->sites = (const uint32_t*)c->md_sites.p;
     out->decode_ms = ms;
@@ -871,8 +797,8 @@ int v2p_generate_tasks_from_lists(v2p_catalogue* c, const v2p_site_lists* lists,
     if (!c || !out || !lists || (lists->n_hap && !lists->site_begin)) return V2P_ERR_INVALID_ARG;
     memset(out, 0, sizeof *out);
     c->err.clear();
-    CU(c, cudaSetDevice(c->device));
-    CU(c, cudaEventRecord(c->ev0, c->stream));
+    CU(c->err, cudaSetDevice(c->device));
+    CU(c->err, cudaEventRecord(c->ev0, c->stream));
     return generate_on_device(c, lists->n_hap, lists->n_sites, lists->site_begin, lists->sites, flags, out);
 }
 
@@ -886,15 +812,19 @@ int generate_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, const u
     if (c->is_ins) return generate_ins_on_device(c, n_hap, n_sel, d_site_begin, d_sites, flags, out);
     cudaStream_t st = c->stream;
     int rc;
-    if ((rc = need(c, c->site_hap, n_sel * 4 + 16)) || (rc = need(c, c->flags, n_sel + 16)) || (rc = need(c, c->mut_dst, n_sel * 8 + 16)) ||
-        (rc = need(c, c->totals, 64)) || (rc = need(c, c->sel_err, 16)))
-        return rc;
-    for (int i = 0; i < 6; ++i)
-        if ((rc = need(c, c->scan_in[i], (n_sel + 1) * 8)) || (rc = need(c, c->scan_out[i], (n_sel + 1) * 8))) return rc;
+    CU(c->err, c->site_hap.need(n_sel * 4 + 16));
+    CU(c->err, c->flags.need(n_sel + 16));
+    CU(c->err, c->mut_dst.need(n_sel * 8 + 16));
+    CU(c->err, c->totals.need(64));
+    CU(c->err, c->sel_err.need(16));
+    for (int i = 0; i < 6; ++i) {
+        CU(c->err, c->scan_in[i].need((n_sel + 1) * 8));
+        CU(c->err, c->scan_out[i].need((n_sel + 1) * 8));
+    }
     const bool fasta = (flags & V2P_GEN_FASTA) != 0;
     if (fasta && (flags & V2P_GEN_ALIGNED))
-        return cfail(c, V2P_ERR_INVALID_ARG, "V2P_GEN_FASTA needs the packed layout (a file image cannot contain pad bytes)");
-    if (fasta && !c->has_names) return cfail(c, V2P_ERR_INVALID_ARG, "V2P_GEN_FASTA needs v2p_catalogue_set_names first");
+        return fail(c->err, V2P_ERR_INVALID_ARG, "V2P_GEN_FASTA needs the packed layout (a file image cannot contain pad bytes)");
+    if (fasta && !c->has_names) return fail(c->err, V2P_ERR_INVALID_ARG, "V2P_GEN_FASTA needs v2p_catalogue_set_names first");
     Cat cat{(const uint64_t*)c->tx_off.p, (const uint32_t*)c->tx.p, (const uint32_t*)c->pos.p, (const uint32_t*)c->rlen.p,
             (const uint32_t*)c->dlen.p, (const uint8_t*)c->cls.p, (const uint64_t*)c->doff.p, (const uint8_t*)c->pool.p,
             (const uint64_t*)c->name_off.p, (const uint8_t*)c->names.p};
@@ -903,7 +833,7 @@ int generate_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, const u
     s.sites = d_sites, s.site_begin = d_site_begin;
     s.site_hap = (uint32_t*)c->site_hap.p, s.flags = (uint8_t*)c->flags.p;
     s.n_cat = c->n_sites, s.bad = (unsigned long long*)c->sel_err.p;
-    CU(c, cudaMemsetAsync(s.bad, 0xFF, 8, st));
+    CU(c->err, cudaMemsetAsync(s.bad, 0xFF, 8, st));
     uint64_t** ins[6] = {&s.cnt, &s.slen, &s.acon, &s.newg, &s.shortc, &s.slotl};
     uint64_t** outs[6] = {&s.task_x, &s.l_x, &s.a_x, &s.g_x, &s.sh_x, &s.sl_x};
     for (int i = 0; i < 6; ++i) *ins[i] = (uint64_t*)c->scan_in[i].p, *outs[i] = (uint64_t*)c->scan_out[i].p;
@@ -911,37 +841,43 @@ int generate_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, const u
     s.fasta = fasta ? 1 : 0;
 
     for (int i = 0; i < 6; ++i)  // sentinel entry [n_sel] of every scan input
-        CU(c, cudaMemsetAsync((char*)c->scan_in[i].p + n_sel * 8, 0, 8, st));
+        CU(c->err, cudaMemsetAsync((char*)c->scan_in[i].p + n_sel * 8, 0, 8, st));
     if (n_sel) {
         k_tg_site_hap<<<blocks(n_sel), 256, 0, st>>>(s);
         k_tg_classify<<<blocks(n_sel), 256, 0, st>>>(s, cat);
     }
     for (int i = 0; i < 5; ++i)
-        if ((rc = xsum(c, *ins[i], *outs[i], n_sel + 1))) return rc;
+        if ((rc = exclusive_sum(c->err, c->cub_tmp, (const uint64_t*)*ins[i], *outs[i], n_sel + 1, st))) return rc;
     // totals: n_tasks, n_groups
-    CU(c, c->pub.reserve(64));
+    CU(c->err, c->pub.reserve(64));
     {
         v2p::PubList pl{};
         pl.src[0] = (const unsigned long long*)(s.task_x + n_sel), pl.src[1] = (const unsigned long long*)(s.g_x + n_sel);
         pl.src[2] = s.bad, pl.n = 3;
         v2p::k_publish_list<<<1, 32, 0, st>>>(c->pub.p, pl);
     }
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaStreamSynchronize(st));
     const uint64_t n_tasks = c->pub.p[0], n_groups = c->pub.p[1];
     if (c->pub.p[2] != ~0ull)
-        return cfail(c, V2P_ERR_INVALID_ARG, "site list entry %llu is not a catalogue site (< %llu) in strictly ascending order "
-                     "inside its haplotype", c->pub.p[2], (unsigned long long)c->n_sites);
+        return fail(c->err, V2P_ERR_INVALID_ARG, "site list entry %llu is not a catalogue site (< %llu) in strictly ascending order "
+                    "inside its haplotype", c->pub.p[2], (unsigned long long)c->n_sites);
 
     Grp g{};
     g.n_groups = n_groups;
-    if ((rc = need(c, c->g_first, (n_groups + 1) * 8)) || (rc = need(c, c->g_len, (n_groups + 1) * 8)) ||
-        (rc = need(c, c->g_slot, (n_groups + 1) * 8)) || (rc = need(c, c->g_slot_x, (n_groups + 1) * 8)) ||
-        (rc = need(c, c->g_hap, (n_groups + 1) * 4)) || (rc = need(c, c->g_tx, (n_groups + 1) * 4)) ||
-        (rc = need(c, c->ann_start, (n_groups + 1) * 8)) || (rc = need(c, c->ann_end, (n_groups + 1) * 8)) ||
-        (rc = need(c, c->tasks, (n_tasks + 1) * sizeof(v2p_task16))) || (rc = need(c, c->task_begin, (n_hap + 1) * 8)) ||
-        (rc = need(c, c->alt_base, (n_hap + 1) * 8)) || (rc = need(c, c->out_base, (n_hap + 1) * 8)) ||
-        (rc = need(c, c->alt_per_hap, (n_hap + 1) * 8)) || (rc = need(c, c->short_tot, (n_hap + 1) * 8)))
-        return rc;
+    CU(c->err, c->g_first.need((n_groups + 1) * 8));
+    CU(c->err, c->g_len.need((n_groups + 1) * 8));
+    CU(c->err, c->g_slot.need((n_groups + 1) * 8));
+    CU(c->err, c->g_slot_x.need((n_groups + 1) * 8));
+    CU(c->err, c->g_hap.need((n_groups + 1) * 4));
+    CU(c->err, c->g_tx.need((n_groups + 1) * 4));
+    CU(c->err, c->ann_start.need((n_groups + 1) * 8));
+    CU(c->err, c->ann_end.need((n_groups + 1) * 8));
+    CU(c->err, c->tasks.need((n_tasks + 1) * sizeof(v2p_task16)));
+    CU(c->err, c->task_begin.need((n_hap + 1) * 8));
+    CU(c->err, c->alt_base.need((n_hap + 1) * 8));
+    CU(c->err, c->out_base.need((n_hap + 1) * 8));
+    CU(c->err, c->alt_per_hap.need((n_hap + 1) * 8));
+    CU(c->err, c->short_tot.need((n_hap + 1) * 8));
     g.g_first = (uint64_t*)c->g_first.p, g.g_len = (uint64_t*)c->g_len.p, g.g_slot = (uint64_t*)c->g_slot.p;
     g.g_slot_x = (uint64_t*)c->g_slot_x.p, g.g_hap = (uint32_t*)c->g_hap.p, g.g_tx = (uint32_t*)c->g_tx.p;
     g.ann_start = (uint64_t*)c->ann_start.p, g.ann_end = (uint64_t*)c->ann_end.p;
@@ -952,14 +888,14 @@ int generate_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, const u
 
     k_tg_groups<<<blocks(n_sel + 1), 256, 0, st>>>(s, cat, g);
     k_tg_group_sizes<<<blocks(n_groups + 1), 256, 0, st>>>(s, cat, g);
-    if ((rc = xsum(c, g.g_slot, g.g_slot_x, n_groups + 1))) return rc;
+    if ((rc = exclusive_sum(c->err, c->cub_tmp, (const uint64_t*)g.g_slot, g.g_slot_x, n_groups + 1, st))) return rc;
     k_tg_hap_bases<<<blocks(n_hap + 1), 256, 0, st>>>(s, g, o);
     if (n_sel) k_tg_emit_tasks<<<blocks(n_sel), 256, 0, st>>>(s, cat, g, o);
     v2p::PubList pl{};
     if (s.aligned) {
-        if ((rc = xsum(c, s.slotl, s.sl_x, n_sel + 1))) return rc;
+        if ((rc = exclusive_sum(c->err, c->cub_tmp, (const uint64_t*)s.slotl, s.sl_x, n_sel + 1, st))) return rc;
         k_tg_alt_sizes<<<blocks(n_hap + 1), 256, 0, st>>>(s, o);
-        if ((rc = xsum(c, o.alt_per_hap, o.alt_base, n_hap + 1))) return rc;
+        if ((rc = exclusive_sum(c->err, c->cub_tmp, (const uint64_t*)o.alt_per_hap, o.alt_base, n_hap + 1, st))) return rc;
         pl.src[0] = (const unsigned long long*)(o.alt_base + n_hap);
     } else {
         pl.src[0] = (const unsigned long long*)(s.a_x + n_sel);
@@ -968,15 +904,16 @@ int generate_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, const u
     pl.src[2] = (const unsigned long long*)(s.sh_x + n_sel);  // FASTA: bytes of the name tape
     pl.n = 3;
     v2p::k_publish_list<<<1, 32, 0, st>>>(c->pub.p, pl);
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaStreamSynchronize(st));
     const uint64_t n_out = c->pub.p[1], n_alt = c->pub.p[0] + (fasta ? c->pub.p[2] : 0);
-    if ((rc = need(c, c->alt, n_alt + 64)) || (rc = need(c, c->out, n_out + 64))) return rc;
+    CU(c->err, c->alt.need(n_alt + 64));
+    CU(c->err, c->out.need(n_out + 64));
     o.alt = (uint8_t*)c->alt.p;
-    CU(c, cudaMemsetAsync(o.alt, '.', n_alt + 16, st));
+    CU(c->err, cudaMemsetAsync(o.alt, '.', n_alt + 16, st));
     if (n_sel) k_tg_emit_alt<<<blocks(n_sel), 256, 0, st>>>(s, cat, o);
-    CU(c, cudaEventRecord(c->ev1, st));
-    CU(c, cudaGetLastError());
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaEventRecord(c->ev1, st));
+    CU(c->err, cudaGetLastError());
+    CU(c->err, cudaStreamSynchronize(st));
     float ms = 0.f;
     cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 
@@ -1008,14 +945,18 @@ int generate_ins_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, con
     cudaStream_t st = c->stream;
     const bool fasta = (flags & V2P_GEN_FASTA) != 0;
     if (flags & V2P_GEN_ALIGNED)
-        return cfail(c, V2P_ERR_INVALID_ARG, "the general catalogue generates the reference's packed layout only (no V2P_GEN_ALIGNED)");
-    if (fasta && !c->has_names) return cfail(c, V2P_ERR_INVALID_ARG, "V2P_GEN_FASTA needs v2p_catalogue_set_names first");
+        return fail(c->err, V2P_ERR_INVALID_ARG, "the general catalogue generates the reference's packed layout only (no V2P_GEN_ALIGNED)");
+    if (fasta && !c->has_names) return fail(c->err, V2P_ERR_INVALID_ARG, "V2P_GEN_FASTA needs v2p_catalogue_set_names first");
     int rc;
-    if ((rc = need(c, c->site_hap, n_sel * 4 + 16)) || (rc = need(c, c->gi_newg, (n_sel + 1) * 8)) ||
-        (rc = need(c, c->gi_gx, (n_sel + 1) * 8)) || (rc = need(c, c->gi_err, 16)) || (rc = need(c, c->sel_err, 16)) || (rc = need(c, c->task_begin, (n_hap + 1) * 8)) ||
-        (rc = need(c, c->alt_base, (n_hap + 1) * 8)) || (rc = need(c, c->out_base, (n_hap + 1) * 8)))
-        return rc;
-    CU(c, c->pub.reserve(64));
+    CU(c->err, c->site_hap.need(n_sel * 4 + 16));
+    CU(c->err, c->gi_newg.need((n_sel + 1) * 8));
+    CU(c->err, c->gi_gx.need((n_sel + 1) * 8));
+    CU(c->err, c->gi_err.need(16));
+    CU(c->err, c->sel_err.need(16));
+    CU(c->err, c->task_begin.need((n_hap + 1) * 8));
+    CU(c->err, c->alt_base.need((n_hap + 1) * 8));
+    CU(c->err, c->out_base.need((n_hap + 1) * 8));
+    CU(c->err, c->pub.reserve(64));
     InsCat cat{(const uint64_t*)c->tx_off.p, (const uint32_t*)c->tx.p, (const uint8_t*)c->i_code.p, (const uint8_t*)c->i_flags.p,
                (const uint32_t*)c->i_pos_ref.p, (const uint32_t*)c->i_pos_res.p, (const uint32_t*)c->i_len.p,
                (const uint32_t*)c->dlen.p, (const uint64_t*)c->doff.p, (const uint8_t*)c->pool.p,
@@ -1027,10 +968,10 @@ int generate_ins_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, con
     g.err = (unsigned long long*)c->gi_err.p;
     g.fasta = fasta ? 1 : 0;
     g.skip_aborts = (flags & V2P_GEN_SKIP_ABORTS) ? 1 : 0;
-    CU(c, cudaMemsetAsync(g.err, 0xFF, 8, st));
-    CU(c, cudaMemsetAsync(g.err + 1, 0, 8, st));
+    CU(c->err, cudaMemsetAsync(g.err, 0xFF, 8, st));
+    CU(c->err, cudaMemsetAsync(g.err + 1, 0, 8, st));
     g.bad_site = (const unsigned long long*)c->sel_err.p;
-    CU(c, cudaMemsetAsync(c->sel_err.p, 0xFF, 8, st));
+    CU(c->err, cudaMemsetAsync(c->sel_err.p, 0xFF, 8, st));
     if (n_sel) {
         Sel sh{};
         sh.n_sel = n_sel, sh.n_hap = n_hap, sh.site_begin = d_site_begin, sh.site_hap = (uint32_t*)c->site_hap.p;
@@ -1038,23 +979,28 @@ int generate_ins_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, con
         k_tg_site_hap<<<blocks(n_sel), 256, 0, st>>>(sh);
     }
     k_ti_mark<<<blocks(n_sel + 1), 256, 0, st>>>(g, cat);
-    if ((rc = xsum(c, g.newg, g.g_x, n_sel + 1))) return rc;
+    if ((rc = exclusive_sum(c->err, c->cub_tmp, (const uint64_t*)g.newg, g.g_x, n_sel + 1, st))) return rc;
     {
         v2p::PubList pl{};
         pl.src[0] = (const unsigned long long*)(g.g_x + n_sel), pl.src[1] = g.bad_site, pl.n = 2;
         v2p::k_publish_list<<<1, 32, 0, st>>>(c->pub.p, pl);
     }
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaStreamSynchronize(st));
     const uint64_t G = c->pub.p[0];
     if (c->pub.p[1] != ~0ull)
-        return cfail(c, V2P_ERR_INVALID_ARG, "site list entry %llu is not a catalogue site (< %llu) in strictly ascending order "
-                     "inside its haplotype", c->pub.p[1], (unsigned long long)c->n_sites);
+        return fail(c->err, V2P_ERR_INVALID_ARG, "site list entry %llu is not a catalogue site (< %llu) in strictly ascending order "
+                    "inside its haplotype", c->pub.p[1], (unsigned long long)c->n_sites);
     g.n_groups = G;
-    if ((rc = need(c, c->gi_first, (G + 1) * 8)) || (rc = need(c, c->gi_size, (G + 1) * 8)) || (rc = need(c, c->gi_hap, (G + 1) * 4)) ||
-        (rc = need(c, c->gi_tx, (G + 1) * 4)) || (rc = need(c, c->gi_nsites, (G + 1) * 4)) || (rc = need(c, c->gi_status, G + 1)))
-        return rc;
-    for (int i = 0; i < 7; ++i)
-        if ((rc = need(c, c->gi_c[i], (G + 1) * 8)) || (rc = need(c, c->gi_x[i], (G + 1) * 8))) return rc;
+    CU(c->err, c->gi_first.need((G + 1) * 8));
+    CU(c->err, c->gi_size.need((G + 1) * 8));
+    CU(c->err, c->gi_hap.need((G + 1) * 4));
+    CU(c->err, c->gi_tx.need((G + 1) * 4));
+    CU(c->err, c->gi_nsites.need((G + 1) * 4));
+    CU(c->err, c->gi_status.need(G + 1));
+    for (int i = 0; i < 7; ++i) {
+        CU(c->err, c->gi_c[i].need((G + 1) * 8));
+        CU(c->err, c->gi_x[i].need((G + 1) * 8));
+    }
     g.g_first = (uint64_t*)c->gi_first.p, g.g_size = (uint64_t*)c->gi_size.p, g.g_hap = (uint32_t*)c->gi_hap.p;
     g.g_tx = (uint32_t*)c->gi_tx.p, g.g_nsites = (uint32_t*)c->gi_nsites.p, g.g_status = (uint8_t*)c->gi_status.p;
     uint64_t** cin[7] = {&g.c_tasks, &g.c_alt, &g.c_name, &g.c_adv, &g.c_tape, &g.c_rows, &g.c_skip};
@@ -1062,7 +1008,7 @@ int generate_ins_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, con
     for (int i = 0; i < 7; ++i) *cin[i] = (uint64_t*)c->gi_c[i].p, *cx[i] = (uint64_t*)c->gi_x[i].p;
     k_ti_count<<<blocks(n_sel + 1), 256, 0, st>>>(g, cat);
     for (int i = 0; i < 7; ++i)
-        if ((rc = xsum(c, *cin[i], *cx[i], G + 1))) return rc;
+        if ((rc = exclusive_sum(c->err, c->cub_tmp, (const uint64_t*)*cin[i], *cx[i], G + 1, st))) return rc;
     {
         v2p::PubList pl{};
         const uint64_t* tot[8] = {g.x_tasks + G, g.x_alt + G, g.x_name + G, g.x_tape + G, g.x_rows + G, g.x_skip + G,
@@ -1071,29 +1017,32 @@ int generate_ins_on_device(v2p_catalogue* c, uint64_t n_hap, uint64_t n_sel, con
         pl.n = 8;
         v2p::k_publish_list<<<1, 32, 0, st>>>(c->pub.p, pl);
     }
-    CU(c, cudaGetLastError());
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaGetLastError());
+    CU(c->err, cudaStreamSynchronize(st));
     const uint64_t n_tasks = c->pub.p[0], n_alt = c->pub.p[1] + c->pub.p[2], n_out = c->pub.p[3], n_rows = c->pub.p[4],
                    n_skip = c->pub.p[5], bad = c->pub.p[6], n_abort = c->pub.p[7];
     if (bad != ~0ull && !g.skip_aborts) {  // name the transcript the reference aborts on
         uint32_t hh = 0, tt = 0;
         cudaMemcpy(&hh, g.g_hap + bad, 4, cudaMemcpyDeviceToHost);
         cudaMemcpy(&tt, g.g_tx + bad, 4, cudaMemcpyDeviceToHost);
-        return cfail(c, V2P_ERR_TASKGEN,
-                     "haplotype %u transcript %u: the reference aborts while generating its tasks (usize underflow in "
-                     "add_till_next_ins / add_last_instruction, or a negative result size)", hh, tt);
+        return fail(c->err, V2P_ERR_TASKGEN,
+                    "haplotype %u transcript %u: the reference aborts while generating its tasks (usize underflow in "
+                    "add_till_next_ins / add_last_instruction, or a negative result size)", hh, tt);
     }
-    if ((rc = need(c, c->tasks, (n_tasks + 1) * sizeof(v2p_task16))) || (rc = need(c, c->alt, n_alt + 64)) ||
-        (rc = need(c, c->out, n_out + 64)) || (rc = need(c, c->g_hap, (n_rows + 1) * 4)) || (rc = need(c, c->g_tx, (n_rows + 1) * 4)) ||
-        (rc = need(c, c->ann_start, (n_rows + 1) * 8)) || (rc = need(c, c->ann_end, (n_rows + 1) * 8)))
-        return rc;
+    CU(c->err, c->tasks.need((n_tasks + 1) * sizeof(v2p_task16)));
+    CU(c->err, c->alt.need(n_alt + 64));
+    CU(c->err, c->out.need(n_out + 64));
+    CU(c->err, c->g_hap.need((n_rows + 1) * 4));
+    CU(c->err, c->g_tx.need((n_rows + 1) * 4));
+    CU(c->err, c->ann_start.need((n_rows + 1) * 8));
+    CU(c->err, c->ann_end.need((n_rows + 1) * 8));
     InsOut o{(v2p_task16*)c->tasks.p, (uint64_t*)c->task_begin.p, (uint64_t*)c->alt_base.p, (uint64_t*)c->out_base.p,
              (uint8_t*)c->alt.p, (uint32_t*)c->g_hap.p, (uint32_t*)c->g_tx.p, (uint64_t*)c->ann_start.p, (uint64_t*)c->ann_end.p};
     k_ti_hap_bases<<<blocks(n_hap + 1), 256, 0, st>>>(g, o);
     if (G) k_ti_emit<<<blocks(G), 256, 0, st>>>(g, cat, o);
-    CU(c, cudaEventRecord(c->ev1, st));
-    CU(c, cudaGetLastError());
-    CU(c, cudaStreamSynchronize(st));
+    CU(c->err, cudaEventRecord(c->ev1, st));
+    CU(c->err, cudaGetLastError());
+    CU(c->err, cudaStreamSynchronize(st));
     float ms = 0.f;
     cudaEventElapsedTime(&ms, c->ev0, c->ev1);
     out->batch.task_begin = o.task_begin, out->batch.tasks = o.tasks;

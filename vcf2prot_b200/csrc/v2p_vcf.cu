@@ -26,7 +26,6 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <cub/block/block_scan.cuh>
@@ -35,17 +34,15 @@
 #include <string>
 #include <vector>
 
+#include "v2p_hostres.cuh"
 #include "v2p_inflate.cuh"
 #include "v2p_mapped.cuh"
 #include "v2p_vcf.h"
 #include "v2p_vcf_bgzf.h"
 
-namespace {
+using namespace v2p;
 
-struct Buf {
-    void* p = nullptr;
-    size_t cap = 0;
-};
+namespace {
 
 constexpr int kThreads = 256;
 constexpr int kChunksPerThread = 4;                                          // 16-byte chunks, contiguous per thread
@@ -415,87 +412,35 @@ __global__ void k_check(ParseArgs a) {
 
 }  // namespace
 
-struct HostBuf {  // pinned host memory
-    void* p = nullptr;
-    size_t cap = 0;
-};
-
 struct v2p_vcf {
     int device = 0;
     int sms = 148;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[7] = {};
     std::string err;
-    v2p::MappedBuf pub;
+    MappedBuf pub;
     // the loaded text and its index
     bool loaded = false;
     const uint8_t* text = nullptr;  // owned copy (buf_text) or the caller's device text
     uint64_t n_bytes = 0, n_lines = 0, n_samples = 0;
-    Buf buf_text, tile_cnt, tile_x, starts, ends, is_data, data_x, line_begin, line_end, line_no, cells_begin, has_cells, ctr, cub_tmp;
+    DevBuf buf_text, tile_cnt, tile_x, starts, ends, is_data, data_x, line_begin, line_end, line_no, cells_begin, has_cells, ctr, cub_tmp;
     std::vector<uint64_t> h_line_begin, h_cells_begin;
     // BGZF input: compressed bytes, block table; columns 1-9 for the host
-    Buf comp, blocks, fixed_len, fixed_x, fixed;
+    DevBuf comp, blocks, fixed_len, fixed_x, fixed;
     std::vector<BgzfBlock> h_blocks;
-    HostBuf h_head, h_fixed, h_fixed_begin;
+    PinnedBuf h_head, h_fixed, h_fixed_begin;
     // parse
-    Buf rec_line, n_seg, seg_begin, seg_tabs, seg_tab_x, seg_err, seg_rec, masks;
+    DevBuf rec_line, n_seg, seg_begin, seg_tabs, seg_tab_x, seg_err, seg_rec, masks;
 };
 
 namespace {
 
-int vfail(v2p_vcf* v, int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (v) v->err = buf;
-    return code;
-}
-#define CU(v, call)                                                                                                  \
-    do {                                                                                                             \
-        cudaError_t _st = (call);                                                                                    \
-        if (_st != cudaSuccess) return vfail((v), V2P_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_st), \
-                                             __FILE__, __LINE__);                                                     \
-    } while (0)
-
-int need(v2p_vcf* v, Buf& b, size_t bytes) {
-    bytes = bytes < 256 ? 256 : bytes;
-    if (b.cap >= bytes) return V2P_OK;
-    if (b.p) CU(v, cudaFree(b.p));
-    b.p = nullptr, b.cap = 0;
-    CU(v, cudaMalloc(&b.p, bytes + bytes / 8));
-    b.cap = bytes + bytes / 8;
-    return V2P_OK;
-}
-
-int xsum(v2p_vcf* v, const uint64_t* in, uint64_t* out, uint64_t n) {
-    size_t tmp = 0;
-    CU(v, cub::DeviceScan::ExclusiveSum(nullptr, tmp, in, out, (int64_t)n, v->stream));
-    int rc = need(v, v->cub_tmp, tmp);
-    if (rc) return rc;
-    CU(v, cub::DeviceScan::ExclusiveSum(v->cub_tmp.p, tmp, in, out, (int64_t)n, v->stream));
-    return V2P_OK;
-}
-
 // device words -> mapped host memory -> dst, after everything queued so far
 int fetch(v2p_vcf* v, const void* src, uint64_t n_words, void* dst) {
-    CU(v, v->pub.reserve(n_words));
-    CU(v, v2p::publish_words(v->pub.p, src, n_words, v->stream));
-    CU(v, cudaStreamSynchronize(v->stream));
+    CU(v->err, v->pub.reserve(n_words));
+    CU(v->err, v2p::publish_words(v->pub.p, src, n_words, v->stream));
+    CU(v->err, cudaStreamSynchronize(v->stream));
     memcpy(dst, v->pub.p, n_words * 8);
-    return V2P_OK;
-}
-
-inline unsigned blocks(uint64_t n) { return (unsigned)((n + 255) / 256); }
-
-int hneed(v2p_vcf* v, HostBuf& b, size_t bytes) {
-    bytes = bytes < 256 ? 256 : bytes;
-    if (b.cap >= bytes) return V2P_OK;
-    if (b.p) CU(v, cudaFreeHost(b.p));
-    b.p = nullptr, b.cap = 0;
-    CU(v, cudaHostAlloc(&b.p, bytes + bytes / 8, cudaHostAllocDefault));
-    b.cap = bytes + bytes / 8;
     return V2P_OK;
 }
 
@@ -506,31 +451,35 @@ int index_text(v2p_vcf* v, uint64_t n, cudaEvent_t done, LoadCtr& h) {
     int rc;
     const uint64_t n_tiles = (n + kTile - 1) / kTile;
     h = LoadCtr{0, kNone, 0, 0, 0};
-    if ((rc = need(v, v->ctr, sizeof(LoadCtr))) || (rc = need(v, v->tile_cnt, (n_tiles + 1) * 8)) ||
-        (rc = need(v, v->tile_x, (n_tiles + 1) * 8)))
-        return rc;
+    CU(v->err, v->ctr.need(sizeof(LoadCtr)));
+    CU(v->err, v->tile_cnt.need((n_tiles + 1) * 8));
+    CU(v->err, v->tile_x.need((n_tiles + 1) * 8));
     LoadCtr* ctr = (LoadCtr*)v->ctr.p;
-    CU(v, cudaMemcpyAsync(ctr, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    CU(v->err, cudaMemcpyAsync(ctr, &h, sizeof h, cudaMemcpyHostToDevice, st));
     uint64_t n_nl = 0;
     if (n) {
         k_nl_count<<<(unsigned)n_tiles, kThreads, 0, st>>>(v->text, n, (uint64_t*)v->tile_cnt.p, n_tiles);
-        if ((rc = xsum(v, (const uint64_t*)v->tile_cnt.p, (uint64_t*)v->tile_x.p, n_tiles + 1))) return rc;
+        if ((rc = exclusive_sum(v->err, v->cub_tmp, (const uint64_t*)v->tile_cnt.p, (uint64_t*)v->tile_x.p, n_tiles + 1, st))) return rc;
         if ((rc = fetch(v, (const uint64_t*)v->tile_x.p + n_tiles, 1, &n_nl))) return rc;
     }
     const uint64_t n_raw = n ? n_nl + 1 : 0;
-    if (n_raw >> 32) return vfail(v, V2P_ERR_INVALID_ARG, "more than 2^32 lines");
-    if ((rc = need(v, v->starts, (n_raw + 1) * 8)) || (rc = need(v, v->ends, (n_raw + 1) * 8)) ||
-        (rc = need(v, v->is_data, (n_raw + 1) * 8)) || (rc = need(v, v->data_x, (n_raw + 1) * 8)) ||
-        (rc = need(v, v->line_begin, n_raw * 8)) || (rc = need(v, v->line_end, n_raw * 8)) || (rc = need(v, v->line_no, n_raw * 4)) ||
-        (rc = need(v, v->cells_begin, n_raw * 8)) || (rc = need(v, v->has_cells, n_raw)))
-        return rc;
+    if (n_raw >> 32) return fail(v->err, V2P_ERR_INVALID_ARG, "more than 2^32 lines");
+    CU(v->err, v->starts.need((n_raw + 1) * 8));
+    CU(v->err, v->ends.need((n_raw + 1) * 8));
+    CU(v->err, v->is_data.need((n_raw + 1) * 8));
+    CU(v->err, v->data_x.need((n_raw + 1) * 8));
+    CU(v->err, v->line_begin.need(n_raw * 8));
+    CU(v->err, v->line_end.need(n_raw * 8));
+    CU(v->err, v->line_no.need(n_raw * 4));
+    CU(v->err, v->cells_begin.need(n_raw * 8));
+    CU(v->err, v->has_cells.need(n_raw));
     if (n) {
         const uint64_t* starts = (const uint64_t*)v->starts.p;
         k_nl_emit<<<(unsigned)n_tiles, kThreads, 0, st>>>(v->text, n, (const uint64_t*)v->tile_x.p, (uint64_t*)v->starts.p);
         k_classify<<<blocks(n_raw + 1), 256, 0, st>>>(v->text, n, starts, n_raw, (uint64_t*)v->is_data.p, (uint64_t*)v->ends.p, ctr);
         k_header_range<<<1, 1, 0, st>>>(starts, (const uint64_t*)v->ends.p, ctr);
         k_header_tabs<<<(unsigned)v->sms, 256, 0, st>>>(v->text, ctr);
-        if ((rc = xsum(v, (const uint64_t*)v->is_data.p, (uint64_t*)v->data_x.p, n_raw + 1))) return rc;
+        if ((rc = exclusive_sum(v->err, v->cub_tmp, (const uint64_t*)v->is_data.p, (uint64_t*)v->data_x.p, n_raw + 1, st))) return rc;
         k_compact<<<blocks(n_raw), 256, 0, st>>>(starts, (const uint64_t*)v->ends.p, (const uint64_t*)v->is_data.p,
                                                  (const uint64_t*)v->data_x.p, n_raw, (uint64_t*)v->line_begin.p,
                                                  (uint64_t*)v->line_end.p, (uint32_t*)v->line_no.p, ctr);
@@ -538,19 +487,19 @@ int index_text(v2p_vcf* v, uint64_t n, cudaEvent_t done, LoadCtr& h) {
         k_find_cells<<<(unsigned)std::min<uint64_t>((n_raw + 7) / 8, (uint64_t)v->sms * 32), 256, 0, st>>>(
             v->text, (const uint64_t*)v->line_begin.p, (const uint64_t*)v->line_end.p, ctr, (uint64_t*)v->cells_begin.p,
             (uint8_t*)v->has_cells.p);
-        CU(v, cudaGetLastError());
+        CU(v->err, cudaGetLastError());
     }
-    CU(v, cudaEventRecord(done, st));
+    CU(v->err, cudaEventRecord(done, st));
     static_assert(sizeof(LoadCtr) == 40, "LoadCtr is published as five 8-byte words");
     if ((rc = fetch(v, ctr, 5, &h))) return rc;
-    if (h.chrom == kNone) return vfail(v, V2P_ERR_VCF_PARSE, "no #CHROM line: the number of samples is unknown");
+    if (h.chrom == kNone) return fail(v->err, V2P_ERR_VCF_PARSE, "no #CHROM line: the number of samples is unknown");
     v->n_lines = h.n_data, v->n_bytes = n, v->n_samples = h.tabs >= 9 ? h.tabs - 8 : 0;
     v->h_line_begin.resize(v->n_lines), v->h_cells_begin.resize(v->n_lines);
     if (v->n_lines) {
-        CU(v, cudaMemcpyAsync(v->h_line_begin.data(), v->line_begin.p, v->n_lines * 8, cudaMemcpyDeviceToHost, st));
-        CU(v, cudaMemcpyAsync(v->h_cells_begin.data(), v->cells_begin.p, v->n_lines * 8, cudaMemcpyDeviceToHost, st));
+        CU(v->err, cudaMemcpyAsync(v->h_line_begin.data(), v->line_begin.p, v->n_lines * 8, cudaMemcpyDeviceToHost, st));
+        CU(v->err, cudaMemcpyAsync(v->h_cells_begin.data(), v->cells_begin.p, v->n_lines * 8, cudaMemcpyDeviceToHost, st));
     }
-    CU(v, cudaStreamSynchronize(st));
+    CU(v->err, cudaStreamSynchronize(st));
     return V2P_OK;
 }
 
@@ -633,19 +582,10 @@ void v2p_vcf_destroy(v2p_vcf* v) {
     if (!v) return;
     cudaSetDevice(v->device);
     if (v->stream) cudaStreamSynchronize(v->stream);
-    Buf* all[] = {&v->buf_text, &v->tile_cnt, &v->tile_x, &v->starts, &v->ends, &v->is_data, &v->data_x, &v->line_begin,
-                  &v->line_end, &v->line_no, &v->cells_begin, &v->has_cells, &v->ctr, &v->cub_tmp, &v->rec_line, &v->n_seg,
-                  &v->seg_begin, &v->seg_tabs, &v->seg_tab_x, &v->seg_err, &v->seg_rec, &v->masks, &v->comp, &v->blocks,
-                  &v->fixed_len, &v->fixed_x, &v->fixed};
-    for (Buf* b : all)
-        if (b->p) cudaFree(b->p);
-    for (HostBuf* b : {&v->h_head, &v->h_fixed, &v->h_fixed_begin})
-        if (b->p) cudaFreeHost(b->p);
-    v->pub.release();
     for (cudaEvent_t e : v->ev)
         if (e) cudaEventDestroy(e);
     if (v->stream) cudaStreamDestroy(v->stream);
-    delete v;
+    delete v;  // frees every buffer
 }
 
 const char* v2p_vcf_last_error(v2p_vcf* v) { return v ? v->err.c_str() : "vcf object is NULL"; }
@@ -655,27 +595,26 @@ int v2p_vcf_load(v2p_vcf* v, const uint8_t* text, uint64_t n_bytes, uint32_t fla
     memset(out, 0, sizeof *out);
     v->err.clear();
     v->loaded = false;
-    if (flags & ~V2P_FLAG_DEVICE_PTRS) return vfail(v, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
-    if (n_bytes && !text) return vfail(v, V2P_ERR_INVALID_ARG, "text is NULL");
+    if (flags & ~V2P_FLAG_DEVICE_PTRS) return fail(v->err, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
+    if (n_bytes && !text) return fail(v->err, V2P_ERR_INVALID_ARG, "text is NULL");
     const bool dev = flags & V2P_FLAG_DEVICE_PTRS;
-    if (dev && ((uintptr_t)text & 15)) return vfail(v, V2P_ERR_INVALID_ARG, "device text must be 16-byte aligned");
-    CU(v, cudaSetDevice(v->device));
+    if (dev && ((uintptr_t)text & 15)) return fail(v->err, V2P_ERR_INVALID_ARG, "device text must be 16-byte aligned");
+    CU(v->err, cudaSetDevice(v->device));
     cudaStream_t st = v->stream;
     int rc;
-    CU(v, cudaEventRecord(v->ev[0], st));
+    CU(v->err, cudaEventRecord(v->ev[0], st));
     if (dev) {
         v->text = text;
     } else {
-        if ((rc = need(v, v->buf_text, n_bytes + 16))) return rc;
-        if (n_bytes) CU(v, cudaMemcpyAsync(v->buf_text.p, text, n_bytes, cudaMemcpyHostToDevice, st));
+        CU(v->err, upload(v->buf_text, text, n_bytes, st));
         v->text = (const uint8_t*)v->buf_text.p;
     }
-    CU(v, cudaEventRecord(v->ev[1], st));
+    CU(v->err, cudaEventRecord(v->ev[1], st));
     LoadCtr h;
     if ((rc = index_text(v, n_bytes, v->ev[2], h))) return rc;
     float h2d = 0, idx = 0;
-    CU(v, cudaEventElapsedTime(&h2d, v->ev[0], v->ev[1]));
-    CU(v, cudaEventElapsedTime(&idx, v->ev[1], v->ev[2]));
+    CU(v->err, cudaEventElapsedTime(&h2d, v->ev[0], v->ev[1]));
+    CU(v->err, cudaEventElapsedTime(&idx, v->ev[1], v->ev[2]));
     fill_lines(v, h, out);
     out->h2d_bytes = dev ? 0 : n_bytes, out->h2d_ms = h2d, out->index_ms = idx;
     v->loaded = true;
@@ -688,39 +627,38 @@ int v2p_vcf_load_bgzf(v2p_vcf* v, const uint8_t* data, uint64_t n_bytes, uint32_
     memset(bz, 0, sizeof *bz);
     v->err.clear();
     v->loaded = false;
-    if (flags & V2P_FLAG_DEVICE_PTRS) return vfail(v, V2P_ERR_INVALID_ARG, "BGZF input must be host memory (V2P_FLAG_DEVICE_PTRS)");
-    if (flags) return vfail(v, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
-    if (n_bytes && !data) return vfail(v, V2P_ERR_INVALID_ARG, "data is NULL");
-    CU(v, cudaSetDevice(v->device));
+    if (flags & V2P_FLAG_DEVICE_PTRS) return fail(v->err, V2P_ERR_INVALID_ARG, "BGZF input must be host memory (V2P_FLAG_DEVICE_PTRS)");
+    if (flags) return fail(v->err, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
+    if (n_bytes && !data) return fail(v->err, V2P_ERR_INVALID_ARG, "data is NULL");
+    CU(v->err, cudaSetDevice(v->device));
     cudaStream_t st = v->stream;
     int rc;
     // the upload runs while the host walks the block headers
-    CU(v, cudaEventRecord(v->ev[0], st));
-    if ((rc = need(v, v->comp, n_bytes + 16))) return rc;
-    if (n_bytes) CU(v, cudaMemcpyAsync(v->comp.p, data, n_bytes, cudaMemcpyHostToDevice, st));
-    CU(v, cudaEventRecord(v->ev[1], st));
+    CU(v->err, cudaEventRecord(v->ev[0], st));
+    CU(v->err, upload(v->comp, data, n_bytes, st));
+    CU(v->err, cudaEventRecord(v->ev[1], st));
     std::vector<uint64_t> at;
     uint64_t text_bytes = 0;
     char why[160] = "";
     const bool walked = walk_bgzf(data, n_bytes, v->h_blocks, at, text_bytes, why, sizeof why);
     const uint64_t n_blk = v->h_blocks.size();
-    if ((rc = need(v, v->blocks, n_blk * sizeof(BgzfBlock))) || (rc = need(v, v->buf_text, text_bytes + 16)) ||
-        (rc = need(v, v->ctr, sizeof(LoadCtr))))
-        return rc;
-    if (n_blk) CU(v, cudaMemcpyAsync(v->blocks.p, v->h_blocks.data(), n_blk * sizeof(BgzfBlock), cudaMemcpyHostToDevice, st));
+    CU(v->err, v->blocks.need(n_blk * sizeof(BgzfBlock)));
+    CU(v->err, v->buf_text.need(text_bytes + 16));
+    CU(v->err, v->ctr.need(sizeof(LoadCtr)));
+    if (n_blk) CU(v->err, cudaMemcpyAsync(v->blocks.p, v->h_blocks.data(), n_blk * sizeof(BgzfBlock), cudaMemcpyHostToDevice, st));
     unsigned long long* ekey = (unsigned long long*)v->ctr.p;
-    CU(v, cudaMemsetAsync(ekey, 0xff, 8, st));
+    CU(v->err, cudaMemsetAsync(ekey, 0xff, 8, st));
     v->text = (const uint8_t*)v->buf_text.p;
-    CU(v, cudaEventRecord(v->ev[2], st));
+    CU(v->err, cudaEventRecord(v->ev[2], st));
     if (n_blk) {
         int per_sm = 1;
-        CU(v, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_inflate, kInfWarps * 32, 0));
+        CU(v->err, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_inflate, kInfWarps * 32, 0));
         const uint64_t grid = std::min<uint64_t>((uint64_t)v->sms * std::max(per_sm, 1), (n_blk + kInfWarps - 1) / kInfWarps);
         k_inflate<<<(unsigned)grid, kInfWarps * 32, 0, st>>>((const uint8_t*)v->comp.p, (const BgzfBlock*)v->blocks.p, n_blk,
                                                              (uint8_t*)v->buf_text.p, ekey);
-        CU(v, cudaGetLastError());
+        CU(v->err, cudaGetLastError());
     }
-    CU(v, cudaEventRecord(v->ev[3], st));
+    CU(v->err, cudaEventRecord(v->ev[3], st));
     unsigned long long key = kNone;
     if ((rc = fetch(v, ekey, 1, &key))) return rc;
     // blocks before a bad header were inflated: a bad one among them comes first in file order
@@ -729,37 +667,40 @@ int v2p_vcf_load_bgzf(v2p_vcf* v, const uint8_t* data, uint64_t n_bytes, uint32_
         const unsigned cls = key != kNone ? (unsigned)(key & 7) : (unsigned)BGZF_HEADER;
         const unsigned long long off = at[b];
         if (cls == BGZF_HEADER)
-            return vfail(v, V2P_ERR_BGZF, "BGZF block %llu at byte %llu: %s (%s)", (unsigned long long)b, off, kBgzfWhat[cls], why);
-        return vfail(v, V2P_ERR_BGZF, "BGZF block %llu at byte %llu: %s", (unsigned long long)b, off, kBgzfWhat[cls]);
+            return fail(v->err, V2P_ERR_BGZF, "BGZF block %llu at byte %llu: %s (%s)", (unsigned long long)b, off, kBgzfWhat[cls], why);
+        return fail(v->err, V2P_ERR_BGZF, "BGZF block %llu at byte %llu: %s", (unsigned long long)b, off, kBgzfWhat[cls]);
     }
-    CU(v, cudaEventRecord(v->ev[4], st));
+    CU(v->err, cudaEventRecord(v->ev[4], st));
     LoadCtr h;
     if ((rc = index_text(v, text_bytes, v->ev[5], h))) return rc;
     // columns 1-9 of every data line and the header lines back to the host
     const uint64_t nl = v->n_lines;
     uint64_t n_fixed = 0;
     for (uint64_t l = 0; l < nl; ++l) n_fixed += v->h_cells_begin[l] - v->h_line_begin[l];
-    if ((rc = need(v, v->fixed_len, (nl + 1) * 8)) || (rc = need(v, v->fixed_x, (nl + 1) * 8)) || (rc = need(v, v->fixed, n_fixed)) ||
-        (rc = hneed(v, v->h_fixed_begin, (nl + 1) * 8)) || (rc = hneed(v, v->h_fixed, n_fixed)) || (rc = hneed(v, v->h_head, h.he)))
-        return rc;
+    CU(v->err, v->fixed_len.need((nl + 1) * 8));
+    CU(v->err, v->fixed_x.need((nl + 1) * 8));
+    CU(v->err, v->fixed.need(n_fixed));
+    CU(v->err, v->h_fixed_begin.need((nl + 1) * 8));
+    CU(v->err, v->h_fixed.need(n_fixed));
+    CU(v->err, v->h_head.need(h.he));
     const uint64_t* lb = (const uint64_t*)v->line_begin.p;
     const uint64_t* cb = (const uint64_t*)v->cells_begin.p;
     k_fixed_len<<<blocks(nl + 1), 256, 0, st>>>(lb, cb, nl, (uint64_t*)v->fixed_len.p);
-    if ((rc = xsum(v, (const uint64_t*)v->fixed_len.p, (uint64_t*)v->fixed_x.p, nl + 1))) return rc;
+    if ((rc = exclusive_sum(v->err, v->cub_tmp, (const uint64_t*)v->fixed_len.p, (uint64_t*)v->fixed_x.p, nl + 1, st))) return rc;
     if (nl)
         k_fixed<<<(unsigned)std::min<uint64_t>((nl + 7) / 8, (uint64_t)v->sms * 32), 256, 0, st>>>(v->text, lb, cb, (const uint64_t*)v->fixed_x.p,
                                                                                                    nl, (uint8_t*)v->fixed.p);
-    CU(v, cudaGetLastError());
-    CU(v, cudaMemcpyAsync(v->h_fixed_begin.p, v->fixed_x.p, (nl + 1) * 8, cudaMemcpyDeviceToHost, st));
-    if (n_fixed) CU(v, cudaMemcpyAsync(v->h_fixed.p, v->fixed.p, n_fixed, cudaMemcpyDeviceToHost, st));
-    if (h.he) CU(v, cudaMemcpyAsync(v->h_head.p, v->text, h.he, cudaMemcpyDeviceToHost, st));
-    CU(v, cudaEventRecord(v->ev[6], st));
-    CU(v, cudaStreamSynchronize(st));
+    CU(v->err, cudaGetLastError());
+    CU(v->err, cudaMemcpyAsync(v->h_fixed_begin.p, v->fixed_x.p, (nl + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (n_fixed) CU(v->err, cudaMemcpyAsync(v->h_fixed.p, v->fixed.p, n_fixed, cudaMemcpyDeviceToHost, st));
+    if (h.he) CU(v->err, cudaMemcpyAsync(v->h_head.p, v->text, h.he, cudaMemcpyDeviceToHost, st));
+    CU(v->err, cudaEventRecord(v->ev[6], st));
+    CU(v->err, cudaStreamSynchronize(st));
     float h2d = 0, inf = 0, idx = 0, fix = 0;
-    CU(v, cudaEventElapsedTime(&h2d, v->ev[0], v->ev[1]));
-    CU(v, cudaEventElapsedTime(&inf, v->ev[2], v->ev[3]));
-    CU(v, cudaEventElapsedTime(&idx, v->ev[4], v->ev[5]));
-    CU(v, cudaEventElapsedTime(&fix, v->ev[5], v->ev[6]));
+    CU(v->err, cudaEventElapsedTime(&h2d, v->ev[0], v->ev[1]));
+    CU(v->err, cudaEventElapsedTime(&inf, v->ev[2], v->ev[3]));
+    CU(v->err, cudaEventElapsedTime(&idx, v->ev[4], v->ev[5]));
+    CU(v->err, cudaEventElapsedTime(&fix, v->ev[5], v->ev[6]));
     fill_lines(v, h, out);
     out->h2d_bytes = n_bytes, out->h2d_ms = h2d, out->index_ms = idx;
     bz->n_blocks = n_blk, bz->text_bytes = text_bytes, bz->text = v->text;
@@ -773,22 +714,23 @@ int v2p_vcf_parse_masks(v2p_vcf* v, uint64_t n_records, const uint64_t* rec_line
     if (!v || !out) return V2P_ERR_INVALID_ARG;
     memset(out, 0, sizeof *out);
     v->err.clear();
-    if (!v->loaded) return vfail(v, V2P_ERR_INVALID_ARG, "no text loaded (v2p_vcf_load failed or was not called)");
-    if (flags) return vfail(v, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
-    if (n_records && !rec_line) return vfail(v, V2P_ERR_INVALID_ARG, "rec_line is NULL");
+    if (!v->loaded) return fail(v->err, V2P_ERR_INVALID_ARG, "no text loaded (v2p_vcf_load failed or was not called)");
+    if (flags) return fail(v->err, V2P_ERR_INVALID_ARG, "unknown flags 0x%x", flags);
+    if (n_records && !rec_line) return fail(v->err, V2P_ERR_INVALID_ARG, "rec_line is NULL");
     for (uint64_t r = 0; r < n_records; ++r)
         if (rec_line[r] >= v->n_lines)
-            return vfail(v, V2P_ERR_INVALID_ARG, "rec_line[%llu] = %llu: the text has %llu data lines", (unsigned long long)r,
-                         (unsigned long long)rec_line[r], (unsigned long long)v->n_lines);
-    if (n_records >> 32) return vfail(v, V2P_ERR_INVALID_ARG, "more than 2^32 records");
-    CU(v, cudaSetDevice(v->device));
+            return fail(v->err, V2P_ERR_INVALID_ARG, "rec_line[%llu] = %llu: the text has %llu data lines", (unsigned long long)r,
+                        (unsigned long long)rec_line[r], (unsigned long long)v->n_lines);
+    if (n_records >> 32) return fail(v->err, V2P_ERR_INVALID_ARG, "more than 2^32 records");
+    CU(v->err, cudaSetDevice(v->device));
     cudaStream_t st = v->stream;
     int rc;
-    CU(v, cudaEventRecord(v->ev[0], st));
-    if ((rc = need(v, v->rec_line, n_records * 8)) || (rc = need(v, v->n_seg, (n_records + 1) * 8)) ||
-        (rc = need(v, v->seg_begin, (n_records + 1) * 8)) || (rc = need(v, v->ctr, 16)))
-        return rc;
-    if (n_records) CU(v, cudaMemcpyAsync(v->rec_line.p, rec_line, n_records * 8, cudaMemcpyHostToDevice, st));
+    CU(v->err, cudaEventRecord(v->ev[0], st));
+    CU(v->err, v->rec_line.need(n_records * 8));
+    CU(v->err, v->n_seg.need((n_records + 1) * 8));
+    CU(v->err, v->seg_begin.need((n_records + 1) * 8));
+    CU(v->err, v->ctr.need(16));
+    if (n_records) CU(v->err, cudaMemcpyAsync(v->rec_line.p, rec_line, n_records * 8, cudaMemcpyHostToDevice, st));
     // segments: at most one per 512 bytes of each selected line (from its 16-byte block of cells_begin) plus one
     uint64_t seg_cap = 0;
     for (uint64_t r = 0; r < n_records; ++r) {
@@ -796,12 +738,13 @@ int v2p_vcf_parse_masks(v2p_vcf* v, uint64_t n_records, const uint64_t* rec_line
         const uint64_t e = l + 1 < v->n_lines ? v->h_line_begin[l + 1] : v->n_bytes;  // >= the line's end
         seg_cap += e > a0 ? (e - a0 + kSeg - 1) / kSeg : 1;
     }
-    if ((rc = need(v, v->seg_tabs, (seg_cap + 1) * 8)) || (rc = need(v, v->seg_tab_x, (seg_cap + 1) * 8)) ||
-        (rc = need(v, v->seg_err, seg_cap * 4)) || (rc = need(v, v->seg_rec, seg_cap * 4)))
-        return rc;
+    CU(v->err, v->seg_tabs.need((seg_cap + 1) * 8));
+    CU(v->err, v->seg_tab_x.need((seg_cap + 1) * 8));
+    CU(v->err, v->seg_err.need(seg_cap * 4));
+    CU(v->err, v->seg_rec.need(seg_cap * 4));
     unsigned long long* ctr = (unsigned long long*)v->ctr.p;
-    CU(v, cudaMemsetAsync(ctr, 0, 8, st));
-    CU(v, cudaMemsetAsync(ctr + 1, 0xff, 8, st));
+    CU(v->err, cudaMemsetAsync(ctr, 0, 8, st));
+    CU(v->err, cudaMemsetAsync(ctr + 1, 0xff, 8, st));
     ParseArgs a{};
     a.text = v->text, a.rec_line = (const uint64_t*)v->rec_line.p, a.cells_begin = (const uint64_t*)v->cells_begin.p;
     a.line_end = (const uint64_t*)v->line_end.p, a.has_cells = (const uint8_t*)v->has_cells.p, a.line_no = (const uint32_t*)v->line_no.p;
@@ -810,17 +753,17 @@ int v2p_vcf_parse_masks(v2p_vcf* v, uint64_t n_records, const uint64_t* rec_line
     a.seg_rec = (uint32_t*)v->seg_rec.p, a.ctr = ctr;
     // k_parse hands every warp an equal run of segments; one resident wave of blocks
     int per_sm = 1;
-    CU(v, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_parse<false>, kThreads, 0));
+    CU(v->err, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_parse<false>, kThreads, 0));
     const unsigned grid = (unsigned)(v->sms * std::max(per_sm, 1));
     unsigned long long hc[2] = {0, kNone};
     if (n_records) {
         k_rec_segs<<<blocks(n_records + 1), 256, 0, st>>>(a.rec_line, n_records, a.cells_begin, a.line_end, (uint64_t*)v->n_seg.p);
-        if ((rc = xsum(v, (const uint64_t*)v->n_seg.p, (uint64_t*)v->seg_begin.p, n_records + 1))) return rc;
+        if ((rc = exclusive_sum(v->err, v->cub_tmp, (const uint64_t*)v->n_seg.p, (uint64_t*)v->seg_begin.p, n_records + 1, st))) return rc;
         k_parse<false><<<grid, kThreads, 0, st>>>(a);
         // entries past the segment total are not written; the scan values up to the total do not depend on them
-        if ((rc = xsum(v, a.seg_tabs, (uint64_t*)v->seg_tab_x.p, seg_cap + 1))) return rc;
+        if ((rc = exclusive_sum(v->err, v->cub_tmp, (const uint64_t*)a.seg_tabs, (uint64_t*)v->seg_tab_x.p, seg_cap + 1, st))) return rc;
         k_check<<<grid, 256, 0, st>>>(a);
-        CU(v, cudaGetLastError());
+        CU(v->err, cudaGetLastError());
         if ((rc = fetch(v, ctr, 2, hc))) return rc;
     }
     if (hc[1] != kNone) {
@@ -828,20 +771,20 @@ int v2p_vcf_parse_masks(v2p_vcf* v, uint64_t n_records, const uint64_t* rec_line
                                      "a mask word above 2^32-1", "a number of sample cells other than the #CHROM line's"};
         const uint64_t col = (hc[1] >> 3) & ((1ull << 29) - 1);
         const unsigned cls = (unsigned)(hc[1] & 7);
-        return vfail(v, V2P_ERR_VCF_PARSE, "VCF line %llu, sample column %llu: %s", (unsigned long long)(hc[1] >> 32) + 1,
-                     (unsigned long long)col + 1, cls <= E_COUNT ? what[cls] : "?");
+        return fail(v->err, V2P_ERR_VCF_PARSE, "VCF line %llu, sample column %llu: %s", (unsigned long long)(hc[1] >> 32) + 1,
+                    (unsigned long long)col + 1, cls <= E_COUNT ? what[cls] : "?");
     }
     const uint32_t W = hc[0] ? (uint32_t)hc[0] : 1;
     const uint64_t n_words = n_records * v->n_samples * W;
-    if (n_records && v->n_samples && n_words / n_records / v->n_samples != W) return vfail(v, V2P_ERR_INVALID_ARG, "matrix size overflows");
-    if ((rc = need(v, v->masks, n_words * 4))) return rc;
+    if (n_records && v->n_samples && n_words / n_records / v->n_samples != W) return fail(v->err, V2P_ERR_INVALID_ARG, "matrix size overflows");
+    CU(v->err, v->masks.need(n_words * 4));
     a.masks = (uint32_t*)v->masks.p, a.W = W;
     if (n_records && v->n_samples) k_parse<true><<<grid, kThreads, 0, st>>>(a);
-    CU(v, cudaGetLastError());
-    CU(v, cudaEventRecord(v->ev[1], st));
-    CU(v, cudaStreamSynchronize(st));
+    CU(v->err, cudaGetLastError());
+    CU(v->err, cudaEventRecord(v->ev[1], st));
+    CU(v->err, cudaStreamSynchronize(st));
     float ms = 0;
-    CU(v, cudaEventElapsedTime(&ms, v->ev[0], v->ev[1]));
+    CU(v->err, cudaEventElapsedTime(&ms, v->ev[0], v->ev[1]));
     out->masks = (const uint32_t*)v->masks.p, out->n_records = n_records, out->n_samples = v->n_samples, out->words_per_cell = W;
     out->parse_ms = ms;
     return V2P_OK;
