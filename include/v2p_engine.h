@@ -158,7 +158,9 @@ typedef struct {
  * reference's serial semantics (later task wins), only slower.
  * Without V2P_FLAG_DEVICE_PTRS all pointers are host memory (pinned recommended) and the call performs
  * H2D of tasks/tapes and D2H of `out` on the engine's streams.
- * With V2P_FLAG_ASYNC `*done` receives an event; result via v2p_event_wait.  Otherwise `res` is filled. */
+ * With V2P_FLAG_ASYNC `*done` receives an event; result via v2p_event_wait.  Otherwise `res` is filled.
+ * Any number of V2P_FLAG_DEVICE_PTRS | V2P_FLAG_ASYNC launches may be in flight at once, waited in any order
+ * (host-pointer launches: up to 3, one per staging slot). */
 int v2p_execute_batch(v2p_engine* e, const v2p_batch* batch, uint32_t flags, v2p_result* res, v2p_event** done);
 int v2p_event_wait(v2p_engine* e, v2p_event* ev, v2p_result* res); /* also releases the event */
 

@@ -29,8 +29,8 @@ using namespace v2p;
 
 namespace {
 
-struct Scratch {  // per-stream planning scratch
-    DevBuf lb, tile_hap, chunk_hap, order, status, hap_flags, ser_list;
+struct Scratch {  // per-stream planning scratch: used only by the kernels of the launch group itself
+    DevBuf lb, tile_hap, chunk_hap, order, status, hap_flags;
 };
 
 constexpr int kSlots = 3;
@@ -47,7 +47,7 @@ constexpr int kSoaSlots = 16;  // concurrent v2p_execute_soa / v2p_gir_execute c
 struct SoaSlot {  // everything one in-flight single-haplotype call needs: nobody else touches it until the call returns
     cudaStream_t stream = nullptr;
     Scratch sc;
-    DevBuf d_soa[4], tasks, ref, alt, out, bases;
+    DevBuf d_soa[4], tasks, ref, alt, out, bases, ser_list;
     MappedBuf h_status;  // one DevStatus
     PinnedBuf h_stage;   // staging of the 1-byte tapes (ref | alt | res), grown on demand
     bool busy = false;
@@ -59,6 +59,7 @@ struct v2p_event {
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_done = nullptr, ev_copy = nullptr;
     MappedBuf h_status;             // one DevStatus, published right behind the launch group
     KParams kp;                     // for the deferred serial fallback
+    DevBuf ser_list;                // kp.ser_list: k_serial reads it at the wait, after any later launch's plan
     cudaStream_t stream = nullptr;
     Slot* slot = nullptr;  // host-pointer mode
     uint8_t* h_out = nullptr;
@@ -127,8 +128,9 @@ constexpr int kNumVariants = (int)(sizeof(kVariants) / sizeof(kVariants[0]));
 constexpr int kAutoTma = 8, kAutoPlain = 0;  // measured best per path (profiles/r1)
 
 // plan + copy on stream s.  kp.{lb,tile_hap,status,n_tiles,tile_bytes} are filled here.
-int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, KParams& kp, cudaEvent_t ev_start, cudaEvent_t ev_stop,
-                 DevStatus* h_status, bool init_status, cudaEvent_t ev_copy, bool aligned_layout) {
+// ser_list is the launch's own (k_serial may read it long after the launch group, see k_serial).
+int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, DevBuf& ser_list, KParams& kp, cudaEvent_t ev_start,
+                 cudaEvent_t ev_stop, DevStatus* h_status, bool init_status, cudaEvent_t ev_copy, bool aligned_layout) {
     const CopyVariant& cv = kVariants[e->variant >= 0 ? e->variant : (kp.tma_mode ? kAutoTma : kAutoPlain)];
     const int T = cv.tile;
     kp.tile_bytes = (uint32_t)T;
@@ -144,9 +146,9 @@ int launch_group(v2p_engine* e, cudaStream_t s, Scratch& sc, KParams& kp, cudaEv
     kp.chunk_hap = (uint32_t*)sc.chunk_hap.p;
     // per-haplotype "needs serial order" flags (+ one counter word behind them) and the compacted list of those
     CU(t_err, sc.hap_flags.need((kp.n_hap + 1) * sizeof(uint32_t)));
-    CU(t_err, sc.ser_list.need(std::max<uint64_t>(kp.n_hap, 1) * sizeof(uint32_t)));
+    CU(t_err, ser_list.need(std::max<uint64_t>(kp.n_hap, 1) * sizeof(uint32_t)));
     kp.hap_flags = (uint32_t*)sc.hap_flags.p;
-    kp.ser_list = (uint32_t*)sc.ser_list.p;
+    kp.ser_list = (uint32_t*)ser_list.p;
     // tile order: 16-byte header (s_max) + one slot per (tile rank within its haplotype, haplotype)
     if (kp.n_tiles >= 0xFFF00000ull) return fail(t_err, V2P_ERR_INVALID_ARG, "more than 2^32 tiles in one launch");
     // tape order = identity over n_tiles (n_hap "1"): the cap then only has to hold the identity
@@ -603,8 +605,8 @@ int v2p_execute_batch(v2p_engine* e, const v2p_batch* b, uint32_t flags, v2p_res
         kp.tma_mode = e->ref_tma_mode;
     }
     ev->stream = s;
-    rc = launch_group(e, s, *sc, kp, ev->ev_start, ev->ev_stop, reinterpret_cast<DevStatus*>(ev->h_status.p), true, ev->ev_copy,
-                      (flags & V2P_FLAG_ALIGNED_LAYOUT) != 0);
+    rc = launch_group(e, s, *sc, ev->ser_list, kp, ev->ev_start, ev->ev_stop, reinterpret_cast<DevStatus*>(ev->h_status.p),
+                      true, ev->ev_copy, (flags & V2P_FLAG_ALIGNED_LAYOUT) != 0);
     if (rc) return bail(rc);
     // host mode: the copy-back is enqueued right away (a batch that needs the serial-order kernel repeats it later)
     if (ev->slot && ev->out_bytes &&
@@ -730,7 +732,9 @@ int soa_run(v2p_engine* e, SoaSlot* sl, size_t n_tasks, const uint64_t* exec_cod
     kp.n_out = n_res * unit;
     kp.fill_word = unit == 1 ? 0x2E2E2E2Eu : 0x0000002Eu;  // '.' per byte, or as one UTF-32 unit
     kp.keep_out = keep ? 1 : 0;
-    kp.validate = (flags & V2P_FLAG_VALIDATE) ? 1 : 0;
+    // kp.validate stays 0: k_soa_pack judges contiguity on the caller's 64-bit values, and the packed tasks it hands
+    // to the plan have every rejected task zeroed, which the plan would take for a contiguity break of its own
+    const int validate = (flags & V2P_FLAG_VALIDATE) ? 1 : 0;
 
     // pack (and judge every reference panic on the original 64-bit values), then plan + copy
     kp.status = (DevStatus*)sl->sc.status.p;
@@ -739,10 +743,10 @@ int soa_run(v2p_engine* e, SoaSlot* sl, size_t n_tasks, const uint64_t* exec_cod
     if (n_tasks) {
         k_soa_pack<<<(unsigned)((n_tasks + 255) / 256), 256, 0, s>>>(
             n_tasks, (const uint64_t*)sl->d_soa[0].p, (const uint64_t*)sl->d_soa[1].p, (const uint64_t*)sl->d_soa[2].p,
-            (const uint64_t*)sl->d_soa[3].p, n_ref, n_alt, n_res, unit, kp.validate, (v2p_task16*)sl->tasks.p, kp.status);
+            (const uint64_t*)sl->d_soa[3].p, n_ref, n_alt, n_res, unit, validate, (v2p_task16*)sl->tasks.p, kp.status);
         e->launches++;
     }
-    rc = launch_group(e, s, sl->sc, kp, nullptr, nullptr, h_status, /*init_status=*/false, nullptr, false);
+    rc = launch_group(e, s, sl->sc, sl->ser_list, kp, nullptr, nullptr, h_status, /*init_status=*/false, nullptr, false);
     if (rc) return rc;
     CU(t_err, cudaStreamSynchronize(s));
     if (needs_serial(*h_status)) {

@@ -221,6 +221,9 @@ __device__ __forceinline__ void plan_one(const KParams& p, const PlanHap& m, con
     const bool bad_stream = stream > 1u;                                           // haplotype_instruction.rs:154
     const bool bad_res = (uint64_t)dst + len > m.n_res;                            // task.rs:44/48 (result slice)
     const bool bad_src = (uint64_t)src + len > (stream == 0 ? m.n_ref : m.n_alt);  // task.rs:44/48 (source slice)
+    // gir.rs:208 contiguity (VALIDATE): the validator sees the whole Task array before any task runs, so a task that
+    // does not start where the previous one ended is reported as such, whether it leaves a gap, goes back or has a bad slice
+    if (p.validate && tr != m.tb0 && dst != (uint64_t)p_dst + p_len) atomicMin(&p.status->gap_key, (unsigned long long)tr);
     if (bad_stream | bad_res | bad_src) {
         if (bad_stream) atomicMin(&p.status->stream_key, (unsigned long long)tr);
         else atomicMin(&p.status->err_key, ((unsigned long long)tr << 8) | (bad_res ? V2P_ERR_RES_OOB : V2P_ERR_SRC_OOB));
@@ -231,16 +234,13 @@ __device__ __forceinline__ void plan_one(const KParams& p, const PlanHap& m, con
     auto mark_gap = [&](uint64_t a, uint64_t b) {  // launch-relative byte range [a, b)
         for (uint64_t k = a >> p.tile_shift; k <= ((b - 1) >> p.tile_shift) && k < p.n_tiles; ++k) atomicOr(p.tile_hap + k, kTileHasGap);
     };
-    if (tr != m.tb0) {  // previous task is in the same haplotype: gir.rs:208 contiguity + sortedness
+    if (tr != m.tb0) {  // previous task is in the same haplotype: sortedness
         const uint64_t pend = (uint64_t)p_dst + p_len;
         if (dst < pend) {  // this haplotype needs the reference's order semantics (later task wins): k_serial
             if (atomicExch(p.hap_flags + m.h, 1u) == 0u) atomicAdd(&p.status->unsorted, 1u);
             return;
         }
-        if (dst != pend) {
-            if (p.validate) atomicMin(&p.status->gap_key, (unsigned long long)tr);
-            mark_gap(m.orel + pend, m.orel + dst);
-        }
+        if (dst != pend) mark_gap(m.orel + pend, m.orel + dst);
     } else if (dst != 0u) {
         mark_gap(m.orel, m.orel + dst);  // in front of the haplotype's first task
     }
@@ -1022,8 +1022,9 @@ __global__ void __launch_bounds__(kThreads, MINB) k_copy_tiles(const KParams p) 
 // span, clipped to it, one after the other.  Every byte therefore sees its writers in array order, with no
 // inter-CTA ordering needed; the price is that every span re-reads the haplotype's task array (L2-resident, ~20k
 // tasks), which is why this is not the main path.
-// Launched by the host only after the plan reported `unsorted` and no error (status is not re-read here: a later
-// asynchronous launch may already have re-initialised the shared status block; the count is passed by value).
+// Launched by the host only after the plan reported `unsorted` and no error, when the call is waited -- possibly after
+// later asynchronous launches on the same stream have reused the engine's scratch.  So nothing here is read from that
+// scratch: the count is passed by value, and ser_list belongs to the launch (its event, or its single-haplotype slot).
 constexpr int kSerialThreads = 512;
 constexpr uint32_t kSerialSpan = 16384;
 __global__ void __launch_bounds__(kSerialThreads) k_serial(const KParams p, const uint32_t n_ser) {
